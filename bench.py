@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port)
+    python bench.py ... --dump-outputs DIR                   # also write X, y, S after the timed steps as DIR/*.npy
 
 A "step" is one sGS-ADMM iteration (src/solver.cu:469-799 of the reference): two A A^T y-solves, three
 SpMV with A, two with A^T, the PSD projection of every block and the residual / sigma update.  Workload
@@ -42,7 +43,13 @@ def parse_args():
                     help="c2b (default, BASELINE.json configs[1]); c3 = max-cut n=4000 (configs[2]); c4 = 10k mixed "
                          "blocks {10,50,200,800}, m=1e6 (configs[3], the multi-GPU scaling configuration); "
                          "c5 = 4 x 8000 + 500 small blocks (configs[4])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the iterate X, y, S the timed steps end on as DIR/<name>.npy (float64; a fixed seeded sample "
+                         "of each when they exceed 64 MB together), so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
+    return args
 
 
 def workload(name, args):
@@ -171,7 +178,8 @@ def fp64_peak_tflops(torch):
 # (oracle/cpu_baseline.cpp) inside the oracle's ADMM iteration, sparse solves by SuperLU
 # (CHOLMOD-substitute).  The only places bench.py may execute oracle/ (cpu_baseline and --impl reference).
 # ---------------------------------------------------------------------------------------------
-def cpu_reference_iterations(P, n_iters, threads, budget_s=60.0):
+def cpu_reference_iterations(P, n_iters, threads, budget_s=None):
+    """n_iters timed iterations; with budget_s, fewer when they would run longer than budget_s seconds (at least one)"""
     sys.path.insert(0, os.path.join(ROOT, "oracle"))
     import oracle_np as onp
     blk = np.ascontiguousarray(P["blk"], np.int32)
@@ -182,7 +190,7 @@ def cpu_reference_iterations(P, n_iters, threads, budget_s=60.0):
     t_init = time.time() - t0
     o.solve(1, -1.0, 500, 50, 100, 1 << 30, 1.05)          # one untimed iteration
     done, t0 = 0, time.time()
-    while done < n_iters and (done == 0 or time.time() - t0 < budget_s):
+    while done < n_iters and (budget_s is None or done == 0 or time.time() - t0 < budget_s):
         o.solve(1, -1.0, 500, 50, 100, 1 << 30, 1.05)
         done += 1
     dt = time.time() - t0
@@ -196,7 +204,7 @@ def run_reference(args):
     P, cfg = workload(args.workload, args)
     cores = os.cpu_count() or 1
     threads = min(30, cores)          # the reference's default cpu_eig_thread_num (src/main.cu:11)
-    val, dt, t_init, steps = cpu_reference_iterations(P, max(1, args.steps), threads, budget_s=90.0)
+    val, dt, t_init, steps = cpu_reference_iterations(P, max(1, args.steps), threads)     # exactly --steps timed iterations
     line = {"impl": "reference", "metric": "ADMM iterations/s", "value": val, "unit": "iter/s", "n_gpus": args.gpus,
             "steps": steps, "warmup": 1, "ms_per_step": 1e3 / val, "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic", "config": cfg,
@@ -272,8 +280,27 @@ class Job:
         return bytes(idt.cpu().numpy().tolist())
 
 
-def measure(job, cu, P, steps, warmup, e2e_steps, sampler=None):
-    """init + K timed iterations + profiled pass (+ e2e) of one workload on job.world GPUs"""
+DUMP_BYTES = 60_000_000     # data of all dumped arrays; with the .npy headers under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays (name -> float64 vector) as out_dir/<name>.npy.  Beyond DUMP_BYTES in all, every array keeps the same
+    fraction k of its entries: one per stratum [i n // k, (i+1) n // k), at an offset drawn by default_rng(0), so the
+    indices are sorted and distinct.  They depend only on the array's length: runs with the same arguments sample the
+    same entries."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            k = len(a) * DUMP_BYTES // total
+            lo = np.arange(k + 1, dtype=np.int64) * len(a) // k
+            a = a[lo[:-1] + (np.random.default_rng(0).random(k) * np.diff(lo)).astype(np.int64)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def measure(job, cu, P, steps, warmup, e2e_steps, sampler=None, keep_outputs=False):
+    """init + K timed iterations (+ the iterate they end on, read back to the host) + profiled pass (+ e2e) of one
+    workload on job.world GPUs"""
     torch = job.torch
     s = cu.Solver(verbose=False)
     s.set_device(job.local)
@@ -292,6 +319,8 @@ def measure(job, cu, P, steps, warmup, e2e_steps, sampler=None):
     job.barrier()
     ms_total = job.max(r["total_ms"])
     launches = s.launches - launches0
+    # read before the profiled pass moves the iterate on; X and S are gathered over the ranks, so all of them read
+    outputs = {"X": s.X, "y": s.y, "S": s.S} if keep_outputs else None
     # stage breakdown (separate profiled pass: events around every y-solve and projection)
     nprof = min(steps, 50)
     prof = s.run_iterations(nprof, sgs=True, profile=True)
@@ -305,7 +334,7 @@ def measure(job, cu, P, steps, warmup, e2e_steps, sampler=None):
     out = {"ms_total": ms_total, "launches": int(launches), "init_s": t_init,
            "stage": {"projection": prof["projection_ms"] / nprof, "ysolve_x2": prof["ysolve_ms"] / nprof,
                      "spmv_and_rest": prof["other_ms"] / nprof},
-           "t_load": (t_load0, t_load1), "ysolve": s.ysolve_stats()}
+           "t_load": (t_load0, t_load1), "ysolve": s.ysolve_stats(), "outputs": outputs}
     if e2e_steps > 0:
         # e2e: the same iteration through the public C ABI with HOST buffers — every step uploads the iterate
         # (X, y, S) from pinned host memory, runs one iteration (solve(max_iter=1, if_first=False), the
@@ -353,8 +382,11 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     big = args.workload in ("c4", "c5")
-    R = measure(job, cu, P, args.steps, args.warmup, max(3, min(args.steps, 10 if big else 30)), sampler)
+    R = measure(job, cu, P, args.steps, args.warmup, max(3, min(args.steps, 10 if big else 30)), sampler,
+                keep_outputs=args.dump_outputs is not None)
     clocks = sampler.stop(*R["t_load"]) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, R.pop("outputs"))     # after the clock window: files are written with the GPU idle
 
     # C4 sub-record: the configuration north_star names for multi-GPU scaling, measured the same way
     scale_c4 = None

@@ -22,11 +22,30 @@ def test_maps_bit_exact_vs_oracle(ohost, blk):
     assert p.vec_len == sum(n * (n + 1) // 2 for n in blk)
 
 
-def test_maps_and_partition_bit_exact_vs_reference_build(oref):
+def test_maps_and_partition_bit_exact_vs_reference_build(ohost, request):
     rng = np.random.default_rng(7)
     planar = np.loadtxt(os.path.join(ROOT, "tests", "golden", "planarhand_n1_blk.txt"), dtype=np.int32)
-    for blk in CASES + [planar.tolist(), rng.integers(1, 60, 500).tolist()]:
-        blk = np.array(blk, np.int32)
+    lists = [np.array(blk, np.int32) for blk in CASES + [planar.tolist(), rng.integers(1, 60, 500).tolist()]]
+    # the same lists against the C restatement of analyze_blk / MatrixSizes / get_maps, which needs no reference build
+    for blk in lists:
+        p = cu.Plan(blk, device=-1)
+        assert all(np.array_equal(a, b) for a, b in zip(p.maps(), oracle_maps(ohost, blk)))
+        n = len(blk)
+        sizes = np.zeros(n, np.int32); nums = np.zeros(n, np.int32)
+        ns = ohost.oracle_analyze_blk(ip(blk), n, ip(sizes), ip(nums))
+        ls, ln, lm, lw, ss, sn, sm, sw = (np.zeros(ns + 2, np.int32) for _ in range(8))
+        tot = np.zeros(6, np.int32)
+        packed = ohost.oracle_matrix_sizes(ip(sizes), ip(nums), ns, ip(ls), ip(ln), ip(lm), ip(lw), ip(ss), ip(sn), ip(sm),
+                                           ip(sw), ip(tot))
+        nl, nsm = packed & 0xffff, packed >> 16
+        s, c, l = p.sizes()
+        assert s.tolist() == sizes[:ns].tolist() and c.tolist() == nums[:ns].tolist()
+        assert l.tolist() == [ohost.oracle_is_large_mat(int(a), int(b)) for a, b in zip(sizes[:ns], nums[:ns])]
+        assert p.totals().tolist() == tot.tolist()
+        assert p.start_indices(0).tolist() == lm[:nl + 1].tolist() and p.start_indices(1).tolist() == lw[:nl + 1].tolist()
+        assert p.start_indices(2).tolist() == sm[:nsm + 1].tolist() and p.start_indices(3).tolist() == sw[:nsm + 1].tolist()
+    oref = request.getfixturevalue("oref")      # skips here when the reference build is absent
+    for blk in lists:
         p = cu.Plan(blk, device=-1)
         L = p.vec_len
         B, M1, M2 = p.maps()
