@@ -48,6 +48,18 @@ def _p(a, t):
     return a.ctypes.data_as(t) if a is not None else None
 
 
+def _types(types, nblk):
+    """block cones as the C ABI takes them: nblk letters 's' (PSD), 'l' (nonnegative), 'u' (free); None stays None
+    (every block PSD).  Accepts a string, bytes or a sequence of one-letter strings."""
+    if types is None:
+        return None
+    t = types.encode() if isinstance(types, str) else bytes(types) if isinstance(types, (bytes, bytearray)) \
+        else "".join(types).encode()
+    if len(t) != nblk:
+        raise ValueError(f"{len(t)} block types for {nblk} blocks")
+    return t
+
+
 def version():
     return lib.cuadmm_version().decode()
 
@@ -66,6 +78,7 @@ def _sig(name, restype, *argtypes):
 
 # ---------------------------------------------------------------- plan
 _sig("cuadmm_plan_create", C.c_int, c_i32p, C.c_int64, C.c_int, C.POINTER(vp))
+_sig("cuadmm_plan_create_typed", C.c_int, C.c_char_p, c_i32p, C.c_int64, C.c_int, C.POINTER(vp))
 _sig("cuadmm_plan_destroy", None, vp)
 _sig("cuadmm_plan_vec_len", C.c_int64, vp)
 _sig("cuadmm_plan_nblk", C.c_int64, vp)
@@ -83,18 +96,24 @@ _sig("cuadmm_plan_last_ms", C.c_double, vp)
 _sig("cuadmm_plan_last_launches", C.c_int64, vp)
 _sig("cuadmm_project_psd", C.c_int, vp, vp, vp, vp)
 _sig("cuadmm_project_psd_host", C.c_int, vp, c_f64p, c_f64p)
+_sig("cuadmm_project_epilogue", C.c_int, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp)
 _sig("cuadmm_project_psd_eig_host", C.c_int, vp, c_f64p, c_f64p, c_f64p, c_i32p)
 _sig("cuadmm_svec_to_smat", C.c_int, vp, vp, vp, vp, vp)
 _sig("cuadmm_smat_to_svec", C.c_int, vp, vp, vp, vp, vp)
 
 
 class Plan:
-    """Block plan + PSD projection (cuadmm_plan_*, cuadmm_project_psd*)."""
+    """Block plan + cone projection (cuadmm_plan_*, cuadmm_project_psd*).  types: one letter per block, 's' PSD,
+    'l' nonnegative orthant, 'u' free (None: all 's')."""
 
-    def __init__(self, blk, device=0):
+    def __init__(self, blk, device=0, types=None):
         self.blk = _i32(blk)
+        self.types = _types(types, len(self.blk))
         self.h = vp()
-        _check(lib.cuadmm_plan_create(_p(self.blk, c_i32p), len(self.blk), device, C.byref(self.h)))
+        if self.types is None:
+            _check(lib.cuadmm_plan_create(_p(self.blk, c_i32p), len(self.blk), device, C.byref(self.h)))
+        else:
+            _check(lib.cuadmm_plan_create_typed(self.types, _p(self.blk, c_i32p), len(self.blk), device, C.byref(self.h)))
         self.device = device
 
     def close(self):
@@ -129,6 +148,8 @@ class Plan:
 
     def start_indices(self, which):
         k = lib.cuadmm_plan_start_indices(self.h, which, None)
+        if k < 0:
+            raise CuadmmError(k, lib.cuadmm_last_error().decode())
         out = np.zeros(k, np.int64)
         lib.cuadmm_plan_start_indices(self.h, which, _p(out, c_i64p))
         return out
@@ -172,6 +193,12 @@ class Plan:
     def project_device(self, d_in_ptr, d_out_ptr, stream=0):
         """device pointers (ints), e.g. torch tensor .data_ptr()"""
         _check(lib.cuadmm_project_psd(self.h, vp(d_in_ptr), vp(d_out_ptr), vp(stream)))
+
+    def project_epilogue_device(self, d_Xb, d_Xproj, d_X, d_Rd1, d_C, d_S, d_SmC, d_sig, stream=0):
+        """projection with the solver's fused epilogue: S = (Xproj - X)/sig - Rd1, SmC = S - C (S = 0 on 'u' blocks);
+        device pointers (ints), d_sig a device scalar"""
+        _check(lib.cuadmm_project_epilogue(self.h, vp(d_Xb), vp(d_Xproj), vp(d_X), vp(d_Rd1), vp(d_C), vp(d_S), vp(d_SmC),
+                                           vp(d_sig), vp(stream)))
 
     def svec_to_smat_device(self, d_svec, d_large, d_small, stream=0):
         _check(lib.cuadmm_svec_to_smat(self.h, vp(d_svec), vp(d_large), vp(d_small), vp(stream)))
@@ -332,6 +359,9 @@ _maybe("cuadmm_unique_id", C.c_int, C.c_char_p)
 _maybe("cuadmm_solver_set_device", C.c_int, vp, C.c_int)
 _maybe("cuadmm_solver_set_distributed", C.c_int, vp, C.c_int, C.c_int, C.c_char_p)
 _maybe("cuadmm_shard_create", C.c_int, c_i32p, C.c_int64, C.c_int, C.c_int, C.POINTER(vp))
+_maybe("cuadmm_shard_create_typed", C.c_int, C.c_char_p, c_i32p, C.c_int64, C.c_int, C.c_int, C.POINTER(vp))
+_maybe("cuadmm_shard_local_types", C.c_int, vp, C.c_char_p)
+_maybe("cuadmm_solver_set_block_types", C.c_int, vp, C.c_char_p, C.c_int64)
 _maybe("cuadmm_shard_destroy", None, vp)
 _maybe("cuadmm_shard_info", C.c_int, vp, c_i64p)
 _maybe("cuadmm_shard_maps", C.c_int, vp, c_i32p, c_i64p, c_i64p, c_i32p)
@@ -362,10 +392,15 @@ def unique_id():
 class Shard:
     """Block-level sharding of an SDP over `world` GPUs (cuadmm_shard_*; host logic only)."""
 
-    def __init__(self, blk, world, rank):
+    def __init__(self, blk, world, rank, types=None):
         self.blk = _i32(blk)
+        self.types = _types(types, len(self.blk))
         self.h = vp()
-        _check(lib.cuadmm_shard_create(_p(self.blk, c_i32p), len(self.blk), world, rank, C.byref(self.h)))
+        if self.types is None:
+            _check(lib.cuadmm_shard_create(_p(self.blk, c_i32p), len(self.blk), world, rank, C.byref(self.h)))
+        else:
+            _check(lib.cuadmm_shard_create_typed(self.types, _p(self.blk, c_i32p), len(self.blk), world, rank,
+                                                 C.byref(self.h)))
         info = np.zeros(4, np.int64)
         _check(lib.cuadmm_shard_info(self.h, _p(info, c_i64p)))
         self.vec_len_local, self.nblk_local, self.vec_len, self.world = [int(x) for x in info]
@@ -375,6 +410,9 @@ class Shard:
         self.owner = np.zeros(len(self.blk), np.int32)
         _check(lib.cuadmm_shard_maps(self.h, _p(self.local_blk, c_i32p), _p(self.local_block_ids, c_i64p),
                                      _p(self.loc2glob, c_i64p), _p(self.owner, c_i32p)))
+        buf = C.create_string_buffer(max(self.nblk_local, 1))
+        _check(lib.cuadmm_shard_local_types(self.h, buf))
+        self.local_types = buf.raw[:self.nblk_local].decode()
 
     def slice_csc(self, col_ptrs, row_ids, vals):
         col_ptrs, row_ids, vals = _i32(col_ptrs), _i32(row_ids), _f64(vals)
@@ -410,6 +448,12 @@ class Problem:
         _check(lib.cuadmm_problem_dims(self.h, _p(d, c_i64p)))
         self.vec_len, self.con_num, self.mat_num, self.At_nnz, self.b_nnz, self.C_nnz = [int(x) for x in d[:6]]
         self.has_warm = bool(d[6])
+
+    @property
+    def blk_types(self):
+        """the blk.txt letter of every block ('s', 'l' or 'u'), as one string"""
+        ptr = lib.cuadmm_problem_array(self.h, 11)
+        return C.string_at(ptr, self.mat_num).decode() if ptr and self.mat_num else ""
 
     def array(self, which):
         n = {0: self.con_num + 1, 1: self.At_nnz, 2: self.At_nnz, 3: self.b_nnz, 4: self.b_nnz, 5: self.C_nnz,
@@ -465,13 +509,16 @@ class Solver:
 
     def init(self, eig_stream_num_per_gpu, cpu_eig_thread_num, vec_len, con_num,
              At_csc_col_ptrs, At_csc_row_ids, At_csc_vals, b_indices, b_vals, C_indices, C_vals, blk_vals,
-             X_vals=None, y_vals=None, S_vals=None, sig=1.0):
+             X_vals=None, y_vals=None, S_vals=None, sig=1.0, blk_types=None):
+        """blk_types: one letter per block, 's' PSD, 'l' nonnegative, 'u' free (None: all 's')"""
         cp, ri, av = _i32(At_csc_col_ptrs), _i32(At_csc_row_ids), _f64(At_csc_vals)
         bi, bv, ci, cv, blk = _i32(b_indices), _f64(b_vals), _i32(C_indices), _f64(C_vals), _i32(blk_vals)
         X = _f64(X_vals) if X_vals is not None else None
         y = _f64(y_vals) if y_vals is not None else None
         S = _f64(S_vals) if S_vals is not None else None
         self.vec_len, self.con_num = int(vec_len), int(con_num)
+        if blk_types is not None:
+            _check(lib.cuadmm_solver_set_block_types(self.h, _types(blk_types, len(blk)), len(blk)))
         _check(lib.cuadmm_solver_init(self.h, eig_stream_num_per_gpu, cpu_eig_thread_num, vec_len, con_num,
                                       _p(cp, c_i32p), _p(ri, c_i32p), _p(av, c_f64p), len(av),
                                       _p(bi, c_i32p), _p(bv, c_f64p), len(bv), _p(ci, c_i32p), _p(cv, c_f64p), len(cv),

@@ -15,19 +15,31 @@ bool is_large_mat(int mat_size, int mat_num) {
     return ((double)mat_size - 17.0 > (double)mat_num * 1.4);
 }
 
-void BlockLayout::init(const int32_t* blk_vals, int64_t nblk) {
+// LPT cost of one 'l' / 'u' entry in the unit of eig_cost (1e-7 us): proj_linear_kernel with the fused epilogue takes
+// 0.0865 ms for 1e7 entries = 8.65e-6 us per entry (B200, 1000 W, profiles/cones_probe_r03.json)
+static const double LINEAR_COST_PER_ENTRY = 86.0;
+
+bool valid_cone(char type) { return type == 's' || type == 'l' || type == 'u'; }
+
+int64_t block_entries(char type, int64_t n) { return type == 's' ? tri(n) : n; }
+
+void BlockLayout::init(const int32_t* blk_vals, int64_t nblk, const char* types_in) {
     CUADMM_REQUIRE(nblk >= 0, "nblk < 0");
     blk.assign(blk_vals, blk_vals + nblk);
+    if (types_in) types.assign(types_in, types_in + nblk); else types.assign(nblk, 's');
     svec_off.assign(nblk + 1, 0);
+    linear_blocks = 0;
     for (int64_t k = 0; k < nblk; ++k) {
         CUADMM_REQUIRE(blk[k] >= 1, "block size must be >= 1");
-        svec_off[k + 1] = svec_off[k] + tri(blk[k]);
+        CUADMM_REQUIRE(valid_cone(types[k]), std::string("unknown block type '") + types[k] + "' (expected 's', 'l' or 'u')");
+        svec_off[k + 1] = svec_off[k] + block_entries(types[k], blk[k]);
+        if (types[k] != 's') ++linear_blocks;
     }
     vec_len = svec_off[nblk];
 
-    // distinct sizes ascending with multiplicity (std::set order in the reference)
+    // distinct sizes ascending with multiplicity (std::set order in the reference); 's' blocks only
     std::map<int32_t, int32_t> cnt;
-    for (int64_t k = 0; k < nblk; ++k) cnt[blk[k]]++;
+    for (int64_t k = 0; k < nblk; ++k) if (types[k] == 's') cnt[blk[k]]++;
     sizes.clear(); nums.clear(); large.clear();
     for (auto& kv : cnt) {
         sizes.push_back(kv.first);
@@ -64,6 +76,7 @@ void BlockLayout::init(const int32_t* blk_vals, int64_t nblk) {
     std::map<int32_t, uint8_t> is_large_of;
     for (size_t i = 0; i < sizes.size(); ++i) is_large_of[sizes[i]] = large[i];
     for (int64_t k = 0; k < nblk; ++k) {
+        if (types[k] != 's') continue;   // pool 0, offsets 0: never read
         int64_t s = blk[k];
         int64_t j = seen[blk[k]]++;
         int g = group_of[blk[k]];
@@ -79,7 +92,14 @@ void BlockLayout::init(const int32_t* blk_vals, int64_t nblk) {
     }
 }
 
+void BlockLayout::require_all_psd(const char* what) const {
+    if (!all_psd())
+        throw Error(CUADMM_EINVAL, std::string(what) + ": the plan holds 'l'/'u' blocks, which have no place in the "
+                                   "reference's pooled dense layout (only all-'s' plans have one)");
+}
+
 void BlockLayout::maps(int32_t* map_B, int32_t* map_M1, int32_t* map_M2) const {
+    require_all_psd("svec maps");
     CUADMM_REQUIRE(total_large_mat_size <= INT32_MAX && total_small_mat_size <= INT32_MAX &&
                    vec_len <= INT32_MAX,
                    "int32 svec maps requested for a layout that overflows int32 (the reference overflows here)");
@@ -110,12 +130,22 @@ double BlockLayout::eig_cost(int n) {
     return 6.0e5 * (0.5 * T * (T + 1.0)) * nn;
 }
 
+double BlockLayout::block_cost(char type, int n) {
+    if (type == 's') return eig_cost(n);
+    // 'l' / 'u': one streaming pass of the linear-cone kernel (56 B per entry with the fused epilogue) plus the floor of a
+    // PSD block
+    return 2.0e3 + LINEAR_COST_PER_ENTRY * (double)n;
+}
+
 void BlockLayout::partition(int nparts, int32_t* owner, double* part_cost) const {
     CUADMM_REQUIRE(nparts >= 1, "nparts < 1");
     const int64_t nblk = (int64_t)blk.size();
+    std::vector<double> cost(nblk);
+    for (int64_t k = 0; k < nblk; ++k) cost[k] = block_cost(types[k], blk[k]);
     std::vector<int64_t> order(nblk);
     std::iota(order.begin(), order.end(), 0);
-    std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return blk[a] > blk[b]; });
+    // (eig_cost is strictly increasing in n, so for all-'s' layouts this is the order by size)
+    std::stable_sort(order.begin(), order.end(), [&](int64_t a, int64_t b) { return cost[a] > cost[b]; });
     std::vector<double> load(nparts, 0.0);
     // min-heap on (load, part index) keeps ties deterministic
     typedef std::pair<double, int> LP;
@@ -125,7 +155,7 @@ void BlockLayout::partition(int nparts, int32_t* owner, double* part_cost) const
         LP top = heap.top(); heap.pop();
         int64_t k = order[t];
         owner[k] = top.second;
-        top.first += eig_cost(blk[k]);
+        top.first += cost[k];
         load[top.second] = top.first;
         heap.push(top);
     }

@@ -11,6 +11,21 @@ void dense_part_destroy(cuadmm::DensePart* p);
 int dense_part_project(cuadmm::DensePart* D, const double* Xb, double* Xproj, cudaStream_t st,
                        const cuadmm::ProjEpilogue* epi, const int* done_flag);
 
+namespace cuadmm {
+// one CTA of proj_linear_kernel (cones.cu): a run of 'l' or 'u' entries of at most kLinearChunk entries
+struct LinChunk {
+    int64_t off;      // first svec entry
+    int32_t len;
+    int32_t cone;     // 'l' or 'u'
+};
+constexpr int kLinearChunk = 4096;
+// the 'l' / 'u' blocks of a layout as chunks; consecutive blocks of one cone are merged first (they are contiguous)
+std::vector<LinChunk> linear_chunks(const BlockLayout& layout);
+// one launch for all chunks; returns the number of kernel launches (1)
+int linear_project(const LinChunk* d_chunks, int64_t nchunks, const double* Xb, double* Xproj, cudaStream_t st,
+                   const ProjEpilogue* epi, const int* done_flag);
+}  // namespace cuadmm
+
 struct cuadmm_plan {
     int device = -1;
     cuadmm::BlockLayout layout;
@@ -51,6 +66,13 @@ struct cuadmm_plan {
     std::vector<cudaEvent_t> side_events;
     cudaEvent_t fork_event = nullptr;
     cuadmm::DensePart* dense = nullptr;        // blocks n > 168: GEMM-only sign-function path (dense_proj.cu)
+    // 'l' / 'u' blocks: one proj_linear_kernel launch over these chunks (cones.cu), on its own side stream when
+    // anything else runs; a plan without such blocks issues no launch and no extra event
+    std::vector<cuadmm::LinChunk> h_lin;
+    cuadmm::DevBuf<cuadmm::LinChunk> d_lin;
+    cudaStream_t lin_stream = nullptr;
+    cudaEvent_t lin_event = nullptr;
+    int64_t eig_len = 0;                       // sum of n over the 's' blocks: the device eigenvalue slots
     const int* done_flag = nullptr;            // device stop flag honoured by the kernels (solver)
     double last_ms = 0.0;
     int64_t last_launches = 0;

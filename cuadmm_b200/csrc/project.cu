@@ -3,6 +3,7 @@
 // and the svec<->smat kernels on the reference's pooled layout.
 #include "plan.h"
 #include <algorithm>
+#include <limits>
 #include <type_traits>
 #include <numeric>
 #include <stdlib.h>
@@ -816,6 +817,8 @@ cuadmm_plan::~cuadmm_plan() {
         if (ev0) cudaEventDestroy(ev0);
         if (ev1) cudaEventDestroy(ev1);
         if (fork_event) cudaEventDestroy(fork_event);
+        if (lin_stream) cudaStreamDestroy(lin_stream);
+        if (lin_event) cudaEventDestroy(lin_event);
         for (auto s : side_streams) cudaStreamDestroy(s);
         for (auto e : side_events) cudaEventDestroy(e);
         if (dense) dense_part_destroy(dense);
@@ -824,9 +827,12 @@ cuadmm_plan::~cuadmm_plan() {
 
 void cuadmm_plan::build_device() {
     const int64_t nblk = (int64_t)layout.blk.size();
-    // eigenvalue offsets in blk order
+    // eigenvalue offsets in blk order, over the 's' blocks (the debug entry expands them to all blocks)
     std::vector<int64_t> w_off(nblk + 1, 0);
-    for (int64_t k = 0; k < nblk; ++k) w_off[k + 1] = w_off[k] + layout.blk[k];
+    for (int64_t k = 0; k < nblk; ++k) w_off[k + 1] = w_off[k] + (layout.types[k] == 's' ? layout.blk[k] : 0);
+    eig_len = w_off[nblk];
+    // 'l' / 'u' blocks: flat chunk list of the linear-cone kernel; they take no part in the size classes below
+    h_lin = linear_chunks(layout);
 
     // classify
     const std::vector<SizeClass> table = size_classes();
@@ -835,6 +841,7 @@ void cuadmm_plan::build_device() {
     const bool large_dense = !(force_global || (large_env && !strcmp(large_env, "jacobi")));
     std::vector<int64_t> dense_blocks;
     for (int64_t k = 0; k < nblk; ++k) {
+        if (layout.types[k] != 's') continue;
         const int n = layout.blk[k];
         size_t ci = table.size();
         for (size_t c = 0; c < table.size(); ++c) if (n <= table[c].nmax) { ci = c; break; }
@@ -885,6 +892,11 @@ void cuadmm_plan::build_device() {
 
     DeviceGuard g(device);
     d_desc.upload(h_desc);
+    if (!h_lin.empty()) {
+        d_lin.upload(h_lin);
+        CUADMM_CUDA(cudaStreamCreateWithFlags(&lin_stream, cudaStreamNonBlocking));
+        CUADMM_CUDA(cudaEventCreateWithFlags(&lin_event, cudaEventDisableTiming));
+    }
     if (scratch) d_scratch.alloc(scratch);
     d_eig.alloc(std::max<int64_t>(w_off[nblk], 1));
     d_sweeps.alloc(std::max<int64_t>(nblk, 1));
@@ -950,11 +962,14 @@ int cuadmm_plan::project(const double* d_Xb, double* d_Xproj, cudaStream_t strea
     // streams so that small, mid and large blocks overlap (class 0 stays on the caller's stream when
     // there is no dense part)
     const bool has_dense = dense != nullptr;
+    const bool has_lin = !h_lin.empty();
+    // the linear-cone kernel gets its own side stream when anything else runs, else the caller's stream
+    const bool lin_side = has_lin && (has_dense || !classes.empty());
     if (rank_limit > 0) {
         if (has_dense) throw Error(CUADMM_EINVAL, "fixed-rank projection is only available for blocks n <= 168 (the sign iteration of larger blocks has no eigenvalues to rank)");
         for (const Class& cl : classes) if (cl.kind == kGlobalKind) throw Error(CUADMM_EINVAL, "fixed-rank projection is only available for blocks n <= 168");
     }
-    if (classes.size() > 1 || (has_dense && !classes.empty())) CUADMM_CUDA(cudaEventRecord(fork_event, stream));
+    if (classes.size() > 1 || (has_dense && !classes.empty()) || lin_side) CUADMM_CUDA(cudaEventRecord(fork_event, stream));
     for (size_t i = 0; i < classes.size(); ++i) {
         const Class& cl = classes[i];
         cudaStream_t st = stream;
@@ -986,9 +1001,19 @@ int cuadmm_plan::project(const double* d_Xb, double* d_Xproj, cudaStream_t strea
         ++launches;
         if (side) CUADMM_CUDA(cudaEventRecord(side_events[i], st));
     }
+    if (has_lin) {
+        cudaStream_t st = stream;
+        if (lin_side) {
+            st = lin_stream;
+            CUADMM_CUDA(cudaStreamWaitEvent(st, fork_event, 0));
+        }
+        launches += linear_project(d_lin.p, d_lin.n, d_Xb, d_Xproj, st, epi, done_flag);
+        if (lin_side) CUADMM_CUDA(cudaEventRecord(lin_event, st));
+    }
     if (has_dense) launches += dense_part_project(dense, d_Xb, d_Xproj, stream, epi, done_flag);
     for (size_t i = 0; i < classes.size(); ++i)
         if (has_dense || i > 0) CUADMM_CUDA(cudaStreamWaitEvent(stream, side_events[i], 0));
+    if (lin_side) CUADMM_CUDA(cudaStreamWaitEvent(stream, lin_event, 0));
     return launches;
 }
 
@@ -998,12 +1023,16 @@ int cuadmm_plan::project(const double* d_Xb, double* d_Xproj, cudaStream_t strea
 extern "C" {
 
 int cuadmm_plan_create(const int32_t* blk, int64_t nblk, int device, cuadmm_plan** out) {
+    return cuadmm_plan_create_typed(nullptr, blk, nblk, device, out);
+}
+
+int cuadmm_plan_create_typed(const char* types, const int32_t* blk, int64_t nblk, int device, cuadmm_plan** out) {
     return guarded([&] {
         CUADMM_REQUIRE(out != nullptr, "out is null");
         CUADMM_REQUIRE(blk != nullptr || nblk == 0, "blk is null");
         *out = nullptr;
         std::unique_ptr<cuadmm_plan> p(new cuadmm_plan());
-        p->layout.init(blk, nblk);
+        p->layout.init(blk, nblk, types);
         if (device >= 0) {
             int cnt = 0;
             cudaError_t e = cudaGetDeviceCount(&cnt);
@@ -1027,6 +1056,7 @@ int64_t cuadmm_plan_num_sizes(const cuadmm_plan* plan) { return plan ? (int64_t)
 int cuadmm_plan_sizes(const cuadmm_plan* plan, int32_t* sizes, int32_t* nums, int32_t* is_large) {
     return guarded([&] {
         CUADMM_REQUIRE(plan, "plan is null");
+        plan->layout.require_all_psd("cuadmm_plan_sizes");
         for (size_t i = 0; i < plan->layout.sizes.size(); ++i) {
             if (sizes) sizes[i] = plan->layout.sizes[i];
             if (nums) nums[i] = plan->layout.nums[i];
@@ -1039,6 +1069,7 @@ int cuadmm_plan_totals(const cuadmm_plan* plan, int64_t out[6]) {
     return guarded([&] {
         CUADMM_REQUIRE(plan && out, "null argument");
         const BlockLayout& l = plan->layout;
+        l.require_all_psd("cuadmm_plan_totals");
         out[0] = l.large_mat_num; out[1] = l.sum_large_mat_size; out[2] = l.total_large_mat_size;
         out[3] = l.small_mat_num; out[4] = l.sum_small_mat_size; out[5] = l.total_small_mat_size;
     });
@@ -1047,6 +1078,7 @@ int cuadmm_plan_totals(const cuadmm_plan* plan, int64_t out[6]) {
 int64_t cuadmm_plan_start_indices(const cuadmm_plan* plan, int which, int64_t* out) {
     if (!plan) return -1;
     const BlockLayout& l = plan->layout;
+    if (!l.all_psd()) return guarded([&] { l.require_all_psd("cuadmm_plan_start_indices"); });
     const std::vector<int64_t>* v = nullptr;
     switch (which) {
         case 0: v = &l.large_mat_start; break;
@@ -1121,6 +1153,17 @@ int cuadmm_project_psd(cuadmm_plan* plan, const double* d_Xb, double* d_Xproj, v
     });
 }
 
+int cuadmm_project_epilogue(cuadmm_plan* plan, const double* d_Xb, double* d_Xproj, const double* d_X, const double* d_Rd1,
+                            const double* d_C, double* d_S, double* d_SmC, const double* d_sig, void* stream) {
+    return guarded([&] {
+        CUADMM_REQUIRE(plan && d_Xb && d_Xproj && d_X && d_Rd1 && d_C && d_S && d_SmC && d_sig, "null argument");
+        DeviceGuard g(plan->device);
+        ProjEpilogue pe;
+        pe.X = d_X; pe.Rd1 = d_Rd1; pe.Cd = d_C; pe.S = d_S; pe.SmC = d_SmC; pe.sig_ptr = d_sig;
+        plan->last_launches = plan->project(d_Xb, d_Xproj, (cudaStream_t)stream, &pe, false);
+    });
+}
+
 static void project_host_impl(cuadmm_plan* plan, const double* h_Xb, double* h_Xproj,
                               double* h_eig, int32_t* h_sweeps) {
     CUADMM_REQUIRE(plan && h_Xb && h_Xproj, "null argument");
@@ -1133,9 +1176,24 @@ static void project_host_impl(cuadmm_plan* plan, const double* h_Xb, double* h_X
     plan->last_launches = plan->project(plan->d_in.p, plan->d_out.p, 0, nullptr, h_eig || h_sweeps);
     CUADMM_CUDA(cudaEventRecord(plan->ev1, 0));
     plan->d_out.download(h_Xproj, L);
-    if (h_eig) plan->d_eig.download(h_eig, plan->layout.sum_large_mat_size + plan->layout.sum_small_mat_size);
+    const BlockLayout& lay = plan->layout;
+    std::vector<double> eig_s;     // typed plans: the 's' blocks' slots, expanded below
+    if (h_eig) {
+        if (lay.all_psd()) plan->d_eig.download(h_eig, plan->eig_len);
+        else { eig_s.resize((size_t)plan->eig_len); plan->d_eig.download(eig_s.data(), plan->eig_len); }
+    }
     if (h_sweeps) plan->d_sweeps.download(h_sweeps, (int64_t)plan->layout.blk.size());
     CUADMM_CUDA(cudaStreamSynchronize(0));
+    if (h_eig && !lay.all_psd()) {
+        // 'l' / 'u' blocks have no eigenvalues: NaN in their n slots (their sweep counts stay 0)
+        int64_t o = 0, os = 0;
+        for (size_t k = 0; k < lay.blk.size(); ++k) {
+            const int64_t n = lay.blk[k];
+            if (lay.types[k] == 's') { std::copy(eig_s.begin() + os, eig_s.begin() + os + n, h_eig + o); os += n; }
+            else std::fill(h_eig + o, h_eig + o + n, std::numeric_limits<double>::quiet_NaN());
+            o += n;
+        }
+    }
     float ms = 0.f;
     CUADMM_CUDA(cudaEventElapsedTime(&ms, plan->ev0, plan->ev1));
     plan->last_ms = ms;
@@ -1145,7 +1203,7 @@ static void project_host_impl(cuadmm_plan* plan, const double* h_Xb, double* h_X
         // that it is too slow to be useful and the slots stay NaN).  The solver never needs eigenvalues.
         const std::vector<int32_t>& blk = plan->layout.blk;
         std::vector<int64_t> which;
-        for (size_t k = 0; k < blk.size(); ++k) if (blk[k] > 168 && blk[k] <= 1024) which.push_back((int64_t)k);
+        for (size_t k = 0; k < blk.size(); ++k) if (lay.types[k] == 's' && blk[k] > 168 && blk[k] <= 1024) which.push_back((int64_t)k);
         if (!which.empty()) {
             std::vector<int32_t> sb;
             for (int64_t k : which) sb.push_back(blk[k]);
@@ -1157,7 +1215,7 @@ static void project_host_impl(cuadmm_plan* plan, const double* h_Xb, double* h_X
                 plan->eig_plan->build_device();
             }
             cuadmm_plan* E = plan->eig_plan.get();
-            std::vector<double> xin((size_t)E->layout.vec_len), xout((size_t)E->layout.vec_len), ev((size_t)(E->layout.sum_large_mat_size + E->layout.sum_small_mat_size));
+            std::vector<double> xin((size_t)E->layout.vec_len), xout((size_t)E->layout.vec_len), ev((size_t)E->eig_len);
             for (size_t i = 0; i < which.size(); ++i)
                 std::copy(h_Xb + plan->layout.svec_off[which[i]], h_Xb + plan->layout.svec_off[which[i] + 1], xin.begin() + E->layout.svec_off[i]);
             project_host_impl(E, xin.data(), xout.data(), ev.data(), nullptr);
@@ -1174,7 +1232,7 @@ static void project_host_impl(cuadmm_plan* plan, const double* h_Xb, double* h_X
         // ascending per block, like dsyevd / Xsyevd / syevj(sort=1)
         int64_t o = 0;
         for (size_t k = 0; k < plan->layout.blk.size(); ++k) {
-            std::sort(h_eig + o, h_eig + o + plan->layout.blk[k]);
+            if (lay.types[k] == 's') std::sort(h_eig + o, h_eig + o + plan->layout.blk[k]);
             o += plan->layout.blk[k];
         }
     }
@@ -1192,6 +1250,7 @@ int cuadmm_project_psd_eig_host(cuadmm_plan* plan, const double* h_Xb, double* h
 int cuadmm_svec_to_smat(cuadmm_plan* plan, const double* d_svec, double* d_large_mat, double* d_small_mat, void* stream) {
     return guarded([&] {
         CUADMM_REQUIRE(plan && d_svec, "null argument");
+        plan->layout.require_all_psd("cuadmm_svec_to_smat");
         if (plan->device < 0) throw Error(CUADMM_ENODEVICE, "host-only plan");
         DeviceGuard g(plan->device);
         const int nblk = (int)plan->layout.blk.size();
@@ -1207,6 +1266,7 @@ int cuadmm_svec_to_smat(cuadmm_plan* plan, const double* d_svec, double* d_large
 int cuadmm_smat_to_svec(cuadmm_plan* plan, const double* d_large_mat, const double* d_small_mat, double* d_svec, void* stream) {
     return guarded([&] {
         CUADMM_REQUIRE(plan && d_svec, "null argument");
+        plan->layout.require_all_psd("cuadmm_smat_to_svec");
         if (plan->device < 0) throw Error(CUADMM_ENODEVICE, "host-only plan");
         DeviceGuard g(plan->device);
         const int nblk = (int)plan->layout.blk.size();

@@ -13,11 +13,12 @@ void Shard::build(const BlockLayout& layout, int world_, int rank_) {
     layout.partition(world, owner.data(), part_cost.data());
     vec_len = layout.vec_len;
     glob2loc.assign(vec_len, -1);
-    local_blocks.clear(); local_blk.clear(); loc2glob.clear();
+    local_blocks.clear(); local_blk.clear(); local_types.clear(); loc2glob.clear();
     for (int64_t k = 0; k < nblk; ++k) {
         if (owner[k] != rank) continue;
         local_blocks.push_back(k);
         local_blk.push_back(layout.blk[k]);
+        local_types.push_back(layout.types[k]);
         for (int64_t e = layout.svec_off[k]; e < layout.svec_off[k + 1]; ++e) {
             glob2loc[e] = (int64_t)loc2glob.size();
             loc2glob.push_back(e);
@@ -51,11 +52,15 @@ using namespace cuadmm;
 extern "C" {
 
 int cuadmm_shard_create(const int32_t* blk, int64_t nblk, int world, int rank, cuadmm_shard_t** out) {
+    return cuadmm_shard_create_typed(nullptr, blk, nblk, world, rank, out);
+}
+
+int cuadmm_shard_create_typed(const char* types, const int32_t* blk, int64_t nblk, int world, int rank, cuadmm_shard_t** out) {
     return guarded([&] {
         CUADMM_REQUIRE(out && (blk || nblk == 0), "null argument");
         *out = nullptr;
         BlockLayout layout;
-        layout.init(blk, nblk);
+        layout.init(blk, nblk, types);
         std::unique_ptr<cuadmm_shard> s(new cuadmm_shard());
         s->sh.build(layout, world, rank);
         *out = s.release();
@@ -68,6 +73,13 @@ int cuadmm_shard_info(const cuadmm_shard_t* s, int64_t out[4]) {
     return guarded([&] {
         CUADMM_REQUIRE(s && out, "null argument");
         out[0] = s->sh.vec_len_local; out[1] = (int64_t)s->sh.local_blk.size(); out[2] = s->sh.vec_len; out[3] = s->sh.world;
+    });
+}
+
+int cuadmm_shard_local_types(const cuadmm_shard_t* s, char* local_types) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s && local_types, "null argument");
+        std::copy(s->sh.local_types.begin(), s->sh.local_types.end(), local_types);
     });
 }
 

@@ -14,6 +14,7 @@ struct Shard {
     std::vector<int32_t> owner;          // per global block
     std::vector<int64_t> local_blocks;   // global block ids owned by this rank, ascending
     std::vector<int32_t> local_blk;      // their sizes
+    std::vector<char> local_types;       // their cones ('s', 'l', 'u'); a block is never split across ranks
     std::vector<int64_t> glob2loc;       // per global svec entry: local index or -1
     std::vector<int64_t> loc2glob;       // per local svec entry
     int64_t vec_len = 0, vec_len_local = 0;

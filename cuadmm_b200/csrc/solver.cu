@@ -256,15 +256,15 @@ void cuadmm_solver::init(int /*eig_stream_num_per_gpu*/, int /*cpu_eig_thread_nu
 
     // ---- block plan
     {
-        int64_t vl = 0;
-        for (int64_t k = 0; k < mat_num; ++k) { CUADMM_REQUIRE(blk[k] >= 1, "block size must be >= 1"); vl += (int64_t)blk[k] * (blk[k] + 1) / 2; }
-        CUADMM_REQUIRE(vl == vec_len, "vec_len does not match the block sizes");
+        // block cones (cuadmm_solver_set_block_types; none given: all 's'); only the plan looks at them
+        CUADMM_REQUIRE(blk_types.empty() || (int64_t)blk_types.size() == mat_num, "block types were set for a different block count");
         BlockLayout full_layout;
-        full_layout.init(blk, mat_num);
+        full_layout.init(blk, mat_num, blk_types.empty() ? nullptr : blk_types.data());   // checks sizes and letters
+        CUADMM_REQUIRE(full_layout.vec_len == vec_len, "vec_len does not match the block sizes");
         shard.build(full_layout, world, rank);      // world == 1: everything is local
         nloc = shard.vec_len_local;
         plan.reset(new cuadmm_plan());
-        plan->layout.init(shard.local_blk.data(), (int64_t)shard.local_blk.size());
+        plan->layout.init(shard.local_blk.data(), (int64_t)shard.local_blk.size(), shard.local_types.data());
         plan->device = device;
         plan->build_device();
         if (world > 1) {
@@ -853,6 +853,8 @@ int cuadmm_solver_init_from_problem(cuadmm_solver_t* s, const cuadmm_problem_t* 
     return guarded([&] {
         CUADMM_REQUIRE(s && p, "null argument");
         const Problem& q = p->prob;
+        CUADMM_REQUIRE(!s->initialised, "solver already initialised (one instance per problem, like SDPSolver)");
+        s->blk_types = q.blk_types;
         s->init(eig_stream_num_per_gpu, cpu_eig_thread_num, q.vec_len, q.con_num, q.At_csc_col_ptrs.data(), q.At_csc_row_ids.data(),
                 q.At_csc_vals.data(), q.At_nnz, q.b_indices.data(), q.b_vals.data(), q.b_nnz, q.C_indices.data(), q.C_vals.data(),
                 q.C_nnz, q.blk_vals.data(), q.mat_num, q.X_vals.empty() ? nullptr : q.X_vals.data(),
@@ -890,6 +892,18 @@ int cuadmm_solver_set_distributed(cuadmm_solver_t* s, int rank, int world, const
         CUADMM_REQUIRE(world >= 1 && rank >= 0 && rank < world, "bad rank/world");
         s->rank = rank; s->world = world;
         memcpy(s->nccl_id, id, 128);
+    });
+}
+
+int cuadmm_solver_set_block_types(cuadmm_solver_t* s, const char* types, int64_t mat_num) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s, "solver is null");
+        CUADMM_REQUIRE(!s->initialised, "set_block_types must precede init");
+        CUADMM_REQUIRE(mat_num >= 0, "mat_num < 0");
+        if (!types) { s->blk_types.clear(); return; }
+        for (int64_t k = 0; k < mat_num; ++k)
+            CUADMM_REQUIRE(valid_cone(types[k]), std::string("unknown block type '") + types[k] + "' (expected 's', 'l' or 'u')");
+        s->blk_types.assign(types, types + mat_num);
     });
 }
 

@@ -42,6 +42,7 @@ struct cuadmm_solver {
     int rank = 0, world = 1;
     char nccl_id[128] = {0};
     cuadmm::Shard shard;
+    std::vector<char> blk_types;             // block cones ('s', 'l', 'u') set before init; empty: all 's'
     // transport of the partial products: peer memory (default; kernels store into the peers' arenas, peer.h) or
     // NCCL all-reduce (CUADMM_COMM=nccl)
     bool use_peer = true;

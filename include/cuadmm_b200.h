@@ -47,11 +47,19 @@ int cuadmm_device_count(void);
 typedef struct cuadmm_plan cuadmm_plan;
 
 int  cuadmm_plan_create(const int32_t* blk, int64_t nblk, int device, cuadmm_plan** out);
+/* Typed blocks (SDPT3 blk.txt letters), one char per block: 's' PSD n x n (n(n+1)/2 svec entries), 'l' nonnegative
+ * orthant R^n_+ (n entries, projection max(x, 0)), 'u' free R^n (n entries, projection = identity, dual slack S = 0).
+ * The blocks lie contiguously in blk order in the one iterate vector.  types == NULL: every block is 's' (same plan as
+ * cuadmm_plan_create).  device = -1: host-only plan. */
+int  cuadmm_plan_create_typed(const char* types, const int32_t* blk, int64_t nblk, int device, cuadmm_plan** out);
 void cuadmm_plan_destroy(cuadmm_plan* plan);
 int64_t cuadmm_plan_vec_len(const cuadmm_plan* plan);
 int64_t cuadmm_plan_nblk(const cuadmm_plan* plan);
 
-/* analyze_blk: distinct sizes ascending, their counts, and the reference's
+/* Reference-layout helpers (cuadmm_plan_sizes / totals / start_indices / maps, cuadmm_svec_to_smat / smat_to_svec):
+ * the pooled dense layout has no place for 'l' / 'u' blocks, so on a plan that holds any they fail with CUADMM_EINVAL
+ * (cuadmm_plan_start_indices returns CUADMM_EINVAL).
+ * analyze_blk: distinct sizes ascending, their counts, and the reference's
  * large(1)/small(0) classification.  Arrays must hold cuadmm_plan_num_sizes(). */
 int64_t cuadmm_plan_num_sizes(const cuadmm_plan* plan);
 int  cuadmm_plan_sizes(const cuadmm_plan* plan, int32_t* sizes, int32_t* nums, int32_t* is_large);
@@ -79,15 +87,21 @@ int cuadmm_smat_to_svec(cuadmm_plan* plan, const double* d_large_mat,
                         const double* d_small_mat, double* d_svec, void* stream);
 
 /* --------------------------------------------------------------------------
- * PSD projection  Xproj = Pi_+(Xb), svec in -> svec out.
+ * PSD projection  Xproj = Pi_+(Xb), svec in -> svec out (typed plans: max(x, 0) on 'l' blocks, x on 'u' blocks).
  * Replaces the whole stage src/solver.cu:531-647 (vector_to_matrices, Xsyevd /
  * DsyevjBatched, max0, diag scale, gemmStridedBatched, matrices_to_vector).
  * -------------------------------------------------------------------------- */
 int cuadmm_project_psd(cuadmm_plan* plan, const double* d_Xb, double* d_Xproj, void* stream);
+/* same with the solver's fused epilogue (device pointers, d_sig one device scalar sigma):
+ *   Xproj = Pi_K(Xb),  S = (Xproj - X) / sigma - Rd1,  SmC = S - C,
+ * except on 'u' blocks, where S = 0 exactly and SmC = 0 - C (the dual cone of a free block is {0}). */
+int cuadmm_project_epilogue(cuadmm_plan* plan, const double* d_Xb, double* d_Xproj, const double* d_X, const double* d_Rd1,
+                            const double* d_C, double* d_S, double* d_SmC, const double* d_sig, void* stream);
 /* same, host buffers (H2D + kernel + D2H inside the call) */
 int cuadmm_project_psd_host(cuadmm_plan* plan, const double* h_Xb, double* h_Xproj);
 /* parity/debug: also returns per-block eigenvalues ascending, concatenated in blk
  * order (length sum n_k), and the Jacobi sweep count per block (may be NULL).
+ * 'l' / 'u' blocks: NaN in their n eigenvalue slots, 0 sweeps.
  * Blocks n <= 168: eigenvalues of the kernel that produced X.  168 < n <= 1024: X comes from the sign
  * iteration, which has no eigenvalues; they are computed by the global-memory Jacobi kernel on the same
  * input for this entry only.  n > 1024: NaN. */
@@ -174,6 +188,10 @@ int  cuadmm_solver_init(cuadmm_solver_t* s,
         const int32_t* C_indices, const double* C_vals, int64_t C_nnz,
         const int32_t* blk_vals, int64_t mat_num,
         const double* X_vals, const double* y_vals, const double* S_vals, double sig);
+/* Block cones of the problem, one letter per block ('s', 'l', 'u', see cuadmm_plan_create_typed), before init like
+ * set_device / set_distributed; init then checks vec_len against the typed entry counts.  NULL: every block is 's'.
+ * cuadmm_solver_init_from_problem takes the types of the problem instead. */
+int  cuadmm_solver_set_block_types(cuadmm_solver_t* s, const char* types, int64_t mat_num);
 int  cuadmm_solver_solve(cuadmm_solver_t* s, int max_iter, double stop_tol,
         int sig_update_threshold, int sig_update_stage_1, int sig_update_stage_2,
         int switch_admm, double sigscale, int if_first);
@@ -226,7 +244,11 @@ int  cuadmm_solver_set_device(cuadmm_solver_t* s, int device);
 /* sharding logic on its own (host only; CPU tests): */
 typedef struct cuadmm_shard cuadmm_shard_t;
 int  cuadmm_shard_create(const int32_t* blk, int64_t nblk, int world, int rank, cuadmm_shard_t** out);
+/* typed blocks (types == NULL: all 's'); a block is never split across ranks */
+int  cuadmm_shard_create_typed(const char* types, const int32_t* blk, int64_t nblk, int world, int rank, cuadmm_shard_t** out);
 void cuadmm_shard_destroy(cuadmm_shard_t* s);
+/* cones of the local blocks (cuadmm_shard_info out[1] chars) */
+int  cuadmm_shard_local_types(const cuadmm_shard_t* s, char* local_types);
 /* out[0..3] = local svec length, local block count, global svec length, world */
 int  cuadmm_shard_info(const cuadmm_shard_t* s, int64_t out[4]);
 int  cuadmm_shard_maps(const cuadmm_shard_t* s, int32_t* local_blk, int64_t* local_block_ids, int64_t* loc2glob, int32_t* owner);
@@ -252,6 +274,8 @@ int  cuadmm_solve_matlab_like(int eig_stream_num_per_gpu, int max_iter, double s
 
 /* --------------------------------------------------------------------------
  * Problem I/O: Problem::from_txt (src/problem.cu:11-83, src/utils/io.cu).
+ * blk.txt holds one block per line: "s <n>" (or a bare "<n>"), "l <n>" or "u <n>"; any other letter is rejected
+ * with CUADMM_EIO.  vec_len is the sum of the typed entry counts.
  * -------------------------------------------------------------------------- */
 typedef struct cuadmm_problem cuadmm_problem_t;
 int  cuadmm_problem_from_txt(const char* prefix, int warm_start, cuadmm_problem_t** out);
@@ -259,7 +283,8 @@ void cuadmm_problem_destroy(cuadmm_problem_t* p);
 /* out[0..6] = vec_len, con_num, mat_num, At_nnz, b_nnz, C_nnz, has_warm_start */
 int  cuadmm_problem_dims(const cuadmm_problem_t* p, int64_t out[8]);
 /* which: 0 At_csc_col_ptrs(i32) 1 At_csc_row_ids(i32) 2 At_csc_vals(f64) 3 b_indices(i32)
- * 4 b_vals(f64) 5 C_indices(i32) 6 C_vals(f64) 7 blk_vals(i32) 8 X(f64) 9 y(f64) 10 S(f64) */
+ * 4 b_vals(f64) 5 C_indices(i32) 6 C_vals(f64) 7 blk_vals(i32) 8 X(f64) 9 y(f64) 10 S(f64)
+ * 11 block types (char, mat_num letters 's' / 'l' / 'u', not NUL-terminated) */
 const void* cuadmm_problem_array(const cuadmm_problem_t* p, int which);
 int  cuadmm_solver_init_from_problem(cuadmm_solver_t* s, const cuadmm_problem_t* p,
         int eig_stream_num_per_gpu, int cpu_eig_thread_num, double sig);
