@@ -5,7 +5,6 @@
 #include <cmath>
 #include <numeric>
 #include <stdlib.h>
-#include <string.h>
 
 namespace cuadmm {
 
@@ -171,14 +170,11 @@ std::vector<int32_t> min_degree_order(const SymCsc& M) {
         }
         ++k;
     };
-    const char* mode_env = getenv("CUADMM_MD_MODE");          // "classic": one pivot per round (tuning only)
-    const bool classic = mode_env && !strcmp(mode_env, "classic");
     const char* slack_env = getenv("CUADMM_MD_SLACK");        // relative slack in percent (default 25)
     const int64_t slack_pct = slack_env ? atoll(slack_env) : 25;
     while (k < n) {
         ++round;
         while (head[mindeg] < 0) ++mindeg;
-        if (classic) { eliminate(head[mindeg]); continue; }
         const int64_t limit = std::min<int64_t>(n, mindeg + std::max<int64_t>(1, mindeg * slack_pct / 100));
         cands.clear();
         for (int64_t d = mindeg; d <= limit; ++d)

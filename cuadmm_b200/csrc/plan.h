@@ -32,7 +32,7 @@ struct cuadmm_plan {
 
     // launch classes: blocks grouped by size range, each class = one kernel launch
     struct Class {
-        int kind;          // index into the kernel table
+        int kind;          // index into kSizeClasses (project.cu), or the global-memory eigenvalue kernel (force_global)
         int nmax;          // largest n in the class
         int32_t count;     // blocks in the class
         int64_t first;     // first descriptor (in d_desc)
@@ -42,7 +42,7 @@ struct cuadmm_plan {
     std::vector<Class> classes;
     std::vector<cuadmm::BlkDesc> h_desc;       // class-major, n descending inside a class
     cuadmm::DevBuf<cuadmm::BlkDesc> d_desc;
-    cuadmm::DevBuf<double> d_scratch;          // global-memory Jacobi variant / large path
+    cuadmm::DevBuf<double> d_scratch;          // n x n per block of the global-memory eigenvalue kernel (force_global)
     cuadmm::DevBuf<double> d_eig;              // debug eigenvalue output (sum n)
     cuadmm::DevBuf<int32_t> d_sweeps;
     cuadmm::DevBuf<double> d_in, d_out;        // staging for the *_host entry points
@@ -57,10 +57,10 @@ struct cuadmm_plan {
     void reset_warm_start();
     double threshold = 1e-11;     // columns of G count as orthogonal when every |cos| <= threshold (tested on the state after each sweep)
     int max_sweeps = 40;
-    bool force_global = false;    // every block above the shared-memory classes on the global-memory Jacobi kernel (eigenvalue debug plan)
+    bool force_global = false;    // every block above the shared-memory classes on the global-memory Jacobi kernel, which yields
+                                  // eigenvalues only (the shadow plan eig_plan; never set on a plan that projects)
     std::unique_ptr<cuadmm_plan> eig_plan;   // lazily built shadow plan: eigenvalues of the blocks on the dense sign path (debug entry only)
     int rank_limit = 0;           // > 0: fixed-rank projection (cuadmm_plan_set_rank_limit)
-    bool use_gram = true;         // CUADMM_JACOBI_GRAM=0: round-1 stopping rule (a whole sweep without a cosine above the threshold)
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::vector<cudaStream_t> side_streams;    // classes run concurrently on these
     std::vector<cudaEvent_t> side_events;

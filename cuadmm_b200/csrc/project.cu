@@ -7,7 +7,6 @@
 #include <type_traits>
 #include <numeric>
 #include <stdlib.h>
-#include <string.h>
 
 namespace cuadmm {
 
@@ -104,8 +103,8 @@ __device__ __forceinline__ void jacobi_dmma(double& c0, double& c1, double a, do
 // Convergence test on the STATE of the block: are all columns of G mutually orthogonal to `thr` (relative)?
 // The Gram matrix G^T G is formed 8 x 8 tile by tile on the FP64 tensor cores (mma.sync.m8n8k4: n^3/2 MACs in
 // n^3/512 warp instructions — about 2 % of one sweep) and every off-diagonal entry is held against the tracked squared
-// norms w[].  Testing the state after a sweep, instead of the cosines met during the next one, saves the whole
-// verification sweep the rotation loop used to end with (1 of ~3 in the warm-started regime).
+// norms w[].  Testing the state after a sweep, instead of the cosines met during the next one, saves a whole
+// verification sweep (1 of ~3 in the warm-started regime).
 // Entries below 1e-15 in absolute value (G has norm ~1) are rounding noise of null columns and never count.
 template <int NT, bool WARP>
 __device__ __forceinline__ bool jacobi_gram_converged(const double* G, const double* w, int n, int ld, double thr2, int tid) {
@@ -330,7 +329,7 @@ __global__ void __launch_bounds__(T, jacobi_min_ctas(T)) proj_jacobi_kernel(Proj
     // (A "quadratic" early stop -- declare convergence after a sweep that only saw small cosines --
     // is NOT safe: inside a cluster of equal eigenvalues the rotation angle is O(1) however small the
     // cosine, and drags not-yet-visited inner products into pairs already done.  Measured: 1.6e-9
-    // error on +-1 spectra.  So the loop ends on a sweep in which nothing exceeded the threshold.)
+    // error on +-1 spectra.  So the loop ends when the Gram test finds every pair of the state orthogonal.)
     const double thr2 = a.threshold * a.threshold;
     const double tiny2 = 1.2325951644078309e-32;  // 2^-106: rotations below rounding level are skipped
     int sweeps = 0;
@@ -346,9 +345,8 @@ __global__ void __launch_bounds__(T, jacobi_min_ctas(T)) proj_jacobi_kernel(Proj
             if (lane == 0) w[j] = al;
         }
         mat_sync<WARP>();
-        if (a.use_gram && jacobi_gram_converged<NT, WARP>(G, w, n, ld, thr2, tid)) { converged = true; break; }
+        if (jacobi_gram_converged<NT, WARP>(G, w, n, ld, thr2, tid)) { converged = true; break; }
         if (sweeps >= a.max_sweeps) break;
-        int big = 0;
         // The row loops are unrolled and the columns of a pair live in registers, so their trip count is a compile-time
         // constant; a block smaller than its class's largest (n = 36 in the class up to 48) would issue the predicated
         // row steps of the largest one.  Four instantiations per kernel, picked by the block's own row count.
@@ -380,7 +378,6 @@ __global__ void __launch_bounds__(T, jacobi_min_ctas(T)) proj_jacobi_kernel(Proj
     #pragma unroll
                     for (int o = L / 2; o > 0; o >>= 1) ga += __shfl_xor_sync(gmask, ga, o);
                     const double g2 = ga * ga, ab = al * be;
-                    if (g2 > thr2 * ab) big = 1;
                     if (g2 > tiny2 * ab) {
                         double c, sn, an, bn;
                         jacobi_cs2(al, be, ga, c, sn, an, bn);
@@ -407,11 +404,6 @@ __global__ void __launch_bounds__(T, jacobi_min_ctas(T)) proj_jacobi_kernel(Proj
             else run_steps(std::integral_constant<int, RPL>{});
         }
         ++sweeps;
-        if (!a.use_gram) {
-            // rule of round 1: stop after a sweep that met no cosine above the threshold
-            const int any_big = WARP ? __any_sync(0xffffffffu, big) : __syncthreads_or(big);
-            if (!any_big) { converged = true; break; }
-        }
     }
 
     // ---- eigenvalues from the column norms; weights of the positive part ----
@@ -555,13 +547,13 @@ __global__ void __launch_bounds__(T, jacobi_min_ctas(T)) proj_jacobi_kernel(Proj
 }
 
 // ------------------------------------------------------------------------------------------
-// global-memory variant for n > 168 (G lives in HBM/L2): same algorithm, one CTA of 1024
-// threads per block, one warp per column pair, rows streamed twice (dot, then update).
-// Correct for any n; the dense tridiagonal path supersedes it for large n.
+// eigenvalues of blocks n > 168 for the debug entry cuadmm_project_psd_eig_host (their projection is the
+// dense sign path's, which has none): the same shifted one-sided Jacobi with G in HBM/L2, one CTA of
+// 1024 threads per block, one warp per column pair, rows streamed twice (dot, then update).
+// Writes eigenvalues and sweep counts only.
 // ------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) proj_jacobi_global_kernel(ProjArgs a) {
     __shared__ double red[34];
-    __shared__ int s_k;
     const int tid = threadIdx.x;
     const int bi = blockIdx.x;
     if (bi >= a.nblk) return;
@@ -569,12 +561,8 @@ __global__ void __launch_bounds__(1024) proj_jacobi_global_kernel(ProjArgs a) {
     const BlkDesc d = a.desc[bi];
     const int n = d.n;
     const int64_t ld = n;
-    const int64_t ntri = (int64_t)n * (n + 1) / 2;
     double* G = a.scratch + d.scratch_off;          // n*n
-    double* w = G + (int64_t)n * n;                 // n
-    int* pos = (int*)(w + n);                       // n+1 ints
     const double* __restrict__ xin = a.Xb + d.svec_off;
-    double* __restrict__ xout = a.Xproj + d.svec_off;
 
     double f2 = 0.0;
     for (int c = 0; c < n; ++c) {
@@ -591,16 +579,6 @@ __global__ void __launch_bounds__(1024) proj_jacobi_global_kernel(ProjArgs a) {
     const double s = sqrt(f2);
     if (!(s >= 1e-290)) {
         const double fill = (s == s) ? 0.0 : s;
-        for (int64_t idx = tid; idx < ntri; idx += 1024) {
-            xout[idx] = fill;
-            if (a.epi.X) {
-                const int64_t gi = d.svec_off + idx;
-                const double sig = *a.epi.sig_ptr;
-                const double Sv = (fill - a.epi.X[gi]) / sig - a.epi.Rd1[gi];
-                a.epi.S[gi] = Sv;
-                a.epi.SmC[gi] = Sv - a.epi.Cd[gi];
-            }
-        }
         if (tid == 0 && a.sweeps_out) a.sweeps_out[d.index] = 0;
         if (a.eig_out) for (int j = tid; j < n; j += 1024) a.eig_out[d.w_off + j] = fill;
         return;
@@ -660,48 +638,9 @@ __global__ void __launch_bounds__(1024) proj_jacobi_global_kernel(ProjArgs a) {
         for (int r = lane; r < n; r += 32) al = fma(Gj[r], Gj[r], al);
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) al += __shfl_xor_sync(0xffffffffu, al, o);
-        if (lane == 0) {
-            const double sigma = sqrt(al);
-            const double lam = s * (sigma - 1.0);
-            w[j] = (sigma > 1.0) ? sqrt(lam / al) : 0.0;
-            if (a.eig_out) a.eig_out[d.w_off + j] = lam;
-        }
+        if (lane == 0 && a.eig_out) a.eig_out[d.w_off + j] = s * (sqrt(al) - 1.0);
     }
-    __syncthreads();
-    if (tid == 0) {
-        int k = 0;
-        for (int j = 0; j < n; ++j) if (w[j] > 0.0) pos[k++] = j;
-        s_k = k;
-        if (a.sweeps_out) a.sweeps_out[d.index] = sweeps;
-    }
-    __syncthreads();
-    const int kpos = s_k;
-    for (int64_t e = tid; e < (int64_t)kpos * n; e += 1024) {
-        const int jj = (int)(e / n), r = (int)(e - (int64_t)jj * n);
-        const int j = pos[jj];
-        G[r + j * ld] *= w[j];
-    }
-    __syncthreads();
-    double sig = 1.0;
-    if (a.epi.X) sig = *a.epi.sig_ptr;
-    for (int c = 0; c < n; ++c) {
-        const int64_t base = (int64_t)c * (c + 1) / 2;
-        for (int r = tid; r <= c; r += 1024) {
-            double acc = 0.0;
-            for (int jj = 0; jj < kpos; ++jj) {
-                const double* Gj = G + pos[jj] * ld;
-                acc = fma(Gj[r], Gj[c], acc);
-            }
-            const double out = (r == c) ? acc : acc * CUADMM_SQRT2;
-            xout[base + r] = out;
-            if (a.epi.X) {
-                const int64_t gi = d.svec_off + base + r;
-                const double Sv = (out - a.epi.X[gi]) / sig - a.epi.Rd1[gi];
-                a.epi.S[gi] = Sv;
-                a.epi.SmC[gi] = Sv - a.epi.Cd[gi];
-            }
-        }
-    }
+    if (tid == 0 && a.sweeps_out) a.sweeps_out[d.index] = sweeps;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -743,68 +682,36 @@ __global__ void smat_to_svec_kernel(const double* __restrict__ large_mat, const 
 }
 
 // ------------------------------------------------------------------------------------------
-// kernel variants and size classes
+// size classes
 // ------------------------------------------------------------------------------------------
-struct Variant {
-    int nmax_allowed;   // L * RPL rows, and the shared-memory limit
+// A block of n <= nmax runs on the first class that admits it, on proj_jacobi_kernel<T, L, RPL, WARP> with
+// L * RPL >= nmax.  The table is the tuning sweep's result (profiles/jacobi_tuning_r01.md); retuning means
+// instantiating candidate configurations again and timing them.
+struct SizeClass {
+    int nmax;           // largest n of the class; sizes the shared memory
     int threads;
     int L;
     int mats_per_cta;
     void (*fn)(ProjArgs, int);
 };
 
-#define CUADMM_VARIANT(T, L, RPL, WARP) {((L) * (RPL) > 168 ? 168 : (L) * (RPL)), T, L, (WARP) ? (T) / 32 : 1, proj_jacobi_kernel<T, L, RPL, WARP>}
-static const Variant kVariants[] = {
-    /* 0*/ CUADMM_VARIANT(128, 4, 4, true),
-    /* 1*/ CUADMM_VARIANT(64, 4, 8, false),
-    /* 2*/ CUADMM_VARIANT(128, 8, 4, false),
-    /* 3*/ CUADMM_VARIANT(128, 4, 16, false),
-    /* 4*/ CUADMM_VARIANT(256, 8, 8, false),
-    /* 5*/ CUADMM_VARIANT(512, 16, 4, false),
-    /* 6*/ CUADMM_VARIANT(384, 8, 12, false),
-    /* 7*/ CUADMM_VARIANT(768, 16, 6, false),
-    /* 8*/ CUADMM_VARIANT(512, 8, 16, false),
-    /* 9*/ CUADMM_VARIANT(1024, 16, 8, false),
-    /*10*/ CUADMM_VARIANT(672, 16, 11, false),
-    /*11*/ CUADMM_VARIANT(192, 4, 24, false),
-    /*12*/ CUADMM_VARIANT(256, 4, 32, false),
-    /*13*/ CUADMM_VARIANT(352, 8, 21, false),
-    /*14*/ CUADMM_VARIANT(256, 8, 4, true),
-    /*15*/ CUADMM_VARIANT(128, 8, 8, false),
-    /*16*/ CUADMM_VARIANT(128, 4, 12, false),
+#define CUADMM_CLASS(NMAX, T, L, RPL, WARP) {NMAX, T, L, (WARP) ? (T) / 32 : 1, proj_jacobi_kernel<T, L, RPL, WARP>}
+// (a separate class for 33..48 on 12 rows per lane was 3 % faster before the sweep was instantiated per row count, and
+// slower after: more distinct kernels running side by side)
+static const SizeClass kSizeClasses[] = {
+    CUADMM_CLASS(16, 128, 4, 4, true),
+    CUADMM_CLASS(32, 64, 4, 8, false),
+    CUADMM_CLASS(64, 128, 4, 16, false),
+    CUADMM_CLASS(96, 192, 4, 24, false),
+    CUADMM_CLASS(128, 512, 8, 16, false),
+    CUADMM_CLASS(168, 352, 8, 21, false),
 };
-static const int kNumVariants = (int)(sizeof(kVariants) / sizeof(kVariants[0]));
+static const int kNumSizeClasses = (int)(sizeof(kSizeClasses) / sizeof(kSizeClasses[0]));
+// Class::kind of the blocks above every size class in a force_global plan
 static const int kGlobalKind = -1;
 
-// size class = (largest n, variant).  Default table from the tuning sweep in
-// profiles/jacobi_tuning_r01.md; CUADMM_JACOBI_CLASSES="16:0,32:1,..." overrides it (tuning only).
-struct SizeClass { int nmax; int variant; };
-static std::vector<SizeClass> size_classes() {
-    // (a separate class for 33..48 on 12 rows per lane was 3 % faster before the sweep was instantiated per row count, and
-    // slower after: more distinct kernels running side by side)
-    std::vector<SizeClass> t = {{16, 0}, {32, 1}, {64, 3}, {96, 11}, {128, 8}, {168, 13}};
-    const char* env = getenv("CUADMM_JACOBI_CLASSES");
-    if (env && *env) {
-        std::vector<SizeClass> u;
-        const char* q = env;
-        while (*q) {
-            char* end = nullptr;
-            long nm = strtol(q, &end, 10);
-            if (end == q || *end != ':') break;
-            q = end + 1;
-            long v = strtol(q, &end, 10);
-            if (end == q) break;
-            if (v >= 0 && v < kNumVariants && nm >= 1 && nm <= kVariants[v].nmax_allowed) u.push_back({(int)nm, (int)v});
-            q = (*end == ',') ? end + 1 : end;
-            if (*end != ',') break;
-        }
-        if (!u.empty()) t = u;
-    }
-    return t;
-}
-
-static size_t smem_bytes(int nmax, const Variant& v) {
-    return jacobi_per_mat(nmax, v.L) * sizeof(double) * v.mats_per_cta;
+static size_t smem_bytes(int nmax, const SizeClass& sc) {
+    return jacobi_per_mat(nmax, sc.L) * sizeof(double) * sc.mats_per_cta;
 }
 
 }  // namespace cuadmm
@@ -835,17 +742,14 @@ void cuadmm_plan::build_device() {
     h_lin = linear_chunks(layout);
 
     // classify
-    const std::vector<SizeClass> table = size_classes();
-    std::vector<std::vector<int64_t>> members(table.size() + 1);
-    const char* large_env = getenv("CUADMM_LARGE");           // "jacobi": global-memory Jacobi for n > 168 (debug)
-    const bool large_dense = !(force_global || (large_env && !strcmp(large_env, "jacobi")));
+    std::vector<std::vector<int64_t>> members(kNumSizeClasses + 1);
     std::vector<int64_t> dense_blocks;
     for (int64_t k = 0; k < nblk; ++k) {
         if (layout.types[k] != 's') continue;
         const int n = layout.blk[k];
-        size_t ci = table.size();
-        for (size_t c = 0; c < table.size(); ++c) if (n <= table[c].nmax) { ci = c; break; }
-        if (ci == table.size() && large_dense) { dense_blocks.push_back(k); continue; }
+        int ci = kNumSizeClasses;
+        for (int c = 0; c < kNumSizeClasses; ++c) if (n <= kSizeClasses[c].nmax) { ci = c; break; }
+        if (ci == kNumSizeClasses && !force_global) { dense_blocks.push_back(k); continue; }
         members[ci].push_back(k);
     }
     if (dense) { dense_part_destroy(dense); dense = nullptr; }
@@ -853,12 +757,12 @@ void cuadmm_plan::build_device() {
     h_desc.clear(); classes.clear();
     int64_t scratch = 0, q_total = 0;
     // heaviest classes first so their launches start first
-    for (int ci = (int)table.size(); ci >= 0; --ci) {
+    for (int ci = kNumSizeClasses; ci >= 0; --ci) {
         auto& mem = members[ci];
         if (mem.empty()) continue;
         std::stable_sort(mem.begin(), mem.end(), [&](int64_t a, int64_t b) { return layout.blk[a] > layout.blk[b]; });
         Class cl;
-        cl.kind = (ci == (int)table.size()) ? kGlobalKind : table[ci].variant;
+        cl.kind = (ci == kNumSizeClasses) ? kGlobalKind : ci;
         cl.nmax = layout.blk[mem[0]];
         cl.count = (int32_t)mem.size();
         cl.first = (int64_t)h_desc.size();
@@ -866,9 +770,9 @@ void cuadmm_plan::build_device() {
             cl.smem = 0;
             cl.grid = cl.count;
         } else {
-            const Variant& v = kVariants[cl.kind];
-            cl.smem = smem_bytes(cl.nmax, v);
-            cl.grid = (cl.count + v.mats_per_cta - 1) / v.mats_per_cta;
+            const SizeClass& sc = kSizeClasses[cl.kind];
+            cl.smem = smem_bytes(cl.nmax, sc);
+            cl.grid = (cl.count + sc.mats_per_cta - 1) / sc.mats_per_cta;
         }
         for (int64_t k : mem) {
             BlkDesc d;
@@ -879,11 +783,7 @@ void cuadmm_plan::build_device() {
             d.scratch_off = 0;
             d.q_off = 0;
             if (cl.kind != kGlobalKind) { d.q_off = q_total; q_total += (int64_t)d.n * d.n; }
-            if (cl.kind == kGlobalKind) {
-                d.scratch_off = scratch;
-                const int64_t n = d.n;
-                scratch += n * n + n + (n + 2) / 2 + 1;
-            }
+            else { d.scratch_off = scratch; scratch += (int64_t)d.n * d.n; }
             h_desc.push_back(d);
         }
         classes.push_back(cl);
@@ -902,7 +802,6 @@ void cuadmm_plan::build_device() {
     d_sweeps.alloc(std::max<int64_t>(nblk, 1));
     warm_start = true;
     if (const char* e = getenv("CUADMM_JACOBI_WARM")) warm_start = atoi(e) != 0;
-    if (const char* e = getenv("CUADMM_JACOBI_GRAM")) use_gram = atoi(e) != 0;
     if (const char* e = getenv("CUADMM_JACOBI_THR")) { const double v = atof(e); if (v > 0.0 && v < 1e-3) threshold = v; }
     if (warm_start && q_total > 0) {
         d_Q.alloc(q_total);
@@ -923,8 +822,8 @@ void cuadmm_plan::build_device() {
     }
     for (const Class& cl : classes) {
         if (cl.kind == kGlobalKind) continue;
-        CUADMM_CUDA(cudaFuncSetAttribute((const void*)kVariants[cl.kind].fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         (int)smem_bytes(kVariants[cl.kind].nmax_allowed, kVariants[cl.kind])));
+        const SizeClass& sc = kSizeClasses[cl.kind];
+        CUADMM_CUDA(cudaFuncSetAttribute((const void*)sc.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes(sc.nmax, sc)));
     }
     CUADMM_CUDA(cudaDeviceSynchronize());
 }
@@ -967,7 +866,6 @@ int cuadmm_plan::project(const double* d_Xb, double* d_Xproj, cudaStream_t strea
     const bool lin_side = has_lin && (has_dense || !classes.empty());
     if (rank_limit > 0) {
         if (has_dense) throw Error(CUADMM_EINVAL, "fixed-rank projection is only available for blocks n <= 168 (the sign iteration of larger blocks has no eigenvalues to rank)");
-        for (const Class& cl : classes) if (cl.kind == kGlobalKind) throw Error(CUADMM_EINVAL, "fixed-rank projection is only available for blocks n <= 168");
     }
     if (classes.size() > 1 || (has_dense && !classes.empty()) || lin_side) CUADMM_CUDA(cudaEventRecord(fork_event, stream));
     for (size_t i = 0; i < classes.size(); ++i) {
@@ -988,14 +886,13 @@ int cuadmm_plan::project(const double* d_Xb, double* d_Xproj, cudaStream_t strea
         a.sweeps_out = want_eig ? d_sweeps.p : nullptr;
         a.scratch = d_scratch.p;
         a.done_flag = done_flag;
-        a.use_gram = use_gram ? 1 : 0;
         a.rank_limit = rank_limit;
         a.Q = (warm_start && cl.kind != kGlobalKind && d_Q.n > 0) ? d_Q.p : nullptr;
         if (epi) a.epi = *epi; else { a.epi.X = nullptr; a.epi.Rd1 = nullptr; a.epi.Cd = nullptr; a.epi.S = nullptr; a.epi.SmC = nullptr; a.epi.sig_ptr = nullptr; }
         if (cl.kind == kGlobalKind) {
             proj_jacobi_global_kernel<<<cl.grid, 1024, 0, st>>>(a);
         } else {
-            kVariants[cl.kind].fn<<<cl.grid, kVariants[cl.kind].threads, cl.smem, st>>>(a, cl.nmax);
+            kSizeClasses[cl.kind].fn<<<cl.grid, kSizeClasses[cl.kind].threads, cl.smem, st>>>(a, cl.nmax);
         }
         CUADMM_CUDA(cudaGetLastError());
         ++launches;

@@ -59,13 +59,12 @@ struct ProjArgs {
     double* Xproj;
     const BlkDesc* desc;
     int32_t nblk;           // blocks in this launch
-    double threshold;       // converged when max |cos| seen in a sweep <= threshold
+    double threshold;       // converged when every |cos| between two columns <= threshold
     int32_t max_sweeps;
     double* eig_out;        // optional (null): eigenvalues, unsorted, at desc.w_off
     int32_t* sweeps_out;    // optional (null): sweeps used, at desc.index
-    double* scratch;        // global variant
+    double* scratch;        // global-memory eigenvalue kernel
     const int* done_flag;   // optional device flag: kernels return at once when *done_flag != 0
-    int use_gram;           // 1: convergence tested on the state after each sweep (Gram matrix on the tensor cores)
     int rank_limit;         // > 0: fixed-rank projection, only the rank_limit largest eigenvalues survive the clamp
     double* Q;              // optional (null): warm-start bases, n x n column-major at desc.q_off, read AND updated
     ProjEpilogue epi;

@@ -272,8 +272,7 @@ void cuadmm_solver::init(int /*eig_stream_num_per_gpu*/, int /*cpu_eig_thread_nu
             if (const char* c = getenv("CUADMM_COMM")) use_peer = strcmp(c, "nccl") != 0;
             // the collectives are captured into the iteration graph with the kernels (measured on 2 GPUs: 672 ->
             // 857 iter/s on the bench workload; without it the host cannot enqueue ~40 launches per 1.2 ms iteration
-            // fast enough); CUADMM_DIST_GRAPH=0 enqueues them directly
-            if (const char* dg = getenv("CUADMM_DIST_GRAPH")) { if (atoi(dg) == 0) use_graphs = false; }
+            // fast enough)
         }
     }
     // ---- A: normalise the constraints (get_normA, src/solver.cu:79-80), same arithmetic

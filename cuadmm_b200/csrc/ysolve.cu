@@ -755,8 +755,6 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
     };
     std::vector<Packed> packs, blobs;
     std::vector<int32_t> loc(H.n, -1), cidx(H.n, -1), height(H.n, 0), lvl_r(H.n, 0);
-    bool use_packed = true;
-    if (const char* e = getenv("CUADMM_SWEEP_PACKED")) use_packed = atoi(e) != 0;
     int chain_max = kPkChainMax, chain_gain = 6;
     if (const char* e = getenv("CUADMM_SWEEP_CHAIN_MAX")) chain_max = std::min(atoi(e), kPkMaxRowEntries);
     const bool verbose = getenv("CUADMM_YSOLVE_VERBOSE") != nullptr;
@@ -765,7 +763,7 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
     auto same = [&](int32_t u, int64_t p) { return H.sub[H.dep[p]] == H.sub[u]; };
     // one subtree at a time, on a pool of host threads: subtrees own disjoint rows of the scratch arrays (loc, cidx, height,
     // lvl_r), results land in per-subtree slots and are collected in subtree order afterwards (deterministic layout)
-    std::vector<Packed> result(use_packed ? H.n_sub : 0);
+    std::vector<Packed> result(H.n_sub);
     std::atomic<int64_t> a_collapsed{0}, a_before{0}, a_after{0}, a_entries{0};
     auto do_subtree = [&](int64_t t) {
         const std::vector<int32_t>& rows = members[t];       // in solve order
@@ -965,7 +963,7 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
             kind[t] = 2;
         }
     };
-    if (use_packed && H.n_sub > 0) {
+    if (H.n_sub > 0) {
         int nthreads = (int)std::min<int64_t>(std::max(1u, std::thread::hardware_concurrency()), 32);
         if (const char* e = getenv("CUADMM_INIT_THREADS")) nthreads = std::max(1, atoi(e));
         nthreads = (int)std::min<int64_t>(nthreads, H.n_sub);
@@ -1354,11 +1352,6 @@ cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const in
     CUADMM_CUDA(cudaEventCreateWithFlags(&Y->streams.fork, cudaEventDisableTiming));
     CUADMM_CUDA(cudaEventCreateWithFlags(&Y->streams.join, cudaEventDisableTiming));
     Y->alg_bytes = 2 * (12 * Y->nnz_L + 8 * m) + 24 * m;
-    if (const char* e = getenv("CUADMM_TAIL_SIM_WORLD")) {
-        Y->sim_world = atoi(e);
-        const char* r = getenv("CUADMM_TAIL_SIM_RANK");
-        if (Y->sim_world > 1 && n_tail > 0) Y->split_tail_rows(Y->sim_world, r ? atoi(r) : 0);
-    }
     CUADMM_CUDA(cudaDeviceSynchronize());
     return Y.release();
 }
@@ -1432,14 +1425,7 @@ void cuadmm_ysolve_s::solve(const double* d_rhs_, double* d_y_, cudaStream_t st)
     if (n_tail > 0) {
         mark(20);
         // x_tail = L22^-T L22^-1 z_tail, scattered into y
-        if (sim_world > 1 && !peer) {
-            // measurement only (CUADMM_TAIL_SIM_WORLD=W, CUADMM_TAIL_SIM_RANK=r): the rows rank r of W would compute,
-            // no exchange — the result is incomplete, the timing is that of one rank's share
-            const int64_t n0 = tail_row1[0] - tail_row0[0], n1 = tail_row1[1] - tail_row0[1];
-            gemv_split(tail_inv.p, z.p + n_lead, tmpv, tail_tptr.p, tail_tcol.p, 1, tail_row0[0], n0, 0, PeerView(), PeerPtrs());
-            gemv_split(tail_inv_t.p, tmpv, xv + n_lead, tail_tptr_t.p, tail_tcol_t.p, 0, tail_row0[1], n1, 0, PeerView(), PeerPtrs());
-            tail_scatter_kernel<<<(int)((n_tail + 255) / 256), 256, 0, st>>>(n_tail, xv + n_lead, perm.p, n_lead, d_y_, done_flag);
-        } else if (!peer || peer->world == 1) {
+        if (!peer || peer->world == 1) {
             const int blocks = (int)((n_tail + 7) / 8);
             // whole matrix on one GPU: row per warp streams at 69 % of the HBM peak (ncu), the split-column kernel at 55 %
             tail_gemv_row_kernel<<<blocks, 256, 0, st>>>(n_tail, tail_inv.p, z.p + n_lead, tmpv, tail_tptr.p, tail_tcol.p,

@@ -76,7 +76,6 @@ struct cuadmm_ysolve_s {
     std::vector<double> h_tail_cost[2]; // per 64-row tile row: columns read (work per row)
     void enable_peer(const cuadmm::PeerComm* pc, size_t off_tmp, size_t off_x);
     void split_tail_rows(int world, int rank);
-    int sim_world = 0;                  // measurement only: CUADMM_TAIL_SIM_WORLD
     cuadmm::DevBuf<double> split_part;  // split-column GEMV: partial sums per (row block, split)
     cuadmm::DevBuf<unsigned int> split_count;
     const int* done_flag = nullptr;

@@ -1,6 +1,6 @@
 """Projection-stage time and Jacobi sweep counts in the regime the solver runs in: a sequence of slowly drifting
-inputs (successive ADMM iterates), C2b block mix, warm-started plan.  Environment selects the build / rule under
-test (CUADMM_LIB_PATH, CUADMM_JACOBI_GRAM, CUADMM_JACOBI_THR).  One JSON line."""
+inputs (successive ADMM iterates), C2b block mix, warm-started plan.  Environment selects the build / threshold under
+test (CUADMM_LIB_PATH, CUADMM_JACOBI_THR).  One JSON line."""
 import json, os, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -11,7 +11,7 @@ from cuadmm_b200.synthetic import c2b_blocks, random_svec
 import oracle_np as onp
 blk = c2b_blocks(2000, 6, 60, 0)
 x = random_svec(blk, seed=0); d = random_svec(blk, seed=1)
-out = {"lib": os.environ.get("CUADMM_LIB_PATH", "default"), "gram": os.environ.get("CUADMM_JACOBI_GRAM", "1"),
+out = {"lib": os.environ.get("CUADMM_LIB_PATH", "default"),
        "thr": os.environ.get("CUADMM_JACOBI_THR", "default"), "drift": {}}
 for drift in [1e-1, 1e-2, 1e-3, 1e-4, 1e-6, 0.0]:
     p = cu.Plan(blk, device=0); q = cu.Plan(blk, device=0)

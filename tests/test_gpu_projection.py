@@ -104,16 +104,6 @@ def test_large_blocks_degenerate_spectra():
         assert np.linalg.norm(a - b) <= 1e-9 * max(np.linalg.norm(b), 1e-3 * np.linalg.norm(xin)) + 1e-300, k
 
 
-def test_global_memory_jacobi_variant(monkeypatch):
-    monkeypatch.setenv("CUADMM_LARGE", "jacobi")
-    blk = np.array([200], np.int32)
-    x = random_svec(blk, seed=200)
-    out, eig, sweeps = cu.Plan(blk).project_eig_host(x)
-    ref, reig = onp.project_svec(blk, x, want_eig=True)
-    assert np.linalg.norm(out - ref) <= 1e-9 * np.linalg.norm(ref)
-    assert np.abs(eig - reig).max() <= 1e-10 * np.abs(reig).max()
-
-
 def test_mixed_blocks_planarhand_layout():
     blk = np.loadtxt(os.path.join(ROOT, "tests", "golden", "planarhand_n1_blk.txt"), dtype=np.int32)
     _check(blk, random_svec(blk, seed=0))
