@@ -347,6 +347,7 @@ _maybe("cuadmm_solver_get_X", C.c_int, vp, c_f64p)
 _maybe("cuadmm_solver_get_y", C.c_int, vp, c_f64p)
 _maybe("cuadmm_solver_get_S", C.c_int, vp, c_f64p)
 _maybe("cuadmm_solver_set_XyS", C.c_int, vp, c_f64p, c_f64p, c_f64p, C.c_double)
+_maybe("cuadmm_solver_update_data", C.c_int, vp, c_i32p, c_f64p, C.c_int64, c_i32p, c_f64p, C.c_int64, C.c_int, C.c_double)
 _maybe("cuadmm_solver_iter_num", C.c_int64, vp)
 _maybe("cuadmm_solver_history", C.c_int, vp, C.c_int, c_f64p, C.c_int64)
 _maybe("cuadmm_solver_times", C.c_int, vp, c_f64p)
@@ -563,7 +564,7 @@ class Solver:
     def times(self):
         t = np.zeros(8)
         _check(lib.cuadmm_solver_times(self.h, _p(t, c_f64p)))
-        return dict(total=t[0], init=t[1], solve=t[2], projection=t[3], ysolve=t[4], spmv=t[5])
+        return dict(total=t[0], init=t[1], solve=t[2], projection=t[3], ysolve=t[4], spmv=t[5], update=t[6])
 
     @property
     def launches(self):
@@ -585,6 +586,23 @@ class Solver:
     def set_XyS(self, X, y, S, sig):
         X, y, S = _f64(X), _f64(y), _f64(S)
         _check(lib.cuadmm_solver_set_XyS(self.h, _p(X, c_f64p), _p(y, c_f64p), _p(S, c_f64p), float(sig)))
+
+    def update_data(self, b_idx, b_val, C_idx, C_val, keep_iterate=False, sig=1.0):
+        """New b and C (sparse triplets, as in init) for the same A and blocks, keeping the factorisation, the projection
+        plan and the iteration graphs; follow with solve(..., if_first=True).  keep_iterate=False: the next solve is
+        that of a fresh init with these b, C and sig; True: it starts from the X, y, S the last solve returned."""
+        arrs = []
+        for name, idx, val in (("b", b_idx, b_val), ("C", C_idx, C_val)):
+            i, v = np.asarray(idx), np.asarray(val)
+            if i.ndim != 1 or v.ndim != 1 or len(i) != len(v):
+                raise ValueError(f"{name}: indices and values must be 1-D of one length, got shapes {i.shape} and {v.shape}")
+            if len(i) and (not np.issubdtype(i.dtype, np.integer) or i.min() < np.iinfo(np.int32).min
+                           or i.max() > np.iinfo(np.int32).max):
+                raise ValueError(f"{name}: indices must be int32 integers")
+            arrs += [_i32(i), _f64(v)]
+        bi, bv, ci, cv = arrs
+        _check(lib.cuadmm_solver_update_data(self.h, _p(bi, c_i32p), _p(bv, c_f64p), len(bv), _p(ci, c_i32p),
+                                             _p(cv, c_f64p), len(cv), int(bool(keep_iterate)), float(sig)))
 
     def get_into(self, X, y, S):
         """D2H of X, y, S into caller-provided (e.g. pinned) arrays"""

@@ -190,6 +190,80 @@ __global__ void scatter_full_kernel(int64_t nloc, const double* __restrict__ loc
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nloc; i += (int64_t)gridDim.x * blockDim.x) full[loc2glob[i]] = local[i];
 }
 
+// ---- update_data: new b and C on the device
+// triplets -> zeroed dense vector with init's rule for repeated indices (the last triplet wins):
+// pass 1 marks the last triplet of every entry (win starts at -1), pass 2 stores only that one
+__global__ void triplet_mark_kernel(int32_t nnz, const int32_t* __restrict__ idx, int32_t* win) {
+    for (int32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < nnz; k += gridDim.x * blockDim.x) atomicMax(win + idx[k], k);
+}
+__global__ void triplet_store_kernel(int32_t nnz, const int32_t* __restrict__ idx, const double* __restrict__ val,
+                                     const int32_t* __restrict__ win, double* out) {
+    for (int32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < nnz; k += gridDim.x * blockDim.x)
+        if (win[idx[k]] == k) out[idx[k]] = val[k];
+}
+// per-CTA partial pair (sum x^2, sum (x ./ d)^2), the second 0 when d is null; fixed tree inside the CTA
+__global__ void __launch_bounds__(kEwThreads) sumsq_kernel(int64_t n, const double* __restrict__ x, const double* __restrict__ d,
+                                                           double* partial) {
+    __shared__ double red[2][kEwThreads / 32];
+    double a0 = 0.0, a1 = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
+        const double v = x[i];
+        a0 = fma(v, v, a0);
+        if (d) { const double t = v / d[i]; a1 = fma(t, t, a1); }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
+    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a0; red[1][threadIdx.x >> 5] = a1; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double s0 = 0.0, s1 = 0.0;
+        for (int k = 0; k < kEwThreads / 32; ++k) { s0 += red[0][k]; s1 += red[1][k]; }
+        partial[2 * blockIdx.x] = s0; partial[2 * blockIdx.x + 1] = s1;
+    }
+}
+// one CTA of 256 threads: the pairwise sums of na pairs at pa and nb pairs at pb, in scalar_update_kernel's fixed order
+__device__ __forceinline__ void sum_pairs_256(const double* __restrict__ pa, int na, const double* __restrict__ pb, int nb,
+                                              double out[4]) {
+    __shared__ double sm[4][256];
+    double v[4] = {0.0, 0.0, 0.0, 0.0};
+    for (int i = threadIdx.x; i < na; i += 256) { v[0] += pa[2 * i]; v[1] += pa[2 * i + 1]; }
+    for (int i = threadIdx.x; i < nb; i += 256) { v[2] += pb[2 * i]; v[3] += pb[2 * i + 1]; }
+    for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] = v[q];
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] += sm[q][threadIdx.x + o];
+        __syncthreads();
+    }
+    for (int q = 0; q < 4; ++q) out[q] = sm[q][0];
+}
+// the scaling constants (src/solver.cu:113-191): part_b pairs (|b|^2, |b ./ normA|^2), part_c pairs (|C|^2, 0)
+__global__ void __launch_bounds__(256) data_scales_kernel(DevState* st, const double* __restrict__ part_b, int n_b,
+                                                          const double* __restrict__ part_c, int n_c) {
+    double s[4];
+    sum_pairs_256(part_b, n_b, part_c, n_c, s);
+    if (threadIdx.x != 0) return;
+    const double nC = sqrt(s[2]);
+    st->norm_borg = 1 + sqrt(s[0]);
+    st->bscale = 1 + sqrt(s[1]);
+    st->norm_Corg = 1 + nC;
+    st->Cscale = 1 + nC;
+    st->objscale = st->bscale * st->Cscale;
+}
+// the initial residuals and objectives (src/solver.cu:193-228) from the partials of Rd (|Rd|^2, <C, X>) and Rp
+// (|normA .* Rp|^2, <b, y>), with scalar_update_kernel's formulas
+__global__ void __launch_bounds__(256) data_residuals_kernel(DevState* st, const double* __restrict__ part_rd, int n_rd,
+                                                             const double* __restrict__ part_rp, int n_rp) {
+    double s[4];
+    sum_pairs_256(part_rd, n_rd, part_rp, n_rp, s);
+    if (threadIdx.x != 0) return;
+    const double errRp = st->bscale * sqrt(s[2]) / st->norm_borg;
+    const double errRd = st->Cscale * sqrt(s[0]) / st->norm_Corg;
+    const double pobj = s[1] * st->objscale, dobj = s[3] * st->objscale;
+    st->errRp = errRp; st->errRd = errRd; st->pobj = pobj; st->dobj = dobj;
+    st->maxfeas = fmax(errRp, errRd);
+    st->relgap = fabs(pobj - dobj) / (1 + fabs(pobj) + fabs(dobj));
+}
+
 static int ew_grid(int64_t n, int device) {
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -802,6 +876,7 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     scale_vec_kernel<<<gm, 256, 0, stream>>>(m, y.p, normA.p, Cscale, 1);
     scale_kernel<<<gv, 256, 0, stream>>>(n, S.p, Cscale);
     launches += 3;
+    iterate_scaled = false;
     drain(info_iter_num);
     CUADMM_CUDA(cudaEventRecord(ev_now, stream));
     CUADMM_CUDA(cudaStreamSynchronize(stream));
@@ -820,6 +895,144 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
         printf("\n -------------------------------------------------------------------------------\n\n");
         fflush(stdout);
     }
+}
+
+// New b and C for the same A and blocks: everything init derives from b and C, recomputed on the device in place.
+// normA, both SpMV operators, the y-solve, the plan, the shard, the peer arena and the captured graphs are kept.
+// Order (fixed by the data): scatter b, C -> norms -> scales (read back: solve() scales with host copies) -> scaled
+// b, C and the start point -> Rd and Rp through the SpMV epilogues -> residual state.  With keep_iterate = 0 the
+// start point is zero and the two SpMVs still run: one code path for both modes, and A 0 = 0 exactly.
+void cuadmm_solver::update_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                                const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig) {
+    CUADMM_REQUIRE(initialised, "update_data() before init()");
+    CUADMM_REQUIRE(b_nnz >= 0 && C_nnz >= 0, "negative nnz");
+    CUADMM_REQUIRE((b_idx && b_val) || b_nnz == 0, "b is null");
+    CUADMM_REQUIRE((C_idx && C_val) || C_nnz == 0, "C is null");
+    CUADMM_REQUIRE(b_nnz + C_nnz < INT32_MAX, "b and C exceed int32 triplet indices");
+    // every check before the first device write: a rejected call leaves the solver as it was
+    for (int64_t k = 0; k < b_nnz; ++k) CUADMM_REQUIRE(b_idx[k] >= 0 && b_idx[k] < con_num, "b index out of range");
+    for (int64_t k = 0; k < C_nnz; ++k) CUADMM_REQUIRE(C_idx[k] >= 0 && C_idx[k] < vec_len, "C index out of range");
+    CUADMM_CUDA(cudaSetDevice(device));
+    const auto t0 = std::chrono::steady_clock::now();
+    CUADMM_CUDA(cudaEventRecord(ev_start, stream));     // total_time of the next solve counts from here, as from init
+    // this rank's C triplets at local offsets (sharded: the owned svec ranges only)
+    std::vector<int32_t> lci; std::vector<double> lcv;
+    const int32_t* ci = C_idx; const double* cv = C_val; int64_t cn = C_nnz;
+    if (world > 1) {
+        for (int64_t k = 0; k < C_nnz; ++k) {
+            const int64_t l = shard.glob2loc[C_idx[k]];
+            if (l >= 0) { lci.push_back((int32_t)l); lcv.push_back(C_val[k]); }
+        }
+        ci = lci.data(); cv = lcv.data(); cn = (int64_t)lci.size();
+    }
+    // staging: b, all of C, and (sharded) this rank's C
+    const int64_t nt = b_nnz + C_nnz + (world > 1 ? cn : 0);
+    if (upd_idx.n < std::max<int64_t>(nt, 1)) { upd_idx.alloc(std::max<int64_t>(nt, 1)); upd_val.alloc(std::max<int64_t>(nt, 1)); }
+    const int64_t nwin = std::max<int64_t>(std::max(con_num, vec_len), 1);
+    const int gb = ew_grid(con_num, device), gc = ew_grid(vec_len, device);
+    if (upd_win.n < nwin) upd_win.alloc(nwin);
+    if (upd_part.n < 2 * (int64_t)(gb + gc)) upd_part.alloc(2 * (int64_t)(gb + gc));
+    if (upd_zero.n == 0) { upd_zero.alloc(2); upd_zero.zero(stream); }
+    if (world > 1 && upd_full.n < std::max<int64_t>(vec_len, 1)) upd_full.alloc(std::max<int64_t>(vec_len, 1));
+    auto stage_in = [&](int64_t at, const int32_t* idx, const double* val, int64_t n) {
+        if (!n) return;
+        CUADMM_CUDA(cudaMemcpyAsync(upd_idx.p + at, idx, sizeof(int32_t) * n, cudaMemcpyHostToDevice, stream));
+        CUADMM_CUDA(cudaMemcpyAsync(upd_val.p + at, val, sizeof(double) * n, cudaMemcpyHostToDevice, stream));
+    };
+    stage_in(0, b_idx, b_val, b_nnz);
+    stage_in(b_nnz, C_idx, C_val, C_nnz);
+    if (world > 1) stage_in(b_nnz + C_nnz, ci, cv, cn);
+
+    // scalar state as init leaves it (done = 0 also lets the SpMV and reduction kernels below run)
+    const double bscale_old = bscale, Cscale_old = Cscale;
+    memset(h_st, 0, sizeof(DevState));
+    h_st->sig = sig; h_st->tau = 1.95;
+    h_st->sigmax = 1e3; h_st->sigmin = 1e-3; h_st->ratioconst = 1e0;
+    CUADMM_CUDA(cudaMemcpyAsync(st.p, h_st, sizeof(DevState), cudaMemcpyHostToDevice, stream));
+
+    // dense b and C
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
+    auto scatter = [&](const int32_t* idx, const double* val, int64_t nnz, DevBuf<double>& out, int64_t len) {
+        out.zero(stream);
+        if (!nnz) return;
+        CUADMM_CUDA(cudaMemsetAsync(upd_win.p, 0xff, sizeof(int32_t) * (size_t)len, stream));   // -1
+        const int g = (int)std::min<int64_t>((nnz + 255) / 256, (int64_t)sms * 8);
+        triplet_mark_kernel<<<g, 256, 0, stream>>>((int32_t)nnz, idx, upd_win.p);
+        triplet_store_kernel<<<g, 256, 0, stream>>>((int32_t)nnz, idx, val, upd_win.p, out.p);
+        launches += 2;
+    };
+    scatter(upd_idx.p, upd_val.p, b_nnz, bd, con_num);
+    scatter(upd_idx.p + b_nnz, upd_val.p + b_nnz, C_nnz, world > 1 ? upd_full : Cd, vec_len);
+    if (world > 1) scatter(upd_idx.p + b_nnz + C_nnz, upd_val.p + b_nnz + C_nnz, cn, Cd, nloc);
+
+    // |b|, |b ./ normA| and |C| over the full vectors, on grids that depend on con_num and vec_len only: a sharded
+    // solver reduces all of C on every rank (a scratch copy), so its scales are bit-identical to the one-GPU update's
+    double* part_b = upd_part.p;
+    double* part_c = upd_part.p + 2 * (int64_t)gb;
+    double* part_rd = partial.p;
+    double* part_rp = partial.p + 2 * (int64_t)std::max(nAt_blocks, nE_blocks);
+    sumsq_kernel<<<gb, kEwThreads, 0, stream>>>(con_num, bd.p, normA.p, part_b);
+    sumsq_kernel<<<gc, kEwThreads, 0, stream>>>(vec_len, world > 1 ? upd_full.p : Cd.p, nullptr, part_c);
+    data_scales_kernel<<<1, 256, 0, stream>>>(st.p, part_b, gb, part_c, gc);
+    launches += 2;
+    ++launches;
+    CUADMM_CUDA(cudaMemcpyAsync(h_st, st.p, sizeof(DevState), cudaMemcpyDeviceToHost, stream));
+    CUADMM_CUDA(cudaStreamSynchronize(stream));
+    bscale = h_st->bscale; Cscale = h_st->Cscale; objscale = h_st->objscale;
+    norm_borg = h_st->norm_borg; norm_Corg = h_st->norm_Corg;
+
+    // scaled b and C; the start point
+    const int gv = ew_grid(nloc, device), gm = ew_grid(con_num, device);
+    scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, bd.p, normA.p, 1.0 / bscale, 1);
+    scale_kernel<<<gv, 256, 0, stream>>>(nloc, Cd.p, 1.0 / Cscale);
+    launches += 2;
+    if (keep_iterate) {
+        if (iterate_scaled) {     // no solve since init / the last update: back to unscaled with the scales it was made with
+            scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, bscale_old);
+            scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, Cscale_old, 1);
+            scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cscale_old);
+            launches += 3;
+        }
+        // the rescaling of solve(if_first = 0) and of init's X0, y0, S0
+        scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, 1.0 / Cscale, 0);
+        scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, 1.0 / bscale);
+        scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, 1.0 / Cscale);
+        launches += 3;
+    } else {
+        X.zero(stream); y.zero(stream); S.zero(stream);
+        CUADMM_CUDA(cudaStreamSynchronize(stream));
+        plan->reset_warm_start();   // identity bases, as a new plan has them
+    }
+    sub_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cd.p, SmC.p);
+    ++launches;
+
+    // Rd = A^T y - C + S with |Rd|^2 and <C, X> (mode 3 with tau sig = 0 leaves X as it is), then Rp = b - A X with
+    // |normA .* Rp|^2 and <b, y> (K8), then the state; sharded: summed over ranks like the iteration's K7 / K8 scalars
+    SpmvEpilogue e; e.mode = 3; e.aux1 = Cd.p; e.aux2 = S.p; e.out2 = X.p; e.scal = upd_zero.p; e.partial = part_rd;
+    spmv_launch(*At, 1.0, y.p, 0.0, Rd.p, e, stream); ++launches;
+    if (world == 1) {
+        e = SpmvEpilogue(); e.mode = 4; e.aux1 = bd.p; e.aux2 = normA.p; e.aux3 = y.p; e.partial = part_rp;
+        spmv_launch(*A, 1.0, X.p, 0.0, Rp.p, e, stream); ++launches;
+        data_residuals_kernel<<<1, 256, 0, stream>>>(st.p, part_rd, nAt_blocks, part_rp, nA_blocks);
+    } else {
+        reduce_partial_A(true, X.p, 1.0, part_rd, nAt_blocks, part_rp);
+        if (use_peer)
+            data_residuals_kernel<<<1, 256, 0, stream>>>(st.p, peer->local<double>(peer->off_scal_rd), world,
+                                                         peer->local<double>(peer->off_scal_rp), world);
+        else
+            data_residuals_kernel<<<1, 256, 0, stream>>>(st.p, red_buf.p + con_num, 1, part_rp, nE_blocks);
+    }
+    ++launches;
+    CUADMM_CUDA(cudaGetLastError());
+    CUADMM_CUDA(cudaMemcpyAsync(h_st, st.p, sizeof(DevState), cudaMemcpyDeviceToHost, stream));
+    CUADMM_CUDA(cudaStreamSynchronize(stream));
+    if (peer) peer->check(stream);
+    asmc_valid = false;
+    iterate_scaled = true;
+    info_iter_num = 0;
+    for (auto& v : h_hist) v.clear();
+    update_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -876,6 +1089,14 @@ static void get_vec(cuadmm_solver_t* s, const DevBuf<double>& d, int64_t n, doub
     d.download(h, n, s->stream);
     CUADMM_CUDA(cudaStreamSynchronize(s->stream));
 }
+int cuadmm_solver_update_data(cuadmm_solver_t* s, const int32_t* b_idx, const double* b_vals, int64_t b_nnz,
+                              const int32_t* C_idx, const double* C_vals, int64_t C_nnz, int keep_iterate, double sig) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s, "solver is null");
+        s->update_data(b_idx, b_vals, b_nnz, C_idx, C_vals, C_nnz, keep_iterate != 0, sig);
+    });
+}
+
 int cuadmm_solver_get_X(cuadmm_solver_t* s, double* h) {
     return guarded([&] { if (s && s->world > 1) s->gather_full(s->X, h); else get_vec(s, s->X, s->vec_len, h); });
 }
@@ -928,6 +1149,7 @@ int cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* h
         if (h_y) s->y.upload(h_y, s->con_num, s->stream);
         if (h_S) s->S.upload(h_S, s->nloc, s->stream);
         s->asmc_valid = false;
+        s->iterate_scaled = false;
         s->h_st->sig = sig;                 // pinned mirror: stays valid until the copy below has run
         CUADMM_CUDA(cudaMemcpyAsync(&s->st.p->sig, &s->h_st->sig, sizeof(double), cudaMemcpyHostToDevice, s->stream));
         CUADMM_CUDA(cudaStreamSynchronize(s->stream));      // the caller's host buffers may be reused on return
@@ -949,7 +1171,7 @@ int cuadmm_solver_times(const cuadmm_solver_t* s, double out[8]) {
     return guarded([&] {
         CUADMM_REQUIRE(s && out, "null argument");
         out[0] = s->total_time; out[1] = s->init_time; out[2] = s->solve_time; out[3] = s->proj_time;
-        out[4] = s->ysolve_time; out[5] = s->spmv_time; out[6] = 0; out[7] = 0;
+        out[4] = s->ysolve_time; out[5] = s->spmv_time; out[6] = s->update_time; out[7] = 0;
     });
 }
 

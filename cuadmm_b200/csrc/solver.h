@@ -78,7 +78,12 @@ struct cuadmm_solver {
     std::vector<double> h_normA;
     int64_t info_iter_num = 0;
     std::vector<double> h_hist[8];           // drained from the device ring while solve() runs
-    double total_time = 0, init_time = 0, solve_time = 0, proj_time = 0, ysolve_time = 0, spmv_time = 0;
+    double total_time = 0, init_time = 0, solve_time = 0, proj_time = 0, ysolve_time = 0, spmv_time = 0, update_time = 0;
+    // update_data: X, y, S hold the scaled iterate (after init / update_data) or the unscaled one (after solve / set_XyS)
+    bool iterate_scaled = true;
+    cuadmm::DevBuf<int32_t> upd_idx, upd_win;   // b then C triplets on the device; last-write-wins marks per dense entry
+    cuadmm::DevBuf<double> upd_val, upd_part, upd_zero;   // their values; per-CTA norm partials; (sig, tau) = (0, 0)
+    cuadmm::DevBuf<double> upd_full;         // sharded: all of C, for the norm every rank takes over the full vector
     int64_t launches = 0;
     int nA_blocks = 0, nAt_blocks = 0, nE_blocks = 0;
     bool profile = false;
@@ -93,6 +98,9 @@ struct cuadmm_solver {
               const int32_t* blk, int64_t mat_num, const double* X0, const double* y0, const double* S0, double sig);
     void solve(int max_iter, double stop_tol, int sig_update_threshold, int sig_update_stage_1,
                int sig_update_stage_2, int switch_admm, double sigscale, bool if_first);
+    // new b and C on the same A and blocks; every device buffer is written in place (the graphs hold the pointers)
+    void update_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                     const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig);
     void enqueue_iteration(int iter, int switch_admm, bool prof = false);
     void run_iterations(int n_iters, bool sgs, bool profile, double out_ms[8]);
     void enqueue_half_step();

@@ -201,12 +201,29 @@ int  cuadmm_solver_get_y(cuadmm_solver_t* s, double* h_y);
 int  cuadmm_solver_get_S(cuadmm_solver_t* s, double* h_S);
 /* warm-restart: replace X,y,S (unscaled) before solve(..., if_first=0) (src/solver.cu:385-409) */
 int  cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* h_y, const double* h_S, double sig);
+/* New b and C for the same A, blocks and cones (receding-horizon re-solves), keeping everything init derived from A
+ * and the blocks: normA, the SpMV operators, the A A^T factorisation, the projection plan, the shard and peer arena,
+ * and the captured iteration graphs.  b and C are sparse host triplets as in cuadmm_solver_init (0-based, C by typed
+ * svec offset, a repeated index keeps its last value, copied and never mutated); their pattern may differ from init's.
+ * Collective on a sharded solver: every rank passes the same full arrays.  Out-of-range indices return CUADMM_EINVAL
+ * and leave the solver as it was.  Follow with solve(..., if_first = 1).
+ *   keep_iterate = 0: the next solve behaves like a fresh init with the same A / blocks, this b, C and sig and no
+ *                     X0 / y0 / S0 (the Jacobi warm-start bases are reset to the identity);
+ *   keep_iterate = 1: the start point is the X, y, S the last solve returned, as if given to a fresh init as
+ *                     X0 / y0 / S0 (the Jacobi bases are kept, so agreement with that init is to rounding).
+ * The residuals and scales are computed on the device, in another order than init's host loops: a cold update
+ * agrees with a fresh init to rounding, not bit for bit.  Its wall time is cuadmm_solver_times out[6]. */
+int  cuadmm_solver_update_data(cuadmm_solver_t* s,
+        const int32_t* b_idx, const double* b_vals, int64_t b_nnz,
+        const int32_t* C_idx, const double* C_vals, int64_t C_nnz,
+        int keep_iterate, double sig);
 /* info_iter_num and the per-iteration history (info_*_arr, src/solver.cu:802-810).
  * which: 0 pobj 1 dobj 2 errRp 3 errRd 4 relgap 5 sig 6 bscale 7 Cscale */
 int64_t cuadmm_solver_iter_num(const cuadmm_solver_t* s);
 int  cuadmm_solver_history(const cuadmm_solver_t* s, int which, double* out, int64_t cap);
-/* timings in seconds: out[0]=total_time (since init, as the reference), out[1]=init,
- * out[2]=solve loop, out[3]=projection total, out[4]=y-solve total, out[5]=spmv total */
+/* timings in seconds: out[0]=total_time (since init or the last update_data, as the reference), out[1]=init,
+ * out[2]=solve loop, out[3]=projection total, out[4]=y-solve total, out[5]=spmv total,
+ * out[6]=last cuadmm_solver_update_data (0 before the first) */
 int  cuadmm_solver_times(const cuadmm_solver_t* s, double out[8]);
 int64_t cuadmm_solver_launches(const cuadmm_solver_t* s);
 /* Measurement hook: enqueue `n_iters` iterations (sGS when sgs != 0, plain ADMM otherwise) from the
