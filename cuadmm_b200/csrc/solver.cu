@@ -28,22 +28,10 @@ void spmv_set_done_flag(cuadmm_spmv_s& A, const int* flag);
 static constexpr int kEwThreads = 256;
 static constexpr int64_t kHistRing = 4096;      // device history ring (entries per array)
 
-// ADMM branch of step 4 (no second y-solve): Rd = Rd1 + S ; X += tau*sig*Rd ; partial sums
-__global__ void __launch_bounds__(kEwThreads) x_update_kernel(int64_t n, const double* __restrict__ Rd1,
-        const double* __restrict__ S, const double* __restrict__ Cd, double* Rd, double* X,
-        const DevState* st, double* partial) {
-    if (st->done) return;
+// end of a grid-stride pair reduction of kEwThreads threads: warp shuffle tree, then thread 0 adds the warps in order
+// and stores this CTA's pair at partial[2 * blockIdx.x]
+__device__ __forceinline__ void store_cta_pair(double a0, double a1, double* partial) {
     __shared__ double red[2][kEwThreads / 32];
-    const double ts = st->tau * st->sig;
-    double a0 = 0.0, a1 = 0.0;
-    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
-        const double rd = Rd1[i] + S[i];
-        Rd[i] = rd;
-        const double xn = X[i] + ts * rd;
-        X[i] = xn;
-        a0 = fma(rd, rd, a0);
-        a1 = fma(Cd[i], xn, a1);
-    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
     if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a0; red[1][threadIdx.x >> 5] = a1; }
@@ -55,30 +43,65 @@ __global__ void __launch_bounds__(kEwThreads) x_update_kernel(int64_t n, const d
     }
 }
 
+// one CTA of 256 threads: the pairwise sums of na pairs at pa and (Q = 4) nb pairs at pb, in a fixed order
+template <int Q>
+__device__ __forceinline__ void sum_pairs_256(const double* __restrict__ pa, int na, const double* __restrict__ pb, int nb,
+                                              double out[Q]) {
+    __shared__ double sm[Q][256];
+    double v[Q] = {};
+    for (int i = threadIdx.x; i < na; i += 256) { v[0] += pa[2 * i]; v[1] += pa[2 * i + 1]; }
+    if constexpr (Q == 4)
+        for (int i = threadIdx.x; i < nb; i += 256) { v[2] += pb[2 * i]; v[3] += pb[2 * i + 1]; }
+    for (int q = 0; q < Q; ++q) sm[q][threadIdx.x] = v[q];
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) for (int q = 0; q < Q; ++q) sm[q][threadIdx.x] += sm[q][threadIdx.x + o];
+        __syncthreads();
+    }
+    for (int q = 0; q < Q; ++q) out[q] = sm[q][0];
+}
+
+// residuals and objectives (src/solver.cu:193-228, 772-790) from the sums |Rd|^2, <C, X>, |normA .* Rp|^2, <b, y>
+struct Residuals { double errRp, errRd, pobj, dobj, maxfeas, relgap; };
+__device__ __forceinline__ Residuals residuals(const DevState* st, const double s[4]) {
+    Residuals r;
+    r.errRp = st->bscale * sqrt(s[2]) / st->norm_borg;
+    r.pobj = s[1] * st->objscale;
+    r.errRd = st->Cscale * sqrt(s[0]) / st->norm_Corg;
+    r.dobj = s[3] * st->objscale;
+    r.maxfeas = fmax(r.errRp, r.errRd);
+    r.relgap = fabs(r.pobj - r.dobj) / (1 + fabs(r.pobj) + fabs(r.dobj));
+    return r;
+}
+
+// ADMM branch of step 4 (no second y-solve): Rd = Rd1 + S ; X += tau*sig*Rd ; partial sums
+__global__ void __launch_bounds__(kEwThreads) x_update_kernel(int64_t n, const double* __restrict__ Rd1,
+        const double* __restrict__ S, const double* __restrict__ Cd, double* Rd, double* X,
+        const DevState* st, double* partial) {
+    if (st->done) return;
+    const double ts = st->tau * st->sig;
+    double a0 = 0.0, a1 = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
+        const double rd = Rd1[i] + S[i];
+        Rd[i] = rd;
+        const double xn = X[i] + ts * rd;
+        X[i] = xn;
+        a0 = fma(rd, rd, a0);
+        a1 = fma(Cd[i], xn, a1);
+    }
+    store_cta_pair(a0, a1, partial);
+}
+
 // K9: fixed-order reduction of the per-CTA partials, then the reference's scalar logic
 __global__ void __launch_bounds__(256) scalar_update_kernel(DevState* st, const double* __restrict__ part_rd, int n_rd,
         const double* __restrict__ part_rp, int n_rp, double* hist, int64_t hist_cap) {
     if (st->done) return;
-    __shared__ double sm[4][256];
-    double v[4] = {0.0, 0.0, 0.0, 0.0};
-    for (int i = threadIdx.x; i < n_rd; i += 256) { v[0] += part_rd[2 * i]; v[1] += part_rd[2 * i + 1]; }
-    for (int i = threadIdx.x; i < n_rp; i += 256) { v[2] += part_rp[2 * i]; v[3] += part_rp[2 * i + 1]; }
-    for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] = v[q];
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] += sm[q][threadIdx.x + o];
-        __syncthreads();
-    }
+    double s[4];
+    sum_pairs_256<4>(part_rd, n_rd, part_rp, n_rp, s);
     if (threadIdx.x != 0) return;
-    const double sumRd = sm[0][0], sumCX = sm[1][0], sumRp = sm[2][0], sumby = sm[3][0];
     const int iter = st->iter;
-    const double errRp = st->bscale * sqrt(sumRp) / st->norm_borg;
-    const double pobj = sumCX * st->objscale;
-    const double errRd = st->Cscale * sqrt(sumRd) / st->norm_Corg;
-    const double dobj = sumby * st->objscale;
-    const double maxfeas = fmax(errRp, errRd);
-    const double relgap = fabs(pobj - dobj) / (1 + fabs(pobj) + fabs(dobj));
-    const double feasratio = st->ratioconst * errRp / errRd;
+    const Residuals r = residuals(st, s);
+    const double feasratio = st->ratioconst * r.errRp / r.errRd;
     if (feasratio < 1) st->prim_win += 1; else st->dual_win += 1;
     double sig = st->sig;
     if (((iter <= st->sig_update_threshold) && ((iter % st->sig_update_stage_1) == 1)) ||
@@ -92,22 +115,22 @@ __global__ void __launch_bounds__(256) scalar_update_kernel(DevState* st, const 
         }
     }
     st->sig = sig;
-    st->errRp = errRp; st->errRd = errRd; st->pobj = pobj; st->dobj = dobj;
-    st->maxfeas = maxfeas; st->relgap = relgap; st->feasratio = feasratio;
+    st->errRp = r.errRp; st->errRd = r.errRd; st->pobj = r.pobj; st->dobj = r.dobj;
+    st->maxfeas = r.maxfeas; st->relgap = r.relgap; st->feasratio = feasratio;
     {
         const int64_t k = (int64_t)(iter - 1) % hist_cap;      // ring: the host drains it at every log boundary
-        hist[0 * hist_cap + k] = pobj;  hist[1 * hist_cap + k] = dobj;
-        hist[2 * hist_cap + k] = errRp; hist[3 * hist_cap + k] = errRd;
-        hist[4 * hist_cap + k] = relgap; hist[5 * hist_cap + k] = sig;
+        hist[0 * hist_cap + k] = r.pobj;  hist[1 * hist_cap + k] = r.dobj;
+        hist[2 * hist_cap + k] = r.errRp; hist[3 * hist_cap + k] = r.errRd;
+        hist[4 * hist_cap + k] = r.relgap; hist[5 * hist_cap + k] = sig;
         hist[6 * hist_cap + k] = st->bscale; hist[7 * hist_cap + k] = st->Cscale;
     }
     const int next = iter + 1;
     st->iter = next;
     double tau = (next < st->switch_admm) ? 1.95 : 1.618;
-    if (errRd < st->stop_tol) tau = fmax(1.618, tau / 1.1);
+    if (r.errRd < st->stop_tol) tau = fmax(1.618, tau / 1.1);
     st->tau = tau;
     // stop test that the reference evaluates at the top of iteration `next`
-    if (fmax(maxfeas, relgap) < st->stop_tol) { st->done = 1; st->stop_reason = 1; }
+    if (fmax(r.maxfeas, r.relgap) < st->stop_tol) { st->done = 1; st->stop_reason = 1; }
     if (next > st->max_iter) { st->done = 1; st->stop_reason = 2; }
 }
 
@@ -152,22 +175,14 @@ __global__ void rhsy_kernel(int64_t m, const double* __restrict__ Rp, const doub
 // local per-CTA partial pairs -> two scalars appended to the all-reduce buffer
 __global__ void __launch_bounds__(256) fold_partials_kernel(const double* __restrict__ part, int n, double* out2, const DevState* st) {
     if (st->done) return;
-    __shared__ double sm[2][256];
-    double a = 0.0, b = 0.0;
-    for (int i = threadIdx.x; i < n; i += 256) { a += part[2 * i]; b += part[2 * i + 1]; }
-    sm[0][threadIdx.x] = a; sm[1][threadIdx.x] = b;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) { sm[0][threadIdx.x] += sm[0][threadIdx.x + o]; sm[1][threadIdx.x] += sm[1][threadIdx.x + o]; }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) { out2[0] = sm[0][0]; out2[1] = sm[1][0]; }
+    double s[2];
+    sum_pairs_256<2>(part, n, nullptr, 0, s);
+    if (threadIdx.x == 0) { out2[0] = s[0]; out2[1] = s[1]; }
 }
 // distributed K8: Rp = b - buf (buf = all-reduced A X) ; partial sums |normA Rp|^2, <b, y>
 __global__ void __launch_bounds__(kEwThreads) rp_kernel(int64_t m, const double* __restrict__ b, const double* __restrict__ buf,
         const double* __restrict__ normA, const double* __restrict__ y, double* Rp, const DevState* st, double* partial) {
     if (st->done) return;
-    __shared__ double red[2][kEwThreads / 32];
     double a0 = 0.0, a1 = 0.0;
     for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < m; i += (int64_t)gridDim.x * kEwThreads) {
         const double rp = b[i] - buf[i];
@@ -176,15 +191,7 @@ __global__ void __launch_bounds__(kEwThreads) rp_kernel(int64_t m, const double*
         a0 = fma(t, t, a0);
         a1 = fma(b[i], y[i], a1);
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
-    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a0; red[1][threadIdx.x >> 5] = a1; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double s0 = 0.0, s1 = 0.0;
-        for (int k = 0; k < kEwThreads / 32; ++k) { s0 += red[0][k]; s1 += red[1][k]; }
-        partial[2 * blockIdx.x] = s0; partial[2 * blockIdx.x + 1] = s1;
-    }
+    store_cta_pair(a0, a1, partial);
 }
 __global__ void scatter_full_kernel(int64_t nloc, const double* __restrict__ local, const int64_t* __restrict__ loc2glob, double* full) {
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nloc; i += (int64_t)gridDim.x * blockDim.x) full[loc2glob[i]] = local[i];
@@ -204,43 +211,19 @@ __global__ void triplet_store_kernel(int32_t nnz, const int32_t* __restrict__ id
 // per-CTA partial pair (sum x^2, sum (x ./ d)^2), the second 0 when d is null; fixed tree inside the CTA
 __global__ void __launch_bounds__(kEwThreads) sumsq_kernel(int64_t n, const double* __restrict__ x, const double* __restrict__ d,
                                                            double* partial) {
-    __shared__ double red[2][kEwThreads / 32];
     double a0 = 0.0, a1 = 0.0;
     for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
         const double v = x[i];
         a0 = fma(v, v, a0);
         if (d) { const double t = v / d[i]; a1 = fma(t, t, a1); }
     }
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
-    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = a0; red[1][threadIdx.x >> 5] = a1; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        double s0 = 0.0, s1 = 0.0;
-        for (int k = 0; k < kEwThreads / 32; ++k) { s0 += red[0][k]; s1 += red[1][k]; }
-        partial[2 * blockIdx.x] = s0; partial[2 * blockIdx.x + 1] = s1;
-    }
-}
-// one CTA of 256 threads: the pairwise sums of na pairs at pa and nb pairs at pb, in scalar_update_kernel's fixed order
-__device__ __forceinline__ void sum_pairs_256(const double* __restrict__ pa, int na, const double* __restrict__ pb, int nb,
-                                              double out[4]) {
-    __shared__ double sm[4][256];
-    double v[4] = {0.0, 0.0, 0.0, 0.0};
-    for (int i = threadIdx.x; i < na; i += 256) { v[0] += pa[2 * i]; v[1] += pa[2 * i + 1]; }
-    for (int i = threadIdx.x; i < nb; i += 256) { v[2] += pb[2 * i]; v[3] += pb[2 * i + 1]; }
-    for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] = v[q];
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) for (int q = 0; q < 4; ++q) sm[q][threadIdx.x] += sm[q][threadIdx.x + o];
-        __syncthreads();
-    }
-    for (int q = 0; q < 4; ++q) out[q] = sm[q][0];
+    store_cta_pair(a0, a1, partial);
 }
 // the scaling constants (src/solver.cu:113-191): part_b pairs (|b|^2, |b ./ normA|^2), part_c pairs (|C|^2, 0)
 __global__ void __launch_bounds__(256) data_scales_kernel(DevState* st, const double* __restrict__ part_b, int n_b,
                                                           const double* __restrict__ part_c, int n_c) {
     double s[4];
-    sum_pairs_256(part_b, n_b, part_c, n_c, s);
+    sum_pairs_256<4>(part_b, n_b, part_c, n_c, s);
     if (threadIdx.x != 0) return;
     const double nC = sqrt(s[2]);
     st->norm_borg = 1 + sqrt(s[0]);
@@ -250,18 +233,15 @@ __global__ void __launch_bounds__(256) data_scales_kernel(DevState* st, const do
     st->objscale = st->bscale * st->Cscale;
 }
 // the initial residuals and objectives (src/solver.cu:193-228) from the partials of Rd (|Rd|^2, <C, X>) and Rp
-// (|normA .* Rp|^2, <b, y>), with scalar_update_kernel's formulas
+// (|normA .* Rp|^2, <b, y>), in scalar_update_kernel's order
 __global__ void __launch_bounds__(256) data_residuals_kernel(DevState* st, const double* __restrict__ part_rd, int n_rd,
                                                              const double* __restrict__ part_rp, int n_rp) {
     double s[4];
-    sum_pairs_256(part_rd, n_rd, part_rp, n_rp, s);
+    sum_pairs_256<4>(part_rd, n_rd, part_rp, n_rp, s);
     if (threadIdx.x != 0) return;
-    const double errRp = st->bscale * sqrt(s[2]) / st->norm_borg;
-    const double errRd = st->Cscale * sqrt(s[0]) / st->norm_Corg;
-    const double pobj = s[1] * st->objscale, dobj = s[3] * st->objscale;
-    st->errRp = errRp; st->errRd = errRd; st->pobj = pobj; st->dobj = dobj;
-    st->maxfeas = fmax(errRp, errRd);
-    st->relgap = fabs(pobj - dobj) / (1 + fabs(pobj) + fabs(dobj));
+    const Residuals r = residuals(st, s);
+    st->errRp = r.errRp; st->errRd = r.errRd; st->pobj = r.pobj; st->dobj = r.dobj;
+    st->maxfeas = r.maxfeas; st->relgap = r.relgap;
 }
 
 static int ew_grid(int64_t n, int device) {
@@ -269,20 +249,6 @@ static int ew_grid(int64_t n, int device) {
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
     return (int)std::max<int64_t>(1, std::min<int64_t>((n + kEwThreads - 1) / kEwThreads, (int64_t)sms * 8));
 }
-
-static double host_norm2(const std::vector<double>& v) {
-    // scaled sum of squares (dnrm2 semantics: no overflow for any finite input)
-    double scale = 0.0, ssq = 1.0;
-    for (double x : v) {
-        if (x != 0.0) {
-            const double a = std::fabs(x);
-            if (scale < a) { ssq = 1.0 + ssq * (scale / a) * (scale / a); scale = a; }
-            else ssq += (a / scale) * (a / scale);
-        }
-    }
-    return scale * std::sqrt(ssq);
-}
-
 }  // namespace cuadmm
 
 using namespace cuadmm;
@@ -308,6 +274,8 @@ void cuadmm_solver::init(int /*eig_stream_num_per_gpu*/, int /*cpu_eig_thread_nu
     CUADMM_REQUIRE(vec_len_ >= 0 && con_num_ >= 0 && At_nnz >= 0, "negative dimension");
     CUADMM_REQUIRE(At_col_ptrs && blk, "null argument");
     CUADMM_REQUIRE(At_col_ptrs[0] == 0 && At_col_ptrs[con_num_] == At_nnz, "At_csc_col_ptrs does not span At_nnz");
+    vec_len = vec_len_; con_num = con_num_;
+    check_data(b_idx, b_val, b_nnz, C_idx, C_val, C_nnz);
     int cnt = 0;
     if (cudaGetDeviceCount(&cnt) != cudaSuccess || cnt == 0) {
         cudaGetLastError();
@@ -321,7 +289,6 @@ void cuadmm_solver::init(int /*eig_stream_num_per_gpu*/, int /*cpu_eig_thread_nu
     if (const char* e = getenv("CUADMM_NO_GRAPH")) use_graphs = atoi(e) == 0;
     CUADMM_REQUIRE(device >= 0 && device < cnt, "device index out of range");
     CUADMM_CUDA(cudaSetDevice(device));
-    vec_len = vec_len_; con_num = con_num_;
     CUADMM_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
     CUADMM_CUDA(cudaEventCreate(&ev_start));
     CUADMM_CUDA(cudaEventCreate(&ev_now));
@@ -409,86 +376,46 @@ void cuadmm_solver::init(int /*eig_stream_num_per_gpu*/, int /*cpu_eig_thread_nu
         }
     }
 
-    // ---- b, C, X, y, S and the scaling (src/solver.cu:113-191)
-    std::vector<double> hb(con_num, 0.0), hC(vec_len, 0.0), hX(vec_len, 0.0), hy(con_num, 0.0), hS(vec_len, 0.0);
-    for (int64_t k = 0; k < b_nnz; ++k) { CUADMM_REQUIRE(b_idx[k] >= 0 && b_idx[k] < con_num, "b index out of range"); hb[b_idx[k]] = b_val[k]; }
-    for (int64_t k = 0; k < C_nnz; ++k) { CUADMM_REQUIRE(C_idx[k] >= 0 && C_idx[k] < vec_len, "C index out of range"); hC[C_idx[k]] = C_val[k]; }
-    if (X0) std::copy(X0, X0 + vec_len, hX.begin());
-    if (y0) std::copy(y0, y0 + con_num, hy.begin());
-    if (S0) std::copy(S0, S0 + vec_len, hS.begin());
-    norm_borg = 1 + host_norm2(hb);
-    norm_Corg = 1 + host_norm2(hC);
-    for (int64_t i = 0; i < con_num; ++i) { hb[i] /= h_normA[i]; hy[i] *= h_normA[i]; }
-    bscale = 1 + host_norm2(hb);
-    Cscale = 1 + host_norm2(hC);
-    objscale = bscale * Cscale;
-    for (auto& v : hb) v /= bscale;
-    for (auto& v : hC) v /= Cscale;
-    for (auto& v : hX) v /= bscale;
-    for (auto& v : hS) v /= Cscale;
-    for (auto& v : hy) v /= Cscale;
-
-    // ---- initial residuals (src/solver.cu:193-228) on the host: init-time, O(nnz)
-    std::vector<double> hRp(con_num), hSmC(vec_len), hRd(vec_len, 0.0);
-    for (int64_t i = 0; i < con_num; ++i) {
-        double acc = 0.0;
-        for (int p = At_col_ptrs[i]; p < At_col_ptrs[i + 1]; ++p) acc += vals[p] * hX[At_row_ids[p]];
-        hRp[i] = hb[i] - acc;
-    }
-    for (int64_t i = 0; i < con_num; ++i)
-        for (int p = At_col_ptrs[i]; p < At_col_ptrs[i + 1]; ++p) hRd[At_row_ids[p]] += vals[p] * hy[i];   // Aty
-    double sRp = 0, sRd = 0, cx = 0, by = 0;
-    {
-        std::vector<double> tmp(con_num);
-        for (int64_t i = 0; i < con_num; ++i) tmp[i] = h_normA[i] * hRp[i] * bscale;
-        sRp = host_norm2(tmp);
-        for (int64_t i = 0; i < vec_len; ++i) { hSmC[i] = hS[i] - hC[i]; hRd[i] = (hRd[i] + hSmC[i]) * Cscale; cx += hC[i] * hX[i]; }
-        sRd = host_norm2(hRd);
-        for (int64_t i = 0; i < con_num; ++i) by += hb[i] * hy[i];
-    }
-
     // ---- device vectors
-    auto up = [&](DevBuf<double>& d, const std::vector<double>& h) {
-        if (d.owned || !d.p) d.alloc(std::max<int64_t>((int64_t)h.size(), 1));     // views of the peer arena are kept
-        d.upload(h.data(), (int64_t)h.size(), stream);
+    auto alloc = [&](DevBuf<double>& d, int64_t len) {
+        if (d.owned || !d.p) d.alloc(std::max<int64_t>(len, 1));     // views of the peer arena are kept
     };
-    if (world > 1) {   // keep only the owned svec ranges of X, S, S-C, C
-        std::vector<double> t;
-        shard.slice_vec(hX.data(), t); hX.swap(t);
-        shard.slice_vec(hS.data(), t); hS.swap(t);
-        shard.slice_vec(hSmC.data(), t); hSmC.swap(t);
-        shard.slice_vec(hC.data(), t); hC.swap(t);
-    }
-    up(X, hX); up(S, hS); up(y, hy); up(Rp, hRp); up(SmC, hSmC); up(Cd, hC); up(bd, hb); up(normA, h_normA);
-    Rd1.alloc(std::max<int64_t>(nloc, 1)); Rd.alloc(std::max<int64_t>(nloc, 1)); Xb.alloc(std::max<int64_t>(nloc, 1));
-    Xproj.alloc(std::max<int64_t>(nloc, 1)); rhsy.alloc(std::max<int64_t>(con_num, 1)); if (asmc.owned || !asmc.p) asmc.alloc(std::max<int64_t>(con_num, 1)); asmc_valid = false;
+    alloc(X, nloc); alloc(S, nloc); alloc(y, con_num); alloc(Rp, con_num); alloc(SmC, nloc); alloc(Cd, nloc); alloc(bd, con_num);
+    alloc(normA, con_num); alloc(Rd1, nloc); alloc(Rd, nloc); alloc(Xb, nloc); alloc(Xproj, nloc); alloc(rhsy, con_num); alloc(asmc, con_num);
+    normA.upload(h_normA.data(), con_num, stream);
     Rd1.zero(stream); Rd.zero(stream);
     nA_blocks = spmv_grid(*A); nAt_blocks = spmv_grid(*At); nE_blocks = ew_grid(std::max(nloc, con_num), device);
     partial.alloc(2 * (int64_t)(std::max(nAt_blocks, nE_blocks) + std::max(nA_blocks, nE_blocks)) + 4);
     partial.zero(stream);
-
     st.alloc(1);
     CUADMM_CUDA(cudaMallocHost((void**)&h_st, sizeof(DevState)));
-    memset(h_st, 0, sizeof(DevState));
-    h_st->sig = sig; h_st->tau = 1.95;
-    h_st->errRp = sRp / norm_borg; h_st->errRd = sRd / norm_Corg;
-    h_st->maxfeas = std::max(h_st->errRp, h_st->errRd);
-    h_st->pobj = cx * objscale; h_st->dobj = by * objscale;
-    h_st->relgap = std::fabs(h_st->pobj - h_st->dobj) / (1 + std::fabs(h_st->pobj) + std::fabs(h_st->dobj));
-    h_st->bscale = bscale; h_st->Cscale = Cscale; h_st->objscale = objscale;
-    h_st->norm_borg = norm_borg; h_st->norm_Corg = norm_Corg;
-    h_st->sigmax = 1e3; h_st->sigmin = 1e-3; h_st->ratioconst = 1e0;
-    h_st->prim_win = 0; h_st->dual_win = 0;
-    CUADMM_CUDA(cudaMemcpyAsync(st.p, h_st, sizeof(DevState), cudaMemcpyHostToDevice, stream));
-
     const int* done_ptr = &st.p->done;
     spmv_set_done_flag(*A, done_ptr);
     spmv_set_done_flag(*At, done_ptr);
     ys->done_flag = done_ptr;
     plan->done_flag = done_ptr;
-    CUADMM_CUDA(cudaStreamSynchronize(stream));
+
+    // ---- b, C, the scaling, the start point and the initial residuals (src/solver.cu:113-228): the path of
+    // update_data with the iterate kept, from X0, y0, S0 (zero where not given)
+    X.zero(stream); y.zero(stream); S.zero(stream);
+    set_iterate(X0, y0, S0);
+    load_data(b_idx, b_val, b_nnz, C_idx, C_val, C_nnz, true, sig);
+    // the staging buffers are only needed again by update_data
+    upd_idx.release(); upd_win.release(); upd_val.release(); upd_part.release(); upd_zero.release(); upd_full.release();
     init_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
     initialised = true;
+}
+
+// K1: rhsy = Rp/sig - A(S-C).  The product asmc = -A(S-C) is kept: in an sGS iteration K5 computes it for
+// the NEW S, which is exactly what K1 of the next iteration needs (S does not change in between), so that
+// K1 is then only the vector update — one SpMV (and, multi-GPU, one all-reduce) less per sGS iteration than
+// the reference's loop (src/solver.cu:478-482 recomputes it).  Multi-GPU: partial -A_g (S-C)_g, all-reduce.
+void cuadmm_solver::enqueue_k1(bool asmc_cached) {
+    if (!asmc_cached) {
+        if (world == 1) { SpmvEpilogue e; spmv_launch(*A, -1.0, SmC.p, 0.0, asmc.p, e, stream); ++launches; }
+        else reduce_partial_A(false, SmC.p, -1.0, nullptr, 0, nullptr);
+    }
+    rhsy_kernel<<<ew_grid(con_num, device), 256, 0, stream>>>(con_num, Rp.p, asmc.p, rhsy.p, st.p); ++launches;
 }
 
 // Steps 1 .. 5 of iteration `iter` (src/solver.cu:469-799); every kernel is a no-op once st->done
@@ -506,19 +433,7 @@ void cuadmm_solver::enqueue_iteration(int iter, int switch_admm, bool prof) {
     };
     ys->prof_ev = prof ? &prof_ev : nullptr;       // the y-solve brackets its dense-tail stage (tags 20 / 21)
     ys->prof_tag = prof ? &prof_tag : nullptr;
-    const int gm_ = ew_grid(con_num, device);
-    // K1: rhsy = Rp/sig - A(S-C).  The product asmc = -A(S-C) is kept: in an sGS iteration K5 computes it for
-    // the NEW S, which is exactly what K1 of the next iteration needs (S does not change in between), so that
-    // K1 is then only the vector update — one SpMV (and, multi-GPU, one all-reduce) less per sGS iteration than
-    // the reference's loop (src/solver.cu:478-482 recomputes it).  Multi-GPU: partial -A_g (S-C)_g, all-reduce.
-    auto k1 = [&](bool cached) {
-        if (!cached) {
-            if (world == 1) { e = SpmvEpilogue(); spmv_launch(*A, -1.0, SmC.p, 0.0, asmc.p, e, stream); ++launches; }
-            else reduce_partial_A(false, SmC.p, -1.0, nullptr, 0, nullptr);
-        }
-        rhsy_kernel<<<gm_, 256, 0, stream>>>(con_num, Rp.p, asmc.p, rhsy.p, st.p); ++launches;
-    };
-    k1(asmc_valid);
+    enqueue_k1(asmc_valid);
     // K2
     mark(0);
     ys->solve(rhsy.p, y.p, stream); launches += ys->launches_per_solve;
@@ -544,7 +459,7 @@ void cuadmm_solver::enqueue_iteration(int iter, int switch_admm, bool prof) {
     if (iter < switch_admm) {
         // K5-K7: the sGS second half-step
         mark(6);
-        k1(false);
+        enqueue_k1(false);
         mark(7);
         mark(4);
         ys->solve(rhsy.p, y.p, stream); launches += ys->launches_per_solve;
@@ -653,12 +568,7 @@ void cuadmm_solver::reduce_partial_A(bool for_rp, const double* x_local, double 
 // what the reference still executes at the top of the iteration in which it breaks
 // (step 1 and step 2a, src/solver.cu:478-528): y is overwritten by the next half-step.
 void cuadmm_solver::enqueue_half_step() {
-    SpmvEpilogue e;
-    if (!asmc_valid) {
-        if (world == 1) { spmv_launch(*A, -1.0, SmC.p, 0.0, asmc.p, e, stream); ++launches; }
-        else reduce_partial_A(false, SmC.p, -1.0, nullptr, 0, nullptr);
-    }
-    rhsy_kernel<<<ew_grid(con_num, device), 256, 0, stream>>>(con_num, Rp.p, asmc.p, rhsy.p, st.p); ++launches;
+    enqueue_k1(asmc_valid);
     ys->solve(rhsy.p, y.p, stream); launches += ys->launches_per_solve;
 }
 
@@ -746,7 +656,6 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     CUADMM_CUDA(cudaSetDevice(device));
     const auto t0 = std::chrono::steady_clock::now();
     const int64_t n = nloc, m = con_num;
-    const int gv = ew_grid(n, device), gm = ew_grid(m, device);
     if (X_best.n < std::max<int64_t>(n, 1)) {   // always allocated: the ADMM graph bakes these pointers
         X_best.alloc(std::max<int64_t>(n, 1)); y_best.alloc(std::max<int64_t>(m, 1)); S_best.alloc(std::max<int64_t>(n, 1));
     }
@@ -787,11 +696,8 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     CUADMM_CUDA(cudaMemcpyAsync(h_st, st.p, sizeof(DevState), cudaMemcpyDeviceToHost, stream));
     CUADMM_CUDA(cudaStreamSynchronize(stream));
     if (!if_first) {
-        // second call: X, y, S were replaced by unscaled values (src/solver.cu:385-409)
-        scale_vec_kernel<<<gm, 256, 0, stream>>>(m, y.p, normA.p, 1.0 / Cscale, 0);
-        scale_kernel<<<gv, 256, 0, stream>>>(n, X.p, 1.0 / bscale);
-        scale_kernel<<<gv, 256, 0, stream>>>(n, S.p, 1.0 / Cscale);
-        sub_kernel<<<gv, 256, 0, stream>>>(n, S.p, Cd.p, SmC.p);
+        // second call: X, y, S were replaced by unscaled values
+        scale_iterate_in();
         h_st->done = 0;
         CUADMM_CUDA(cudaMemcpyAsync(st.p, h_st, sizeof(DevState), cudaMemcpyHostToDevice, stream));
         CUADMM_CUDA(cudaStreamSynchronize(stream));      // h_st is mutated below: the copy must have read it first
@@ -802,7 +708,6 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
         } else {
             reduce_partial_A(true, X.p, 1.0, nullptr, 0, partial.p);
         }
-        launches += 4;
     }
     h_st->iter = 1;
     h_st->max_iter = max_iter; h_st->stop_tol = stop_tol;
@@ -871,11 +776,7 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     }
     h_st->done = 1;
     CUADMM_CUDA(cudaMemcpyAsync(&st.p->done, &h_st->done, sizeof(int), cudaMemcpyHostToDevice, stream));
-    // unscale (src/solver.cu:814-816)
-    scale_kernel<<<gv, 256, 0, stream>>>(n, X.p, bscale);
-    scale_vec_kernel<<<gm, 256, 0, stream>>>(m, y.p, normA.p, Cscale, 1);
-    scale_kernel<<<gv, 256, 0, stream>>>(n, S.p, Cscale);
-    launches += 3;
+    unscale_iterate(bscale, Cscale);
     iterate_scaled = false;
     drain(info_iter_num);
     CUADMM_CUDA(cudaEventRecord(ev_now, stream));
@@ -897,24 +798,72 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     }
 }
 
-// New b and C for the same A and blocks: everything init derives from b and C, recomputed on the device in place.
-// normA, both SpMV operators, the y-solve, the plan, the shard, the peer arena and the captured graphs are kept.
-// Order (fixed by the data): scatter b, C -> norms -> scales (read back: solve() scales with host copies) -> scaled
-// b, C and the start point -> Rd and Rp through the SpMV epilogues -> residual state.  With keep_iterate = 0 the
-// start point is zero and the two SpMVs still run: one code path for both modes, and A 0 = 0 exactly.
-void cuadmm_solver::update_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
-                                const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig) {
-    CUADMM_REQUIRE(initialised, "update_data() before init()");
+// b and C triplets as the caller passes them to init and update_data; every check comes before the first device
+// write, so a rejected call leaves the solver as it was
+void cuadmm_solver::check_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                               const int32_t* C_idx, const double* C_val, int64_t C_nnz) const {
     CUADMM_REQUIRE(b_nnz >= 0 && C_nnz >= 0, "negative nnz");
     CUADMM_REQUIRE((b_idx && b_val) || b_nnz == 0, "b is null");
     CUADMM_REQUIRE((C_idx && C_val) || C_nnz == 0, "C is null");
     CUADMM_REQUIRE(b_nnz + C_nnz < INT32_MAX, "b and C exceed int32 triplet indices");
-    // every check before the first device write: a rejected call leaves the solver as it was
     for (int64_t k = 0; k < b_nnz; ++k) CUADMM_REQUIRE(b_idx[k] >= 0 && b_idx[k] < con_num, "b index out of range");
     for (int64_t k = 0; k < C_nnz; ++k) CUADMM_REQUIRE(C_idx[k] >= 0 && C_idx[k] < vec_len, "C index out of range");
+}
+
+// Unscaled X, y, S from the caller (full-length X and S; sharded: this rank's ranges are kept); a null vector is left
+// as it is.  The next solve(if_first = 0) or load_data scales them.
+void cuadmm_solver::set_iterate(const double* h_X, const double* h_y, const double* h_S) {
+    std::vector<double> lx, ls;
+    if (world > 1) {
+        if (h_X) { shard.slice_vec(h_X, lx); h_X = lx.data(); }
+        if (h_S) { shard.slice_vec(h_S, ls); h_S = ls.data(); }
+    }
+    if (h_X) X.upload(h_X, nloc, stream);
+    if (h_y) y.upload(h_y, con_num, stream);
+    if (h_S) S.upload(h_S, nloc, stream);
+    asmc_valid = false;
+    iterate_scaled = false;
+    CUADMM_CUDA(cudaStreamSynchronize(stream));      // lx, ls and the caller's buffers may be reused on return
+}
+
+// the start point into the scaled variables (src/solver.cu:385-409): y .* normA / Cscale, X / bscale, S / Cscale, S - C
+void cuadmm_solver::scale_iterate_in() {
+    const int gv = ew_grid(nloc, device), gm = ew_grid(con_num, device);
+    scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, 1.0 / Cscale, 0);
+    scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, 1.0 / bscale);
+    scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, 1.0 / Cscale);
+    sub_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cd.p, SmC.p);
+    launches += 4;
+}
+
+// the scaled iterate back to the caller's variables with the scales it was made with (src/solver.cu:814-816)
+void cuadmm_solver::unscale_iterate(double bs, double Cs) {
+    const int gv = ew_grid(nloc, device), gm = ew_grid(con_num, device);
+    scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, bs);
+    scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, Cs, 1);
+    scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cs);
+    launches += 3;
+}
+
+// New b and C for the same A and blocks: everything init derives from b and C, recomputed on the device in place.
+// normA, both SpMV operators, the y-solve, the plan, the shard, the peer arena and the captured graphs are kept.
+void cuadmm_solver::update_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                                const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig) {
+    CUADMM_REQUIRE(initialised, "update_data() before init()");
+    check_data(b_idx, b_val, b_nnz, C_idx, C_val, C_nnz);
     CUADMM_CUDA(cudaSetDevice(device));
     const auto t0 = std::chrono::steady_clock::now();
     CUADMM_CUDA(cudaEventRecord(ev_start, stream));     // total_time of the next solve counts from here, as from init
+    load_data(b_idx, b_val, b_nnz, C_idx, C_val, C_nnz, keep_iterate, sig);
+    update_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+}
+
+// Everything init derives from b and C, on the device, in the same order for init and update_data.  Order (fixed by
+// the data): scatter b, C -> norms -> scales (read back: solve() scales with host copies) -> scaled b, C and the start
+// point -> Rd and Rp through the SpMV epilogues -> residual state.  keep_iterate = 0 zeroes the start point; the
+// scalings and the two SpMVs still run, as they do in init for a start vector that was not given: one code path.
+void cuadmm_solver::load_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                              const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig) {
     // this rank's C triplets at local offsets (sharded: the owned svec ranges only)
     std::vector<int32_t> lci; std::vector<double> lcv;
     const int32_t* ci = C_idx; const double* cv = C_val; int64_t cn = C_nnz;
@@ -983,29 +932,17 @@ void cuadmm_solver::update_data(const int32_t* b_idx, const double* b_val, int64
     norm_borg = h_st->norm_borg; norm_Corg = h_st->norm_Corg;
 
     // scaled b and C; the start point
-    const int gv = ew_grid(nloc, device), gm = ew_grid(con_num, device);
-    scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, bd.p, normA.p, 1.0 / bscale, 1);
-    scale_kernel<<<gv, 256, 0, stream>>>(nloc, Cd.p, 1.0 / Cscale);
+    scale_vec_kernel<<<ew_grid(con_num, device), 256, 0, stream>>>(con_num, bd.p, normA.p, 1.0 / bscale, 1);
+    scale_kernel<<<ew_grid(nloc, device), 256, 0, stream>>>(nloc, Cd.p, 1.0 / Cscale);
     launches += 2;
-    if (keep_iterate) {
-        if (iterate_scaled) {     // no solve since init / the last update: back to unscaled with the scales it was made with
-            scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, bscale_old);
-            scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, Cscale_old, 1);
-            scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cscale_old);
-            launches += 3;
-        }
-        // the rescaling of solve(if_first = 0) and of init's X0, y0, S0
-        scale_vec_kernel<<<gm, 256, 0, stream>>>(con_num, y.p, normA.p, 1.0 / Cscale, 0);
-        scale_kernel<<<gv, 256, 0, stream>>>(nloc, X.p, 1.0 / bscale);
-        scale_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, 1.0 / Cscale);
-        launches += 3;
-    } else {
+    if (!keep_iterate) {
         X.zero(stream); y.zero(stream); S.zero(stream);
         CUADMM_CUDA(cudaStreamSynchronize(stream));
         plan->reset_warm_start();   // identity bases, as a new plan has them
+    } else if (iterate_scaled) {    // no solve since init / the last update: back to unscaled with the scales it was made with
+        unscale_iterate(bscale_old, Cscale_old);
     }
-    sub_kernel<<<gv, 256, 0, stream>>>(nloc, S.p, Cd.p, SmC.p);
-    ++launches;
+    scale_iterate_in();
 
     // Rd = A^T y - C + S with |Rd|^2 and <C, X> (mode 3 with tau sig = 0 leaves X as it is), then Rp = b - A X with
     // |normA .* Rp|^2 and <b, y> (K8), then the state; sharded: summed over ranks like the iteration's K7 / K8 scalars
@@ -1032,7 +969,6 @@ void cuadmm_solver::update_data(const int32_t* b_idx, const double* b_val, int64
     iterate_scaled = true;
     info_iter_num = 0;
     for (auto& v : h_hist) v.clear();
-    update_time = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1140,19 +1076,10 @@ int cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* h
     return guarded([&] {
         CUADMM_REQUIRE(s && s->initialised, "solver not initialised");
         CUADMM_CUDA(cudaSetDevice(s->device));
-        std::vector<double> lx, ls;
-        if (s->world > 1) {
-            if (h_X) { s->shard.slice_vec(h_X, lx); h_X = lx.data(); }
-            if (h_S) { s->shard.slice_vec(h_S, ls); h_S = ls.data(); }
-        }
-        if (h_X) s->X.upload(h_X, s->nloc, s->stream);
-        if (h_y) s->y.upload(h_y, s->con_num, s->stream);
-        if (h_S) s->S.upload(h_S, s->nloc, s->stream);
-        s->asmc_valid = false;
-        s->iterate_scaled = false;
+        s->set_iterate(h_X, h_y, h_S);
         s->h_st->sig = sig;                 // pinned mirror: stays valid until the copy below has run
         CUADMM_CUDA(cudaMemcpyAsync(&s->st.p->sig, &s->h_st->sig, sizeof(double), cudaMemcpyHostToDevice, s->stream));
-        CUADMM_CUDA(cudaStreamSynchronize(s->stream));      // the caller's host buffers may be reused on return
+        CUADMM_CUDA(cudaStreamSynchronize(s->stream));
     });
 }
 

@@ -101,6 +101,15 @@ struct cuadmm_solver {
     // new b and C on the same A and blocks; every device buffer is written in place (the graphs hold the pointers)
     void update_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
                      const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig);
+    void check_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                    const int32_t* C_idx, const double* C_val, int64_t C_nnz) const;
+    // b, C, their scales, the scaled start point and the initial residual state, on the device (init and update_data)
+    void load_data(const int32_t* b_idx, const double* b_val, int64_t b_nnz,
+                   const int32_t* C_idx, const double* C_val, int64_t C_nnz, bool keep_iterate, double sig);
+    void set_iterate(const double* h_X, const double* h_y, const double* h_S);
+    void scale_iterate_in();
+    void unscale_iterate(double bs, double Cs);
+    void enqueue_k1(bool asmc_cached);
     void enqueue_iteration(int iter, int switch_admm, bool prof = false);
     void run_iterations(int n_iters, bool sgs, bool profile, double out_ms[8]);
     void enqueue_half_step();

@@ -211,8 +211,9 @@ int  cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* 
  *                     X0 / y0 / S0 (the Jacobi warm-start bases are reset to the identity);
  *   keep_iterate = 1: the start point is the X, y, S the last solve returned, as if given to a fresh init as
  *                     X0 / y0 / S0 (the Jacobi bases are kept, so agreement with that init is to rounding).
- * The residuals and scales are computed on the device, in another order than init's host loops: a cold update
- * agrees with a fresh init to rounding, not bit for bit.  Its wall time is cuadmm_solver_times out[6]. */
+ * init loads b and C through the same device path, so a cold update agrees with a fresh init bit for bit unless a
+ * block takes the dense sign path (n > 168), which is not reproducible run to run.  Its wall time is
+ * cuadmm_solver_times out[6]. */
 int  cuadmm_solver_update_data(cuadmm_solver_t* s,
         const int32_t* b_idx, const double* b_vals, int64_t b_nnz,
         const int32_t* C_idx, const double* C_vals, int64_t C_nnz,
