@@ -291,17 +291,16 @@ void chol_symbolic(const SymCsc& M, const std::vector<int32_t>& perm, CholFactor
     if (permuted) *permuted = std::move(C);
 }
 
-std::vector<int32_t> postorder_perm(const SymCsc& M, const std::vector<int32_t>& perm) {
-    CholFactor F;
-    chol_symbolic(M, perm, F, nullptr);
-    const int64_t n = F.n;
+// post[k] = the k-th node of a postorder of the forest `parent` (-1 = root): roots and children in ascending order
+static std::vector<int32_t> forest_postorder(const std::vector<int32_t>& parent) {
+    const int64_t n = (int64_t)parent.size();
     // children lists (ascending), iterative DFS
     std::vector<int32_t> head(n, -1), nxt(n, -1);
-    for (int64_t j = n - 1; j >= 0; --j) if (F.parent[j] >= 0) { nxt[j] = head[F.parent[j]]; head[F.parent[j]] = (int32_t)j; }
+    for (int64_t j = n - 1; j >= 0; --j) if (parent[j] >= 0) { nxt[j] = head[parent[j]]; head[parent[j]] = (int32_t)j; }
     std::vector<int32_t> post; post.reserve(n);
     std::vector<int32_t> stack;
     for (int64_t r = 0; r < n; ++r) {
-        if (F.parent[r] >= 0) continue;
+        if (parent[r] >= 0) continue;
         stack.push_back((int32_t)r);
         while (!stack.empty()) {
             const int32_t v = stack.back();
@@ -310,9 +309,75 @@ std::vector<int32_t> postorder_perm(const SymCsc& M, const std::vector<int32_t>&
             else { post.push_back(v); stack.pop_back(); }
         }
     }
-    std::vector<int32_t> out(n);
-    for (int64_t k = 0; k < n; ++k) out[k] = perm[post[k]];
+    return post;
+}
+
+std::vector<int32_t> postorder_perm(const SymCsc& M, const std::vector<int32_t>& perm) {
+    CholFactor F;
+    chol_symbolic(M, perm, F, nullptr);
+    const std::vector<int32_t> post = forest_postorder(F.parent);
+    std::vector<int32_t> out(F.n);
+    for (int64_t k = 0; k < F.n; ++k) out[k] = perm[post[k]];
     return out;
+}
+
+// the rows that go to the dense tail: the deep, narrow end of the forward solve's dependency DAG.  Returns the
+// first level of the tail (> depth: no tail) and every row's level.
+static int64_t choose_tail(const CholFactor& F, std::vector<int32_t>& level_out) {
+    const int64_t n = F.n;
+    std::vector<int32_t> lev(n, 0);
+    for (int64_t j = 0; j < n; ++j)
+        for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p) lev[F.Li[p]] = std::max(lev[F.Li[p]], lev[j] + 1);
+    level_out = lev;
+    int depth = 0;
+    for (int64_t i = 0; i < n; ++i) depth = std::max(depth, lev[i] + 1);
+    int64_t max_tail = 10240;
+    int min_depth = 64;
+    if (const char* e = getenv("CUADMM_YSOLVE_MAX_TAIL")) max_tail = atoll(e);
+    if (const char* e = getenv("CUADMM_YSOLVE_MIN_DEPTH")) min_depth = atoi(e);
+    if (depth <= min_depth || max_tail <= 0) return depth + 1;       // no tail
+    std::vector<int64_t> cnt(depth + 1, 0);
+    for (int64_t i = 0; i < n; ++i) cnt[lev[i]]++;
+    // smallest cut >= min_depth/2 with count(level >= cut) <= max_tail
+    int64_t above = 0;
+    int cut = depth;
+    for (int l = depth - 1; l >= min_depth / 2; --l) {
+        if (above + cnt[l] > max_tail) break;
+        above += cnt[l];
+        cut = l;
+    }
+    if (above < 32) return depth + 1;   // a tiny tail is not worth a dense stage
+    return cut;
+}
+
+int64_t order_tail_last(const SymCsc& M, CholFactor& F, SymCsc& C) {
+    const int64_t m = M.n;
+    std::vector<int32_t> perm0 = min_degree_order(M);
+    F = CholFactor();
+    chol_symbolic(M, perm0, F, nullptr);
+    std::vector<int32_t> lev;
+    const int64_t cut = choose_tail(F, lev);
+    std::vector<int32_t> perm1; perm1.reserve(m);
+    for (int64_t k = 0; k < m; ++k) if (lev[k] < cut) perm1.push_back(F.perm[k]);
+    const int64_t n_lead = (int64_t)perm1.size();
+    for (int64_t k = 0; k < m; ++k) if (lev[k] >= cut) perm1.push_back(F.perm[k]);
+    if (n_lead < m) {
+        F = CholFactor();
+        chol_symbolic(M, perm1, F, &C);
+    } else {
+        chol_symbolic(M, perm0, F, &C);
+    }
+    return n_lead;
+}
+
+std::vector<int32_t> tail_postorder(const CholFactor& F, int64_t n_lead) {
+    const int64_t r = F.n - n_lead;
+    std::vector<int32_t> parent(r);
+    for (int64_t i = 0; i < r; ++i) parent[i] = F.parent[n_lead + i] >= 0 ? (int32_t)(F.parent[n_lead + i] - n_lead) : -1;
+    const std::vector<int32_t> post = forest_postorder(parent);
+    std::vector<int32_t> pos(r);
+    for (int64_t k = 0; k < r; ++k) pos[post[k]] = (int32_t)k;
+    return pos;
 }
 
 std::vector<int64_t> find_supernodes(const CholFactor& F, int64_t max_size) {

@@ -48,6 +48,16 @@ std::vector<int64_t> find_supernodes(const CholFactor& F, int64_t max_size);
 
 // symbolic (pattern + etree) only: fills everything but Lx
 void chol_symbolic(const SymCsc& M, const std::vector<int32_t>& perm, CholFactor& F, SymCsc* permuted = nullptr);
+
+// The y-solve's ordering: minimum degree, then the deep, narrow end of the forward solve's dependency DAG (at most
+// CUADMM_YSOLVE_MAX_TAIL rows, default 10,240) moved last as the dense tail.  Fills the symbolic factor F of that
+// order and the permuted matrix C; returns n_lead, the number of rows before the tail.
+int64_t order_tail_last(const SymCsc& M, CholFactor& F, SymCsc& C);
+
+// Postorder of the tail's elimination tree (F.parent restricted to rows >= n_lead): pos[i] = new index of tail
+// row n_lead + i.  Descendants come before ancestors and every subtree is contiguous, so the structure of
+// L22^-1 (entry (i, j) only when j is a descendant of i) stays lower triangular and gathers near the diagonal.
+std::vector<int32_t> tail_postorder(const CholFactor& F, int64_t n_lead);
 // numeric up-looking factorisation of rows [0, n_lead); for rows >= n_lead only the entries in
 // columns < n_lead are computed (the trailing Schur complement is left to the caller).
 // Pivots <= pivot_tol() * M_kk mark redundant constraints (see chol_host.cpp), they do not throw.

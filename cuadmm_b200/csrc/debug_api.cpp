@@ -100,4 +100,21 @@ int cuadmm_debug_chol_solve(int64_t m, int64_t ncols, const int32_t* rowptr, con
     });
 }
 
+// The y-solve's dense-tail relabelling, on the host: the ordering of ysolve_create (order_tail_last) and the postorder of
+// the tail's elimination tree (tail_postorder).  Outputs *n_lead and, for the r = m - n_lead tail rows, parent[i] (the
+// etree parent of tail row i as a tail index, -1 for a root) and pos[i] (its new index).  parent and pos hold m entries.
+int cuadmm_debug_tail_order(int64_t m, int64_t ncols, const int32_t* rowptr, const int32_t* colind, const double* val,
+                            double eps, int64_t* n_lead, int32_t* parent, int32_t* pos) {
+    return guarded([&] {
+        CUADMM_REQUIRE(rowptr && n_lead && parent && pos, "null argument");
+        SymCsc M = form_aat(m, ncols, rowptr, colind, val, eps);
+        CholFactor F; SymCsc C;
+        *n_lead = order_tail_last(M, F, C);
+        const int64_t r = m - *n_lead;
+        for (int64_t i = 0; i < r; ++i) parent[i] = F.parent[*n_lead + i] >= 0 ? (int32_t)(F.parent[*n_lead + i] - *n_lead) : -1;
+        const std::vector<int32_t> p = tail_postorder(F, *n_lead);
+        std::copy(p.begin(), p.end(), pos);
+    });
+}
+
 }  // extern "C"

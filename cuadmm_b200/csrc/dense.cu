@@ -222,34 +222,57 @@ __global__ void scatter_coo_kernel(int64_t nnz, const int32_t* __restrict__ r, c
     if (symmetric && r[e] != c[e]) D[c[e] + (int64_t)r[e] * ld] = v[e];
 }
 
-__global__ void transpose_kernel(int64_t n, const double* __restrict__ in, double* __restrict__ out) {
-    __shared__ double tile[32][33];
-    const int64_t bx = (int64_t)blockIdx.x * 32, by = (int64_t)blockIdx.y * 32;
-    for (int j = threadIdx.y; j < 32; j += blockDim.y) {
-        const int64_t x = bx + threadIdx.x, y = by + j;
-        if (x < n && y < n) tile[j][threadIdx.x] = in[x + y * n];
-    }
-    __syncthreads();
-    for (int j = threadIdx.y; j < 32; j += blockDim.y) {
-        const int64_t x = by + threadIdx.x, y = bx + j;
-        if (x < n && y < n) out[x + y * n] = tile[threadIdx.x][j];
-    }
-}
-
-// which 64 x 64 tiles of a row-major r x r matrix hold a non-zero
-__global__ void tile_occupancy_kernel(int64_t r, int nt, const double* __restrict__ A, int* __restrict__ flags) {
+// which 64 x 64 tiles of P L P^T hold a non-zero (L column-major r x r, ipos[new] = old)
+__global__ void tile_occupancy_kernel(int64_t r, int nt, const double* __restrict__ L, const int32_t* __restrict__ ipos,
+                                      int* __restrict__ flags) {
     const int I = blockIdx.y, J = blockIdx.x;
     int any = 0;
     for (int e = threadIdx.x; e < 64 * 64; e += blockDim.x) {
-        const int64_t i = (int64_t)I * 64 + e / 64, j = (int64_t)J * 64 + e % 64;
-        if (i < r && j < r && A[i * r + j] != 0.0) any = 1;
+        const int64_t i = (int64_t)I * 64 + e % 64, j = (int64_t)J * 64 + e / 64;
+        if (i < r && j < r && L[ipos[i] + (int64_t)ipos[j] * r] != 0.0) any = 1;
     }
     if (__syncthreads_or(any) && threadIdx.x == 0) flags[I * nt + J] = 1;
 }
 
-void build_dense_tail(const SymCsc& C, const CholFactor& F, int64_t n_lead, int64_t r,
-                      DevBuf<double>& tail_inv, DevBuf<double>& tail_inv_t, int64_t* n_deficient,
-                      std::vector<int>* tile_flags) {
+void tile_occupancy(int64_t r, const double* L, const int32_t* ipos, std::vector<int>& flags) {
+    cudaStream_t st = 0;
+    const int nt = (int)((r + 63) / 64);
+    DevBuf<int> d((int64_t)nt * nt);
+    d.zero(st);
+    tile_occupancy_kernel<<<dim3(nt, nt), 256, 0, st>>>(r, nt, L, ipos, d.p);
+    CUADMM_CUDA(cudaGetLastError());
+    flags.resize((size_t)nt * nt);
+    d.download(flags.data(), (int64_t)flags.size(), st);
+    CUADMM_CUDA(cudaStreamSynchronize(st));
+}
+
+// one CTA per tile: tile (I, J) of P L P^T (or of its transpose) -> out[dst + i * w + j], zeros outside the r x r matrix
+__global__ void pack_tiles_kernel(int64_t r, const double* __restrict__ L, const int32_t* __restrict__ ipos, int transpose,
+                                  const int64_t* __restrict__ tiles, double* __restrict__ out) {
+    const int64_t* t = tiles + 4 * (int64_t)blockIdx.x;
+    const int64_t I = t[0], J = t[1], dst = t[2], w = t[3];
+    for (int e = threadIdx.x; e < 64 * 64; e += blockDim.x) {
+        const int i = e / 64, j = e % 64;
+        const int64_t a = I * 64 + i, b = J * 64 + j;
+        double v = 0.0;
+        if (a < r && b < r) v = transpose ? L[ipos[b] + (int64_t)ipos[a] * r] : L[ipos[a] + (int64_t)ipos[b] * r];
+        out[dst + i * w + j] = v;
+    }
+}
+
+void pack_tiles(int64_t r, const double* L, const int32_t* ipos, bool transpose, const std::vector<int64_t>& tiles, double* out) {
+    cudaStream_t st = 0;
+    const int64_t n = (int64_t)tiles.size() / 4;
+    if (n == 0) return;
+    DevBuf<int64_t> d;
+    d.upload(tiles, st);
+    pack_tiles_kernel<<<(unsigned)n, 256, 0, st>>>(r, L, ipos, transpose ? 1 : 0, d.p, out);
+    CUADMM_CUDA(cudaGetLastError());
+    CUADMM_CUDA(cudaStreamSynchronize(st));
+}
+
+void build_dense_tail(const SymCsc& C, const CholFactor& F, int64_t n_lead, int64_t r, DevBuf<double>& tail_inv,
+                      int64_t* n_deficient) {
     cudaStream_t st = 0;
     // S <- M22 (both triangles)
     DevBuf<double> S(r * r);
@@ -304,30 +327,8 @@ void build_dense_tail(const SymCsc& C, const CholFactor& F, int64_t n_lead, int6
     info.download(&h_info, 1, st);
     CUADMM_CUDA(cudaStreamSynchronize(st));
     if (n_deficient) *n_deficient = h_info;
-    tail_inv_t.alloc(r * r);       // column-major L22^-1 == row-major L22^-T
-    trtri_lower(st, r, S.p, r, inv_diag.p, tail_inv_t.p, r);
-    tail_inv.alloc(r * r);         // row-major L22^-1
-    dim3 grid((unsigned)((r + 31) / 32), (unsigned)((r + 31) / 32)), block(32, 8);
-    transpose_kernel<<<grid, block, 0, st>>>(r, tail_inv_t.p, tail_inv.p);
-    CUADMM_CUDA(cudaGetLastError());
-    CUADMM_CUDA(cudaStreamSynchronize(st));
-    // which 64 x 64 tiles of L22^-1 hold anything: the GEMVs skip the empty ones
-    {
-        const int nt = (int)((r + 63) / 64);
-        DevBuf<int> flags((int64_t)nt * nt);
-        flags.zero(st);
-        tile_occupancy_kernel<<<dim3(nt, nt), 256, 0, st>>>(r, nt, tail_inv.p, flags.p);
-        std::vector<int> h((size_t)nt * nt);
-        flags.download(h.data(), (int64_t)h.size(), st);
-        CUADMM_CUDA(cudaStreamSynchronize(st));
-        if (getenv("CUADMM_YSOLVE_VERBOSE")) {
-            int64_t lower = 0, used = 0;
-            for (int I = 0; I < nt; ++I) for (int J = 0; J <= I; ++J) { ++lower; used += h[(size_t)I * nt + J]; }
-            fprintf(stderr, "[ysolve] dense tail %lld: %lld of %lld lower 64x64 tiles of L22^-1 are non-zero (%.1f%%)\n",
-                    (long long)r, (long long)used, (long long)lower, 100.0 * (double)used / (double)lower);
-        }
-        if (tile_flags) tile_flags->swap(h);
-    }
+    tail_inv.alloc(r * r);
+    trtri_lower(st, r, S.p, r, inv_diag.p, tail_inv.p, r);
 }
 
 }  // namespace cuadmm

@@ -20,9 +20,14 @@ void potrf_lower(cudaStream_t st, int64_t n, double* A, int64_t lda, double* inv
 // Linv = L^-1 for lower-triangular L (strict upper of Linv zeroed); needs inv_diag from potrf_lower
 void trtri_lower(cudaStream_t st, int64_t n, const double* L, int64_t ldl, const double* inv_diag, double* Linv, int64_t ldi);
 
-// y-solve: dense trailing block.  tail_inv = row-major L22^-1, tail_inv_t = row-major L22^-T.
-void build_dense_tail(const SymCsc& Cperm, const CholFactor& F, int64_t n_lead, int64_t n_tail,
-                      DevBuf<double>& tail_inv, DevBuf<double>& tail_inv_t, int64_t* n_deficient = nullptr,
-                      std::vector<int>* tile_flags = nullptr);   // nt x nt, row-major, of tail_inv (nt = ceil(n_tail / 64))
+// y-solve: dense trailing block.  tail_inv = column-major L22^-1 (n_tail x n_tail), in the order of F.
+void build_dense_tail(const SymCsc& Cperm, const CholFactor& F, int64_t n_lead, int64_t n_tail, DevBuf<double>& tail_inv,
+                      int64_t* n_deficient = nullptr);
+// flags (nt x nt row-major, nt = ceil(r / 64)): which 64 x 64 tiles of P L P^T hold a non-zero, for L column-major
+// r x r on the device and ipos (device, r entries) = P's map from new to old index
+void tile_occupancy(int64_t r, const double* L, const int32_t* ipos, std::vector<int>& flags);
+// tiles = (I, J, dst, w) per tile: tile (I, J) of P L P^T, or of (P L P^T)^T when transpose, is copied to
+// out[dst + i * w + j] (i, j < 64); entries outside the r x r matrix are written as zeros
+void pack_tiles(int64_t r, const double* L, const int32_t* ipos, bool transpose, const std::vector<int64_t>& tiles, double* out);
 
 }  // namespace cuadmm

@@ -431,50 +431,39 @@ __global__ void __launch_bounds__(kPkWarpThreads, 5) tri_packed_warp_kernel(int6
     }
 }
 
-// dense tail: out[i] = sum_j T[i, j] * in[j] for a row-major r x r triangular matrix (L22^-1 or its
-// transpose).  One warp per row, coalesced; only the 64-column tiles listed for the row's tile row
-// are read (tile_ptr / tile_col: per tile row, runs of consecutive non-empty tiles as column
-// ranges): the inverse of the trailing factor block inherits
-// the block structure of the separators it came from and is often half empty.
-// dense tail, single GPU: out[i] = sum_j T[i, j] * in[j] for a row-major r x r triangular matrix (L22^-1 or its
-// transpose).  One warp per row, coalesced; only the 64-column tiles listed for the row's tile row
-// are read (tile_ptr / tile_col: per tile row, runs of consecutive non-empty tiles as column
-// ranges): the inverse of the trailing factor block inherits
-// the block structure of the separators it came from and is often half empty.
+// dense tail, single GPU: out[i] = sum_j T[i, j] * in[j] for an r x r triangular matrix (L22^-1 or its transpose) in
+// tile-run storage (TailMatrix): per 64-row tile row, tile_ptr / tile_col list the runs of consecutive non-empty
+// 64 x 64 tiles as [first, last) columns, and run t sits at T + tile_off[t], 64 rows of its full width.  Only those
+// tiles are read.  One warp per row, coalesced 16-byte loads (run widths and offsets are multiples of 64 doubles).
+// blk_order lists the 8-row blocks longest rows first, so the grid's tail wave is made of short rows.
 __global__ void __launch_bounds__(256) tail_gemv_row_kernel(int64_t r, const double* __restrict__ T, const double* __restrict__ in,
                                                         double* out, const int32_t* __restrict__ tile_ptr,
-                                                        const int32_t* __restrict__ tile_col, double* out_scatter,
+                                                        const int32_t* __restrict__ tile_col, const int64_t* __restrict__ tile_off,
+                                                        const int32_t* __restrict__ blk_order, double* out_scatter,
                                                         const int32_t* __restrict__ out_perm, int64_t perm_base,
-                                                        const int* __restrict__ done_flag, int longest_last) {
+                                                        const int* __restrict__ done_flag) {
     if (done_flag && *done_flag) return;
     const int lane = threadIdx.x & 31;
-    // the CTAs with the longest rows go first (lower-triangular storage: the last rows), so the grid's tail
-    // wave is made of short rows
-    const int64_t cta = longest_last ? (int64_t)gridDim.x - 1 - blockIdx.x : blockIdx.x;
-    const int64_t row = cta * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int64_t row = (int64_t)blk_order[blockIdx.x] * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (row >= r) return;
-    const double* Ti = T + row * r;
     const int I = (int)(row >> 6);
     double acc0 = 0.0, acc1 = 0.0;
-    const bool vec = (r & 1) == 0 && (reinterpret_cast<uintptr_t>(T) & 15) == 0;   // rows 16-byte aligned (tile columns are multiples of 64)
     const bool in_al = (reinterpret_cast<uintptr_t>(in) & 15) == 0;
-    for (int t = tile_ptr[I]; t < tile_ptr[I + 1]; ++t) {      // runs of consecutive non-empty tiles: [first, last) columns
+    for (int t = tile_ptr[I]; t < tile_ptr[I + 1]; ++t) {
         const int64_t j0 = tile_col[2 * t];
-        const int64_t j1 = min((int64_t)tile_col[2 * t + 1], r);
-        if (vec) {
-            const int64_t jv = j0 + ((j1 - j0) & ~(int64_t)1);
+        const int64_t w = tile_col[2 * t + 1] - j0;
+        const int64_t n = min(w, r - j0);                        // columns of the run inside the matrix
+        const int64_t nv = n & ~(int64_t)1;
+        const double* Ti = T + tile_off[t] + (row & 63) * w;
+        const double* x = in + j0;
 #pragma unroll 4      // measured: 8 or 16 loads in flight per lane are 7-8 % slower per solve (fewer resident warps)
-            for (int64_t j = j0 + 2 * lane; j < jv; j += 64) {
-                const double2 a = __ldcs(reinterpret_cast<const double2*>(Ti + j));   // streamed once: evict first
-                const double2 b = in_al ? *reinterpret_cast<const double2*>(in + j) : make_double2(in[j], in[j + 1]);
-                acc0 = fma(a.x, b.x, acc0);
-                acc1 = fma(a.y, b.y, acc1);
-            }
-            if (lane == 0 && jv < j1) acc0 = fma(Ti[jv], in[jv], acc0);
-        } else {
-#pragma unroll 4
-            for (int64_t j = j0 + lane; j < j1; j += 32) acc0 = fma(Ti[j], in[j], acc0);
+        for (int64_t k = 2 * lane; k < nv; k += 64) {
+            const double2 a = __ldcs(reinterpret_cast<const double2*>(Ti + k));   // streamed once: evict first
+            const double2 b = in_al ? *reinterpret_cast<const double2*>(x + k) : make_double2(x[k], x[k + 1]);
+            acc0 = fma(a.x, b.x, acc0);
+            acc1 = fma(a.y, b.y, acc1);
         }
+        if (lane == 0 && nv < n) acc0 = fma(Ti[nv], x[nv], acc0);
     }
     double acc = acc0 + acc1;
 #pragma unroll
@@ -498,11 +487,13 @@ __global__ void __launch_bounds__(256) tail_gemv_row_kernel(int64_t r, const dou
 // peer_leave handshake, so when it retires every rank holds the complete vector.  No peer_enter is needed: a peer
 // can only reach this kernel after the handshake of the previous one, which this rank joined after its last read of
 // the buffers.  row0 is a multiple of 8, so the 8 rows of a CTA share one 64-row tile row (= one list of column runs).
+// Storage as in tail_gemv_row_kernel; blk_order lists this launch's 8-row blocks (from row0), longest rows first.
 __global__ void __launch_bounds__(256) tail_gemv_kernel(int64_t r, const double* __restrict__ T, const double* in,
                                                         double* out, const int32_t* __restrict__ tile_ptr,
-                                                        const int32_t* __restrict__ tile_col, double* out_scatter,
+                                                        const int32_t* __restrict__ tile_col, const int64_t* __restrict__ tile_off,
+                                                        const int32_t* __restrict__ blk_order, double* out_scatter,
                                                         const int32_t* __restrict__ out_perm, int64_t perm_base,
-                                                        const int* __restrict__ done_flag, int longest_last,
+                                                        const int* __restrict__ done_flag,
                                                         int64_t row0, int64_t nrows, int npush, PeerView pv,
                                                         PeerPtrs outp, PeerPtrs scatp, int splits, double* split_part,
                                                         unsigned int* split_count) {
@@ -516,54 +507,53 @@ __global__ void __launch_bounds__(256) tail_gemv_kernel(int64_t r, const double*
     // the rows is too few CTAs to pull its share of the bytes at one CTA per row block (measured 20 us for 1/8 of the
     // rows).  The CTA that finds the other partials written adds them in split order (bit-identical on every rank).
     const int sp = (int)(blockIdx.x % (unsigned)splits);
-    const int64_t rb = blockIdx.x / (unsigned)splits, nrb = gridDim.x / (unsigned)splits;
-    // the row blocks with the longest rows go first (lower-triangular storage: the last rows), so the grid's tail
-    // wave is made of short rows
-    const int64_t cta = longest_last ? nrb - 1 - rb : rb;
-    const int64_t base = row0 + cta * 8;
+    const int64_t rb = blockIdx.x / (unsigned)splits;
+    const int64_t base = row0 + (int64_t)blk_order[rb] * 8;
     const int nr = (int)max((int64_t)0, min((int64_t)8, row0 + nrows - base));     // rows of this CTA
     double acc[8];
 #pragma unroll
     for (int q = 0; q < 8; ++q) acc[q] = 0.0;
     if (nr > 0) {
         const int I = (int)(base >> 6);
-        const bool vec = (r & 1) == 0 && (reinterpret_cast<uintptr_t>(T) & 15) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0;
-        const double* Tb = T + base * r;
+        const bool vec = (reinterpret_cast<uintptr_t>(in) & 15) == 0;   // run rows are 16-byte aligned
         int g = 0;                                        // running chunk index over the runs of this tile row
         for (int t = tile_ptr[I]; t < tile_ptr[I + 1]; ++t) {
             const int64_t j0 = tile_col[2 * t];
-            const int64_t j1 = min((int64_t)tile_col[2 * t + 1], r);
-            const int nch = (int)((j1 - j0 + 63) >> 6);
+            const int64_t rw = tile_col[2 * t + 1] - j0;              // run width (row stride of the run)
+            const int64_t n = min(rw, r - j0);                        // columns of the run inside the matrix
+            const double* Tb = T + tile_off[t] + (base & 63) * rw;    // Tb[q * rw + k]: row base + q, column j0 + k
+            const double* x = in + j0;
+            const int nch = (int)((n + 63) >> 6);
             // chunk with running index G = g + c belongs to warp G & 7 of split (G >> 3) % splits
             const int g0 = g;
             int c = (w - (g & 7)) & 7;
             g += nch;
             for (; c < nch; c += 8) {
                 if (splits > 1 && (((g0 + c) >> 3) % splits) != sp) continue;
-                const int64_t j = j0 + ((int64_t)c << 6) + 2 * lane;
+                const int64_t k = ((int64_t)c << 6) + 2 * lane;
                 if (vec) {
-                    if (j + 1 < j1) {
-                        const double2 b = *reinterpret_cast<const double2*>(in + j);
+                    if (k + 1 < n) {
+                        const double2 b = *reinterpret_cast<const double2*>(x + k);
 #pragma unroll
                         for (int q = 0; q < 8; ++q) {
                             if (q < nr) {
-                                const double2 a = __ldcs(reinterpret_cast<const double2*>(Tb + q * r + j));   // streamed once
+                                const double2 a = __ldcs(reinterpret_cast<const double2*>(Tb + q * rw + k));   // streamed once
                                 acc[q] = fma(a.x, b.x, fma(a.y, b.y, acc[q]));
                             }
                         }
-                    } else if (j < j1) {
-                        const double b = in[j];
+                    } else if (k < n) {
+                        const double b = x[k];
 #pragma unroll
-                        for (int q = 0; q < 8; ++q) if (q < nr) acc[q] = fma(Tb[q * r + j], b, acc[q]);
+                        for (int q = 0; q < 8; ++q) if (q < nr) acc[q] = fma(Tb[q * rw + k], b, acc[q]);
                     }
                 } else {
 #pragma unroll
                     for (int h = 0; h < 2; ++h) {
-                        const int64_t jj = j0 + ((int64_t)c << 6) + lane + 32 * h;
-                        if (jj < j1) {
-                            const double b = in[jj];
+                        const int64_t kk = ((int64_t)c << 6) + lane + 32 * h;
+                        if (kk < n) {
+                            const double b = x[kk];
 #pragma unroll
-                            for (int q = 0; q < 8; ++q) if (q < nr) acc[q] = fma(Tb[q * r + jj], b, acc[q]);
+                            for (int q = 0; q < 8; ++q) if (q < nr) acc[q] = fma(Tb[q * rw + kk], b, acc[q]);
                         }
                     }
                 }
@@ -1179,32 +1169,97 @@ static int64_t choose_subtrees(const CholFactor& F, int64_t n_lead, std::vector<
     return n_sub;
 }
 
-// choose the rows that go to the dense tail: the deep, narrow end of the elimination DAG.
-static int64_t choose_tail(const CholFactor& F, std::vector<int32_t>& level_out) {
-    const int64_t n = F.n;
-    std::vector<int32_t> lev(n, 0);
-    for (int64_t j = 0; j < n; ++j)
-        for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p) lev[F.Li[p]] = std::max(lev[F.Li[p]], lev[j] + 1);
-    level_out = lev;
-    int depth = 0;
-    for (int64_t i = 0; i < n; ++i) depth = std::max(depth, lev[i] + 1);
-    int64_t max_tail = 10240;
-    int min_depth = 64;
-    if (const char* e = getenv("CUADMM_YSOLVE_MAX_TAIL")) max_tail = atoll(e);
-    if (const char* e = getenv("CUADMM_YSOLVE_MIN_DEPTH")) min_depth = atoi(e);
-    if (depth <= min_depth || max_tail <= 0) return depth + 1;       // no tail
-    std::vector<int64_t> cnt(depth + 1, 0);
-    for (int64_t i = 0; i < n; ++i) cnt[lev[i]]++;
-    // smallest cut >= min_depth/2 with count(level >= cut) <= max_tail
-    int64_t above = 0;
-    int cut = depth;
-    for (int l = depth - 1; l >= min_depth / 2; --l) {
-        if (above + cnt[l] > max_tail) break;
-        above += cnt[l];
-        cut = l;
+// the 8-row blocks of rows [row0, row0 + nrows) (row0 a multiple of 8), counted from row0, longest rows first
+static std::vector<int32_t> longest_first(const std::vector<double>& cost, int64_t row0, int64_t nrows) {
+    std::vector<int32_t> b((size_t)std::max<int64_t>(1, (nrows + 7) / 8));
+    std::iota(b.begin(), b.end(), 0);
+    if (nrows > 0)
+        std::stable_sort(b.begin(), b.end(), [&](int32_t x, int32_t y) { return cost[(row0 + 8 * x) >> 6] > cost[(row0 + 8 * y) >> 6]; });
+    return b;
+}
+
+// Tile-run storage (TailMatrix) of L = P L22^-1 P^T (lower) or of L^T, from the occupancy flags of L.  Linv is L22^-1
+// column-major in F's order, d_ipos P's map from new to old tail index.
+static void pack_tail_matrix(int64_t r, const double* Linv, const int32_t* d_ipos, const std::vector<int>& flags, bool lower,
+                             TailMatrix& T) {
+    const int nt = (int)((r + 63) / 64);
+    std::vector<int32_t> ptr(1, 0), col;
+    std::vector<int64_t> off, tiles;       // tiles: (I, J, destination, row stride) for pack_tiles
+    int64_t size = 0;
+    T.cost.assign(nt, 0.0);
+    for (int I = 0; I < nt; ++I) {
+        const int J0 = lower ? 0 : I, J1 = lower ? I + 1 : nt;
+        auto used = [&](int J) { return flags[lower ? (size_t)I * nt + J : (size_t)J * nt + I] != 0; };
+        for (int J = J0; J < J1;) {
+            if (!used(J)) { ++J; continue; }
+            int E = J;
+            while (E < J1 && used(E)) ++E;
+            const int64_t w = (int64_t)(E - J) * 64;
+            col.push_back(J * 64); col.push_back(E * 64);
+            off.push_back(size);
+            for (int K = J; K < E; ++K) { tiles.push_back(I); tiles.push_back(K); tiles.push_back(size + (K - J) * 64); tiles.push_back(w); }
+            size += 64 * w;
+            T.cost[I] += (double)w;
+            J = E;
+        }
+        ptr.push_back((int32_t)(col.size() / 2));
     }
-    if (above < 32) return depth + 1;   // a tiny tail is not worth a dense stage
-    return cut;
+    if (col.empty()) { col.assign(2, 0); off.push_back(0); }
+    T.val.alloc(std::max<int64_t>(size, 1));
+    pack_tiles(r, Linv, d_ipos, !lower, tiles, T.val.p);
+    T.tptr.upload(ptr); T.tcol.upload(col); T.toff.upload(off);
+    T.order.upload(longest_first(T.cost, 0, r));
+}
+
+// Dense tail.  L22 is factored and inverted in F's order, so its pivots (and pivot floors) are those of that order; the
+// finished inverse is then relabelled symmetrically, tail row i -> pos[i], and only its non-empty 64 x 64 tiles are
+// stored.  L22^-1 (i, j) can be non-zero only when j is a descendant of i in the elimination tree: with pos a
+// postorder of the tail's tree its few non-zeros gather in few tiles near the diagonal (C2b bench operator: 710 of
+// 12,880 lower tiles instead of 8,054 in F's order), and the inverse stays lower triangular.  The numeric tile scan
+// decides what is stored; if it finds a tile above the diagonal, pos falls back to the identity.
+static void build_tail(cuadmm_ysolve_s& Y, const SymCsc& C, const CholFactor& F, std::vector<int32_t>& pos, int64_t* n_def) {
+    const int64_t r = Y.n_tail;
+    const int nt = (int)((r + 63) / 64);
+    DevBuf<double> Linv;                   // r x r: init-time scratch, freed on return
+    build_dense_tail(C, F, Y.n_lead, r, Linv, n_def);
+    DevBuf<int32_t> d_ipos;
+    std::vector<int> flags;
+    auto scan = [&]() {
+        std::vector<int32_t> ipos(r);
+        for (int64_t i = 0; i < r; ++i) ipos[pos[i]] = (int32_t)i;
+        d_ipos.upload(ipos);
+        tile_occupancy(r, Linv.p, d_ipos.p, flags);
+    };
+    auto lower_used = [&]() {
+        int64_t used = 0;
+        for (int I = 0; I < nt; ++I) for (int J = 0; J <= I; ++J) used += flags[(size_t)I * nt + J];
+        return used;
+    };
+    const bool verbose = getenv("CUADMM_YSOLVE_VERBOSE") != nullptr;
+    int64_t used_before = -1;
+    if (verbose) {
+        const std::vector<int32_t> keep(pos);
+        std::iota(pos.begin(), pos.end(), 0);
+        scan();
+        used_before = lower_used();
+        pos = keep;
+    }
+    scan();
+    bool upper = false;
+    for (int I = 0; I < nt && !upper; ++I) for (int J = I + 1; J < nt; ++J) if (flags[(size_t)I * nt + J]) { upper = true; break; }
+    if (upper) {
+        std::iota(pos.begin(), pos.end(), 0);
+        scan();
+    }
+    if (verbose) {
+        const int64_t lower = (int64_t)nt * (nt + 1) / 2, used = lower_used();
+        fprintf(stderr, "[ysolve] dense tail %lld: non-zero lower 64x64 tiles of L22^-1: %lld of %lld (%.1f%%) in the tail order, "
+                "%lld (%.1f%%) stored%s\n", (long long)r, (long long)used_before, (long long)lower,
+                100.0 * (double)used_before / (double)lower, (long long)used, 100.0 * (double)used / (double)lower,
+                upper ? " (postorder left a tile above the diagonal: tail order kept)" : "");
+    }
+    pack_tail_matrix(r, Linv.p, d_ipos.p, flags, true, Y.tail[0]);
+    pack_tail_matrix(r, Linv.p, d_ipos.p, flags, false, Y.tail[1]);
 }
 
 cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const int32_t* rowptr, const int32_t* colind,
@@ -1234,33 +1289,35 @@ cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const in
     SymCsc M = form_aat(m, vec_len, rowptr, colind, val, eps);
     lap("A A^T");
     Y->nnz_aat = M.p[m];
-    std::vector<int32_t> perm0 = min_degree_order(M);
-    lap("minimum-degree ordering");
     CholFactor F;
-    chol_symbolic(M, perm0, F, nullptr);
-    lap("symbolic (1)");
-    std::vector<int32_t> lev;
-    const int64_t cut = choose_tail(F, lev);
-    std::vector<int32_t> perm1; perm1.reserve(m);
-    for (int64_t k = 0; k < m; ++k) if (lev[k] < cut) perm1.push_back(F.perm[k]);
-    const int64_t n_lead = (int64_t)perm1.size();
-    for (int64_t k = 0; k < m; ++k) if (lev[k] >= cut) perm1.push_back(F.perm[k]);
-    const int64_t n_tail = m - n_lead;
     SymCsc C;
-    if (n_tail > 0) {
-        F = CholFactor();
-        chol_symbolic(M, perm1, F, &C);
-    } else {
-        chol_symbolic(M, perm0, F, &C);
-    }
-    lap("symbolic (2, tail last)");
+    const int64_t n_lead = order_tail_last(M, F, C);
+    const int64_t n_tail = m - n_lead;
+    lap("ordering + symbolic (tail last)");
     chol_numeric(C, F, n_lead);
     lap("numeric (sparse lead part)");
     Y->n_lead = n_lead; Y->n_tail = n_tail;
     Y->nnz_L = F.nnz();
     Y->n_deficient = F.n_deficient;
-    Y->h_perm = F.perm;
-    Y->perm.upload(F.perm);
+
+    // ---- dense tail: S = M22 - L21 L21^T, Cholesky, explicit inverse (all on the device), stored relabelled
+    std::vector<int32_t> pos(n_tail);
+    std::iota(pos.begin(), pos.end(), 0);
+    if (n_tail > 0) {
+        const char* e = getenv("CUADMM_YSOLVE_TAIL_POSTORDER");     // "0": keep the tail order (probe of the relabelling)
+        if (!(e && atoi(e) == 0)) pos = tail_postorder(F, n_lead);
+        int64_t tail_def = 0;
+        build_tail(*Y, C, F, pos, &tail_def);
+        Y->n_deficient += tail_def;
+        Y->tail_tmp.alloc(n_tail);
+        lap("dense tail (GPU)");
+    }
+    // The sweeps and perm use the relabelled tail: unknown n_lead + i of F is n_lead + pos[i] here.  Lead unknowns keep
+    // their ids, every row keeps its entries in the same order, so the sweeps do the arithmetic of F's order.
+    auto relabel = [&](int32_t u) { return u < n_lead ? u : (int32_t)(n_lead + pos[u - n_lead]); };
+    Y->h_perm.resize(m);
+    for (int64_t k = 0; k < m; ++k) Y->h_perm[relabel((int32_t)k)] = F.perm[k];
+    Y->perm.upload(Y->h_perm);
 
     std::vector<int32_t> sub;
     const int64_t n_sub = choose_subtrees(F, n_lead, sub);
@@ -1270,13 +1327,13 @@ cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const in
         H.n = m;
         H.ptr.assign(m + 1, 0);
         for (int64_t j = 0; j < n_lead; ++j)
-            for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p) H.ptr[F.Li[p] + 1]++;
+            for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p) H.ptr[relabel(F.Li[p]) + 1]++;
         for (int64_t i = 0; i < m; ++i) H.ptr[i + 1] += H.ptr[i];
         H.dep.resize(H.ptr[m]); H.val.resize(H.ptr[m]);
         std::vector<int64_t> nx(H.ptr.begin(), H.ptr.end() - 1);
         for (int64_t j = 0; j < n_lead; ++j)
             for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p) {
-                const int64_t q = nx[F.Li[p]]++;
+                const int64_t q = nx[relabel(F.Li[p])]++;
                 H.dep[q] = (int32_t)j; H.val[q] = F.Lx[p];
             }
         H.inv_diag.assign(m, 1.0);
@@ -1297,7 +1354,7 @@ cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const in
         H.dep.resize(H.ptr[m]); H.val.resize(H.ptr[m]);
         for (int64_t j = 0; j < n_lead; ++j) {
             int64_t q = H.ptr[j];
-            for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p, ++q) { H.dep[q] = F.Li[p]; H.val[q] = F.Lx[p]; }
+            for (int64_t p = F.Lp[j] + 1; p < F.Lp[j + 1]; ++p, ++q) { H.dep[q] = relabel(F.Li[p]); H.val[q] = F.Lx[p]; }
         }
         H.inv_diag.assign(m, 1.0);
         for (int64_t i = 0; i < n_lead; ++i) H.inv_diag[i] = 1.0 / F.Lx[F.Lp[i]];
@@ -1314,37 +1371,6 @@ cuadmm_ysolve_s* ysolve_create(int64_t m, int64_t vec_len, int64_t nnz, const in
     Y->z.alloc(std::max<int64_t>(m, 1));
     Y->x.alloc(std::max<int64_t>(m, 1));
 
-    // ---- dense tail: S = M22 - L21 L21^T, Cholesky, explicit inverse (all on the device)
-    if (n_tail > 0) {
-        int64_t tail_def = 0;
-        std::vector<int> flags;
-        build_dense_tail(C, F, n_lead, n_tail, Y->tail_inv, Y->tail_inv_t, &tail_def, &flags);
-        const int nt = (int)((n_tail + 63) / 64);
-        std::vector<int32_t> tp(1, 0), tc, tpt(1, 0), tct;
-        auto add_runs = [&](std::vector<int32_t>& ptr, std::vector<int32_t>& col, int J0, int J1, auto used) {
-            for (int J = J0; J < J1;) {
-                if (!used(J)) { ++J; continue; }
-                int E = J;
-                while (E < J1 && used(E)) ++E;
-                col.push_back(J * 64); col.push_back(E * 64);
-                J = E;
-            }
-            ptr.push_back((int32_t)(col.size() / 2));
-        };
-        Y->h_tail_cost[0].assign(nt, 0.0); Y->h_tail_cost[1].assign(nt, 0.0);
-        for (int I = 0; I < nt; ++I) {
-            add_runs(tp, tc, 0, I + 1, [&](int J) { return flags[(size_t)I * nt + J] != 0; });       // L22^-1: lower
-            add_runs(tpt, tct, I, nt, [&](int J) { return flags[(size_t)J * nt + I] != 0; });       // its transpose: upper
-            for (int32_t t = tp[I]; t < tp[I + 1]; ++t) Y->h_tail_cost[0][I] += tc[2 * t + 1] - tc[2 * t];
-            for (int32_t t = tpt[I]; t < tpt[I + 1]; ++t) Y->h_tail_cost[1][I] += tct[2 * t + 1] - tct[2 * t];
-        }
-        if (tc.empty()) tc.assign(2, 0);
-        if (tct.empty()) tct.assign(2, 0);
-        Y->tail_tptr.upload(tp); Y->tail_tcol.upload(tc); Y->tail_tptr_t.upload(tpt); Y->tail_tcol_t.upload(tct);
-        Y->n_deficient += tail_def;
-        Y->tail_tmp.alloc(n_tail);
-        lap("dense tail (GPU)");
-    }
     Y->launches_per_solve = (int)(Y->fwd.phases.size() + Y->bwd.phases.size()) + (n_tail > 0 ? 2 : 0) +
                             (Y->fwd.n_sub_cta > 0 ? 2 : 0) + (Y->fwd.n_sub_warp > 0 ? 2 : 0) + (Y->fwd.n_sub_pack > 0 ? 2 : 0) +
                             (Y->fwd.pk_rows > 0 ? 2 : 0);
@@ -1379,7 +1405,7 @@ void cuadmm_ysolve_s::enable_peer(const PeerComm* pc, size_t off_tmp, size_t off
 // rows of each tail GEMV split into `world` contiguous ranges of equal work (columns read)
 void cuadmm_ysolve_s::split_tail_rows(int world, int rank) {
     for (int k = 0; k < 2; ++k) {
-        const std::vector<double>& c = h_tail_cost[k];
+        const std::vector<double>& c = tail[k].cost;
         double total = 0.0;
         for (int64_t i = 0; i < n_tail; ++i) total += c[i >> 6] + 32.0;
         std::vector<int64_t> cut(world + 1, n_tail);
@@ -1391,6 +1417,7 @@ void cuadmm_ysolve_s::split_tail_rows(int world, int rank) {
             while (q < world && acc >= total * q / world) cut[q++] = std::min<int64_t>(n_tail, (i + 1 + 7) / 8 * 8);   // CTA = 8 rows
         }
         tail_row0[k] = cut[rank]; tail_row1[k] = cut[rank + 1];
+        tail[k].rank_order.upload(longest_first(c, tail_row0[k], tail_row1[k] - tail_row0[k]));
     }
     // scratch of the split-column GEMV (allocated here: solve() may run inside a stream capture)
     const int64_t nrb = std::max<int64_t>(1, (std::max(tail_row1[0] - tail_row0[0], tail_row1[1] - tail_row0[1]) + 7) / 8);
@@ -1414,13 +1441,15 @@ void cuadmm_ysolve_s::solve(const double* d_rhs_, double* d_y_, cudaStream_t st)
         prof_ev->push_back(ev); prof_tag->push_back(tag);
     };
     // split-column GEMV over this rank's rows: enough CTAs per row block to fill the GPU twice
-    auto gemv_split = [&](const double* Tm, const double* in, double* out, const int32_t* tp, const int32_t* tc, int longest_last,
-                          int64_t r0, int64_t nrows_, int npush, const PeerView& pv, const PeerPtrs& outp) {
+    auto gemv_split = [&](const TailMatrix& T, const double* in, double* out, int64_t r0, int64_t nrows_, int npush,
+                          const PeerView& pv, const PeerPtrs& outp) {
         const int64_t nrb = std::max<int64_t>(1, (nrows_ + 7) / 8);
         int splits = (int)std::min<int64_t>(8, std::max<int64_t>(1, (2 * 148 + nrb - 1) / nrb));
-        CUADMM_REQUIRE(split_part.n >= nrb * 8 * 8 && split_count.n >= nrb, "internal: split-column GEMV scratch too small");
-        tail_gemv_kernel<<<(unsigned)(nrb * splits), 256, 0, st>>>(n_tail, Tm, in, out, tp, tc, nullptr, nullptr, 0, done_flag,
-            longest_last, r0, nrows_, npush, pv, outp, PeerPtrs(), splits, split_part.p, split_count.p);
+        CUADMM_REQUIRE(split_part.n >= nrb * 8 * 8 && split_count.n >= nrb && T.rank_order.n >= nrb,
+                       "internal: split-column GEMV scratch too small");
+        tail_gemv_kernel<<<(unsigned)(nrb * splits), 256, 0, st>>>(n_tail, T.val.p, in, out, T.tptr.p, T.tcol.p, T.toff.p,
+            T.rank_order.p, nullptr, nullptr, 0, done_flag, r0, nrows_, npush, pv, outp, PeerPtrs(), splits, split_part.p,
+            split_count.p);
     };
     if (n_tail > 0) {
         mark(20);
@@ -1428,17 +1457,17 @@ void cuadmm_ysolve_s::solve(const double* d_rhs_, double* d_y_, cudaStream_t st)
         if (!peer || peer->world == 1) {
             const int blocks = (int)((n_tail + 7) / 8);
             // whole matrix on one GPU: row per warp streams at 69 % of the HBM peak (ncu), the split-column kernel at 55 %
-            tail_gemv_row_kernel<<<blocks, 256, 0, st>>>(n_tail, tail_inv.p, z.p + n_lead, tmpv, tail_tptr.p, tail_tcol.p,
-                                                         nullptr, nullptr, 0, done_flag, 1);
-            tail_gemv_row_kernel<<<blocks, 256, 0, st>>>(n_tail, tail_inv_t.p, tmpv, xv + n_lead, tail_tptr_t.p, tail_tcol_t.p,
-                                                         d_y_, perm.p, n_lead, done_flag, 0);
+            tail_gemv_row_kernel<<<blocks, 256, 0, st>>>(n_tail, tail[0].val.p, z.p + n_lead, tmpv, tail[0].tptr.p, tail[0].tcol.p,
+                                                         tail[0].toff.p, tail[0].order.p, nullptr, nullptr, 0, done_flag);
+            tail_gemv_row_kernel<<<blocks, 256, 0, st>>>(n_tail, tail[1].val.p, tmpv, xv + n_lead, tail[1].tptr.p, tail[1].tcol.p,
+                                                         tail[1].toff.p, tail[1].order.p, d_y_, perm.p, n_lead, done_flag);
         } else {
             PeerPtrs pxt = peer_x;
             for (int q = 0; q < peer->world; ++q) pxt.p[q] += n_lead;
             const PeerView pv = peer->view();
             const int64_t n0 = tail_row1[0] - tail_row0[0], n1 = tail_row1[1] - tail_row0[1];
-            gemv_split(tail_inv.p, z.p + n_lead, tmpv, tail_tptr.p, tail_tcol.p, 1, tail_row0[0], n0, peer->world, pv, peer_tmp);
-            gemv_split(tail_inv_t.p, tmpv, xv + n_lead, tail_tptr_t.p, tail_tcol_t.p, 0, tail_row0[1], n1, peer->world, pv, pxt);
+            gemv_split(tail[0], z.p + n_lead, tmpv, tail_row0[0], n0, peer->world, pv, peer_tmp);
+            gemv_split(tail[1], tmpv, xv + n_lead, tail_row0[1], n1, peer->world, pv, pxt);
             tail_scatter_kernel<<<(int)((n_tail + 255) / 256), 256, 0, st>>>(n_tail, xv + n_lead, perm.p, n_lead, d_y_, done_flag);
         }
         CUADMM_CUDA(cudaGetLastError());

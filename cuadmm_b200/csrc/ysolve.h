@@ -50,6 +50,17 @@ struct SweepStreams {
     cudaEvent_t fork = nullptr, join = nullptr;
 };
 
+// One triangular matrix of the dense tail (L22^-1 or L22^-T, tail unknowns relabelled, see ysolve_create), stored as
+// its non-empty 64 x 64 tiles only: per 64-row tile row, runs of consecutive non-empty tiles.
+struct TailMatrix {
+    DevBuf<double> val;           // every run as 64 rows x its full width (a multiple of 64), row-major, at toff
+    DevBuf<int32_t> tptr, tcol;   // runs per tile row (CSR); [first, last) column of every run
+    DevBuf<int64_t> toff;
+    DevBuf<int32_t> order;        // 8-row blocks, longest rows first (one-GPU kernel)
+    DevBuf<int32_t> rank_order;   // sharded solver: this rank's 8-row blocks from tail_row0, longest rows first
+    std::vector<double> cost;     // per tile row: columns read (work per row)
+};
+
 }  // namespace cuadmm
 
 struct cuadmm_ysolve_s {
@@ -61,9 +72,9 @@ struct cuadmm_ysolve_s {
     cuadmm::DevBuf<int32_t> perm;      // perm[new] = old
     cuadmm::DevBuf<double> z;          // forward result (permuted order)
     cuadmm::DevBuf<double> x;          // backward result (permuted order)
-    // dense tail: inverse of the trailing Cholesky block, row-major lower and its transpose
-    cuadmm::DevBuf<double> tail_inv, tail_inv_t, tail_tmp;
-    cuadmm::DevBuf<int32_t> tail_tptr, tail_tcol, tail_tptr_t, tail_tcol_t;   // non-empty 64-column tiles per tile row (CSR)
+    // dense tail: inverse of the trailing Cholesky block (lower) and its transpose (upper)
+    cuadmm::TailMatrix tail[2];
+    cuadmm::DevBuf<double> tail_tmp;
     cuadmm::DevBuf<double> d_rhs, d_y; // staging for the host entry
     std::vector<int32_t> h_perm;
     // sharded solver (peer.h): the rows of the two dense-tail GEMVs are split over the ranks by work; every rank
@@ -73,7 +84,6 @@ struct cuadmm_ysolve_s {
     double* x_p = nullptr;              // == x.p, or the arena copy
     cuadmm::PeerPtrs peer_tmp, peer_x;
     int64_t tail_row0[2] = {0, 0}, tail_row1[2] = {0, 0};   // this rank's rows of L22^-1 / L22^-T
-    std::vector<double> h_tail_cost[2]; // per 64-row tile row: columns read (work per row)
     void enable_peer(const cuadmm::PeerComm* pc, size_t off_tmp, size_t off_x);
     void split_tail_rows(int world, int rank);
     cuadmm::DevBuf<double> split_part;  // split-column GEMV: partial sums per (row block, split)
