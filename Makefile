@@ -25,7 +25,7 @@ $(OBJDIR)/%.cpp.o: $(SRC)/%.cpp $(HDRS)
 
 $(LIB): $(OBJS)
 	@mkdir -p $(LIBDIR)
-	$(NVCC) $(ARCH) -shared -o $@ $(OBJS) -lcudart -ldl $(EXTRA_LIBS)
+	$(NVCC) $(ARCH) -shared -o $@ $(OBJS) -lcudart $(EXTRA_LIBS)
 
 $(EXE): $(SRC)/main.cpp $(LIB) $(HDRS)
 	$(NVCC) -O2 -std=c++17 $(ARCH) -o $@ $(SRC)/main.cpp -L$(LIBDIR) -lcuadmm_b200 -Xlinker -rpath -Xlinker '$$ORIGIN'

@@ -371,6 +371,7 @@ _maybe("cuadmm_solver_init_from_problem", C.c_int, vp, vp, C.c_int, C.c_int, C.c
 
 
 def nccl_unique_id():
+    """kept for callers of the removed NCCL transport: the same 128 random bytes as unique_id()"""
     buf = C.create_string_buffer(128)
     _check(lib.cuadmm_nccl_unique_id(buf))
     return buf.raw
@@ -504,9 +505,9 @@ class Solver:
     def set_device(self, device):
         _check(lib.cuadmm_solver_set_device(self.h, int(device)))
 
-    def set_distributed(self, rank, world, nccl_id):
-        """one process per GPU: call before init with the id rank 0 got from nccl_unique_id()"""
-        _check(lib.cuadmm_solver_set_distributed(self.h, int(rank), int(world), nccl_id))
+    def set_distributed(self, rank, world, job_id):
+        """one process per GPU: call before init with the id rank 0 got from unique_id()"""
+        _check(lib.cuadmm_solver_set_distributed(self.h, int(rank), int(world), job_id))
 
     def init(self, eig_stream_num_per_gpu, cpu_eig_thread_num, vec_len, con_num,
              At_csc_col_ptrs, At_csc_row_ids, At_csc_vals, b_indices, b_vals, C_indices, C_vals, blk_vals,

@@ -244,6 +244,8 @@ void peer_scatter_full_launch(const PeerComm& pc, int64_t nloc, const double* lo
 extern "C" int cuadmm_unique_id(char out[128]) {
     return cuadmm::guarded([&] { CUADMM_REQUIRE(out, "null argument"); cuadmm::make_unique_id(out); });
 }
+// kept for callers of the removed NCCL transport: the same job id
+extern "C" int cuadmm_nccl_unique_id(char out[128]) { return cuadmm_unique_id(out); }
 
 // ------------------------------------------------------------------------------------------
 // measurement hook (not in the public header): raw cost of the cross-GPU handshakes

@@ -2,7 +2,7 @@
 // set of PSD blocks = a set of svec ranges, and holds X, S, C restricted to them plus the column slice
 // A[:, I_g].  Replaces the Duo solver's equal-count split + per-iteration peer copies of dense blocks
 // (src/duo_solver.cu:266-295, 517-565): here no block data ever crosses NVLink, only the m-vector
-// partial products A[:, I_g] x_g are all-reduced.  Host-only logic (tested on CPU with gloo).
+// partial products A[:, I_g] x_g are summed over the ranks.  Host-only logic (tested on CPU with gloo).
 #pragma once
 #include "blocks.h"
 #include <vector>

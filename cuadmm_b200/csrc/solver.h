@@ -9,7 +9,6 @@
 #include "ysolve.h"
 #include "problem.h"
 #include "shard.h"
-#include "dist.h"
 #include "peer.h"
 #include "peer_kernels.h"
 
@@ -38,27 +37,24 @@ struct cuadmm_solver {
     bool initialised = false;
     int64_t vec_len = 0, con_num = 0;
     int64_t nloc = 0;                        // svec entries owned by this rank (== vec_len on one GPU)
-    // multi-GPU (one process per GPU): block shard + NCCL communicator
+    // multi-GPU (one process per GPU): block shard; partial products move through peer memory (kernels store into
+    // the peers' arenas, peer.h)
     int rank = 0, world = 1;
-    char nccl_id[128] = {0};
+    char job_id[128] = {0};                  // rendezvous key of the peer board
     cuadmm::Shard shard;
     std::vector<char> blk_types;             // block cones ('s', 'l', 'u') set before init; empty: all 's'
-    // transport of the partial products: peer memory (default; kernels store into the peers' arenas, peer.h) or
-    // NCCL all-reduce (CUADMM_COMM=nccl)
-    bool use_peer = true;
     bool device_set = false;                 // cuadmm_solver_set_device / CUADMM_DEVICE given
     std::unique_ptr<cuadmm::PeerComm> peer;
     int64_t slice = 0;                       // rows of an m-vector reduced by one rank (peer transport)
     double* stage = nullptr;                 // arena: world x slice staged partial rows addressed to this rank
     cuadmm::PeerPtrs p_stage, p_asmc, p_Rp, p_full;
     cuadmm::DevBuf<double> cta_part;         // per-CTA partial sums of peer_reduce_kernel
-    std::unique_ptr<cuadmm::NcclComm> comm;
-    cuadmm::DevBuf<double> red_buf;          // NCCL: m + 2 doubles: partial A_g x_g + two scalars, all-reduced in place
-    cuadmm::DevBuf<double> asmc_part;        // NCCL: this rank's partial -A_g (S-C)_g (all-reduced into asmc)
     cuadmm::DevBuf<int64_t> d_loc2glob;
     cuadmm::DevBuf<double> full_buf;         // vec_len doubles, for gathering full X / S
     void gather_full(const cuadmm::DevBuf<double>& local, double* h_full);
-    void reduce_partial_A(bool for_rp, const double* x_local, double alpha, const double* part_rd, int n_rd, double* part_rp);
+    void reduce_partial_A(bool for_rp, const double* x_local, double alpha, const double* part_rd, int n_rd);
+    struct ScalarPartials { const double* rd; int n_rd; const double* rp; int n_rp; };
+    ScalarPartials scalar_partials(const double* part_rd, int n_rd, const double* part_rp) const;
     std::unique_ptr<cuadmm_plan> plan;
     cuadmm_spmv_s* A = nullptr;    // m x vec_len (row-normalised)
     cuadmm_spmv_s* At = nullptr;   // vec_len x m
@@ -117,7 +113,7 @@ struct cuadmm_solver {
     cudaGraphExec_t graph_sgs = nullptr, graph_admm = nullptr;
     int64_t graph_launches_sgs = 0, graph_launches_admm = 0;
     bool use_graphs = true;
-    cuadmm::DevBuf<double> asmc;             // -A (S-C) (all-reduced when sharded), reused by the next iteration's K1
+    cuadmm::DevBuf<double> asmc;             // -A (S-C) (summed over the ranks when sharded), reused by the next iteration's K1
     bool asmc_valid = false;
     void launch_iteration(int iter, int switch_admm, bool prof);
 };

@@ -243,17 +243,20 @@ int  cuadmm_solver_ysolve_stats(const cuadmm_solver_t* s, int64_t out[8]);
  * Multi-GPU: one process per GPU of one NVSwitch box.  Blocks are sharded by eig cost (cuadmm_plan_partition);
  * every rank owns X, S, C on its svec ranges and the column slice A[:, I_g]; the only per-iteration traffic is
  * the sum over ranks of the m-vector partial products A[:, I_g] x_g (2 per iteration) and the rows of the
- * dense-tail GEMVs of the y-solve, which are split over the ranks.  Default transport: peer memory (CUDA IPC
+ * dense-tail GEMVs of the y-solve, which are split over the ranks.  Transport: peer memory (CUDA IPC
  * arenas; the SpMV / GEMV / reduction kernels store straight into the peers' buffers over NVLink and
- * synchronise with system-scope flags, csrc/peer.h); CUADMM_COMM=nccl selects ncclAllReduce instead.
+ * synchronise with system-scope flags, csrc/peer.h).
  * Replaces SDPDuoSolver's GPU workers + cudaMemcpyPeerAsync of dense blocks
  * (src/duo_solver.cu:266-336, 487-577).  Call cuadmm_solver_set_distributed BEFORE cuadmm_solver_init,
- * with the same 128-byte id on every rank (rank 0 creates it with cuadmm_unique_id — or cuadmm_nccl_unique_id
- * for the NCCL transport — and the launcher broadcasts it); init/solve then take the FULL problem on every
- * rank, get_X/get_S return full vectors (collective calls: every rank must make them).
+ * with the same 128-byte id on every rank (rank 0 creates it with cuadmm_unique_id and the launcher broadcasts
+ * it); init/solve then take the FULL problem on every rank, get_X/get_S return full vectors (collective calls:
+ * every rank must make them).  cuadmm_solver_set_distributed returns CUADMM_EINVAL in a process whose environment
+ * asks for the removed NCCL transport (INTEGRATION.md §6).
  * -------------------------------------------------------------------------- */
+/* kept for compatibility with callers of the removed NCCL transport: fills the same 128 random bytes as
+ * cuadmm_unique_id */
 int  cuadmm_nccl_unique_id(char out[128]);
-/* 128 random bytes; enough for the default peer-memory transport (no NCCL needed to create the job id) */
+/* 128 random bytes: the job id of a sharded solver */
 int  cuadmm_unique_id(char out[128]);
 int  cuadmm_solver_set_distributed(cuadmm_solver_t* s, int rank, int world, const char id[128]);
 /* GPU of this solver (before init).  Default: CUADMM_DEVICE if set, else the calling thread's current device

@@ -11,14 +11,14 @@ torch.cuda.set_device(local); os.environ["CUADMM_DEVICE"] = str(local)
 dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 idt = torch.zeros(128, dtype=torch.uint8, device="cuda")
 if rank == 0:
-    idt.copy_(torch.frombuffer(bytearray(cu.nccl_unique_id()), dtype=torch.uint8))
+    idt.copy_(torch.frombuffer(bytearray(cu.unique_id()), dtype=torch.uint8))
 dist.broadcast(idt, 0)
-nccl_id = bytes(idt.cpu().numpy().tolist())
+job_id = bytes(idt.cpu().numpy().tolist())
 nblk = int(os.environ.get("NBLK", "200")); con = int(os.environ.get("CON", "40000")); iters = int(os.environ.get("ITERS", "60"))
 P = chain_sdp(c2b_blocks(nblk, 6, 60, 0), con, seed=0)
 def make(distributed):
     s = cu.Solver(verbose=False)
-    if distributed: s.set_distributed(rank, world, nccl_id)
+    if distributed: s.set_distributed(rank, world, job_id)
     s.init(15, 30, P["vec_len"], P["con_num"], P["col_ptrs"], P["row_ids"], P["vals"], P["b_idx"], P["b_val"], P["C_idx"], P["C_val"], P["blk"])
     return s
 sd = make(True)

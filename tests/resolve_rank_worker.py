@@ -54,7 +54,7 @@ if rank == 0:
     # atomicAdd, so two runs differ from each other; the sharded run may differ from r by up to 10x that.
     s1.close()
     c = run(make(False))
-    print("world", world, "comm", os.environ.get("CUADMM_COMM", "peer"), "devices", ndev,
+    print("world", world, "devices", ndev,
           "iters sharded", d["iters"], "single", r["iters"])
     ok = d["iters"] == r["iters"] == 60
     for k in ["errRp", "errRd", "pobj", "dobj", "sig", "relgap"]:

@@ -3,7 +3,6 @@ typed problems against the typed oracle (tests/cones_util.py) and against scipy'
 directory, and the block-sharded solver on 2 and 3 ranks."""
 import os
 import subprocess
-import sys
 
 import numpy as np
 import pytest
@@ -11,6 +10,7 @@ import pytest
 import cuadmm_b200 as cu
 import cones_util as cz
 import oracle_np as onp
+from test_gpu_multi import launch
 from util_problems import ROOT, parse_log
 
 pytestmark = pytest.mark.gpu
@@ -255,19 +255,6 @@ def test_exe_on_typed_txt_directory(tmp_path):
 
 @pytest.mark.parametrize("world", [2, 3])
 def test_sharded_typed_solver_matches_single_gpu(world):
-    job = cu.unique_id().hex()
-    procs = []
-    for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), JOB_ID=job, CUADMM_PEER_TIMEOUT_S="20")
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "cones_rank_worker.py")], env=env,
-                                      stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    outs = []
-    for p in procs:
-        try:
-            outs.append(p.communicate(timeout=600)[0])
-        except subprocess.TimeoutExpired:
-            for q in procs:
-                q.kill()
-            raise
+    procs, outs = launch(world, "cones_rank_worker.py")
     assert "CONES_RANK_OK" in outs[0], "\n".join(o[-3000:] for o in outs)
     assert all(p.returncode == 0 for p in procs), "\n".join(o[-3000:] for o in outs)

@@ -1,5 +1,5 @@
-"""Multi-rank parity: the block-sharded solver (one process per rank; peer-memory transport by default, NCCL with
-CUADMM_COMM=nccl) must reproduce the single-GPU trajectory, iterates, y and stop iteration.  With one GPU the
+"""Multi-rank parity: the block-sharded solver (one process per rank, peer-memory transport) must reproduce the
+single-GPU trajectory, iterates, y and stop iteration.  With one GPU the
 ranks share it (CUDA IPC works between processes on the same device), so the sharded data path — SpMV rows pushed
 to the reducing rank, slice reduction, split dense-tail GEMVs, gather by owner — is exercised on every box."""
 import os
@@ -14,13 +14,13 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 pytestmark = pytest.mark.gpu
 
 
-def launch(world, case, extra_env=None, timeout=600):
+def launch(world, worker, timeout=600, **extra_env):
+    """one process per rank running tests/<worker> with a fresh job id; the processes and their outputs"""
     job = cu.unique_id().hex()
     procs = []
     for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), JOB_ID=job, CASE=case, CUADMM_PEER_TIMEOUT_S="20")
-        env.update(extra_env or {})
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "multi_rank_worker.py")], env=env,
+        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), JOB_ID=job, CUADMM_PEER_TIMEOUT_S="20", **extra_env)
+        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", worker)], env=env,
                                       stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
     outs = []
     for p in procs:
@@ -38,21 +38,6 @@ def launch(world, case, extra_env=None, timeout=600):
 def test_sharded_solver_matches_single_gpu(world, case):
     if cu.device_count() < 1:
         pytest.skip("needs a GPU")
-    procs, outs = launch(world, case)
+    procs, outs = launch(world, "multi_rank_worker.py", CASE=case)
     assert "MULTI_RANK_OK" in outs[0], "\n".join(o[-3000:] for o in outs)
     assert all(p.returncode == 0 for p in procs), "\n".join(o[-3000:] for o in outs)
-
-
-@pytest.mark.parametrize("case", ["sgs", "tol"])
-def test_sharded_solver_nccl_transport(case):
-    if cu.device_count() < 2:
-        pytest.skip("NCCL needs one GPU per rank")
-    # the NCCL transport takes its id from ncclGetUniqueId
-    job = cu.nccl_unique_id().hex()
-    procs = []
-    for r in range(2):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE="2", JOB_ID=job, CASE=case, CUADMM_COMM="nccl")
-        procs.append(subprocess.Popen([sys.executable, os.path.join(ROOT, "tests", "multi_rank_worker.py")], env=env,
-                                      stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    outs = [p.communicate(timeout=600)[0] for p in procs]
-    assert "MULTI_RANK_OK" in outs[0], "\n".join(o[-3000:] for o in outs)

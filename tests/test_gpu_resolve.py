@@ -2,14 +2,13 @@
 with the same data, a warm update against a fresh init at the previous solution, the committed PushT_N=10 log through an
 update, rejected input, and the sharded solver on 2 and 3 ranks against the single-GPU update."""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 import cuadmm_b200 as cu
 import cones_util as cz
+from test_gpu_multi import launch
 from util_problems import GOLD, load_fixture, parse_log
 
 pytestmark = pytest.mark.gpu
@@ -198,26 +197,9 @@ def test_bad_input_leaves_solver_usable():
     compare_to_fresh(s, f, P, exact=True)
 
 
-@pytest.mark.parametrize("world,comm", [(2, "peer"), (3, "peer"), (2, "nccl")])
-def test_sharded_update_matches_single_gpu(world, comm):
-    if comm == "nccl" and cu.device_count() < world:
-        pytest.skip("NCCL needs one GPU per rank (the peer transport lets ranks share one)")
-    job = (cu.nccl_unique_id() if comm == "nccl" else cu.unique_id()).hex()
-    procs = []
-    for r in range(world):
-        env = dict(os.environ, RANK=str(r), WORLD_SIZE=str(world), JOB_ID=job, CUADMM_PEER_TIMEOUT_S="20")
-        if comm == "nccl":
-            env["CUADMM_COMM"] = "nccl"
-        procs.append(subprocess.Popen([sys.executable, os.path.join(os.path.dirname(__file__), "resolve_rank_worker.py")],
-                                      env=env, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True))
-    outs = []
-    for p in procs:
-        try:
-            outs.append(p.communicate(timeout=600)[0])
-        except subprocess.TimeoutExpired:
-            for q in procs:
-                q.kill()
-            raise
+@pytest.mark.parametrize("world", [2, 3], ids=["2-peer", "3-peer"])
+def test_sharded_update_matches_single_gpu(world):
+    procs, outs = launch(world, "resolve_rank_worker.py")
     print(outs[0])
     assert "RESOLVE_RANK_OK" in outs[0], "\n".join(o[-3000:] for o in outs)
     assert all(p.returncode == 0 for p in procs), "\n".join(o[-3000:] for o in outs)

@@ -45,10 +45,37 @@ def test_column_slices_reassemble_the_operator():
         s = cu.Shard(P["blk"], world, r)
         cp, ri, v = s.slice_csc(P["col_ptrs"], P["row_ids"], P["vals"])
         Ag = sp.csr_matrix((v, ri, cp), shape=(m, s.vec_len_local))
-        acc += Ag @ x[s.loc2glob]                 # what the NCCL all-reduce sums
+        acc += Ag @ x[s.loc2glob]                 # what the reduction over the ranks sums
         aty[s.loc2glob] = Ag.T @ y                # A^T y needs no communication
     assert np.allclose(acc, A @ x, rtol=0, atol=1e-12 * np.abs(A @ x).max())
     assert np.allclose(aty, A.T @ y, rtol=0, atol=1e-12 * np.abs(A.T @ y).max())
+
+
+CUADMM_EINVAL = -1
+
+
+def test_job_ids_need_no_gpu():
+    # cuadmm_nccl_unique_id stays for callers of the removed NCCL transport and makes the same kind of id
+    ids = [cu.unique_id(), cu.unique_id(), cu.nccl_unique_id(), cu.nccl_unique_id()]
+    assert all(isinstance(i, bytes) and len(i) == 128 for i in ids)
+    assert len(set(ids)) == 4
+
+
+@pytest.mark.parametrize("comm", [None, "peer", "nccl"])
+def test_set_distributed_rejects_the_removed_nccl_transport(monkeypatch, comm):
+    # a job launched with CUADMM_COMM=nccl must fail, not run the peer-memory transport under the NCCL label
+    if comm is None:
+        monkeypatch.delenv("CUADMM_COMM", raising=False)
+    else:
+        monkeypatch.setenv("CUADMM_COMM", comm)
+    s = cu.Solver(verbose=False)
+    if comm == "nccl":
+        with pytest.raises(cu.CuadmmError) as e:
+            s.set_distributed(0, 2, cu.unique_id())
+        assert e.value.code == CUADMM_EINVAL and "NCCL transport was removed" in str(e.value)
+    else:
+        s.set_distributed(0, 2, cu.unique_id())
+    s.close()
 
 
 WORKER = r'''
