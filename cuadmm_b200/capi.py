@@ -287,6 +287,10 @@ _maybe("cuadmm_ysolve", C.c_int, vp, vp, vp, vp)
 _maybe("cuadmm_ysolve_host", C.c_int, vp, c_f64p, c_f64p)
 _maybe("cuadmm_ysolve_stats", C.c_int, vp, c_i64p)
 _maybe("cuadmm_ysolve_perm", C.c_int, vp, c_i32p)
+_maybe("cuadmm_debug_ysolve_paths", C.c_int, vp, c_i64p)
+
+_SWEEP_PATHS = ("n_sub", "n_sub_pack", "n_sub_warp", "n_sub_cta", "pk_rows", "pk_n_heavy", "pk_has_ext", "collapsed",
+                "max_chunks", "long_records", "levels", "narrow_phases", "wide_phases", "top_long_slots")
 
 
 class YSolve:
@@ -323,7 +327,17 @@ class YSolve:
         s = np.zeros(8, np.int64)
         _check(lib.cuadmm_ysolve_stats(self.h, _p(s, c_i64p)))
         return dict(nnz_AAt=int(s[0]), nnz_L=int(s[1]), levels=int(s[2]), dense_tail=int(s[3]),
-                    launches=int(s[4]), bytes=int(s[5]))
+                    launches=int(s[4]), bytes=int(s[5]), deficient=int(s[6]), subtrees=int(s[7]) // 100000,
+                    subtree_depth=int(s[7]) % 100000)
+
+    def paths(self):
+        """the kernel paths a solve takes (cuadmm_debug_ysolve_paths): {"fwd": {...}, "bwd": {...}, "tail": {...}}"""
+        s = np.zeros(32, np.int64)
+        _check(lib.cuadmm_debug_ysolve_paths(self.h, _p(s, c_i64p)))
+        sweep = lambda o: {k: int(s[o + i]) for i, k in enumerate(_SWEEP_PATHS)}
+        return dict(fwd=sweep(0), bwd=sweep(14),
+                    tail=dict(n_tail=int(s[28]), tiles_lower=int(s[29]), tiles_upper=int(s[30]),
+                              postorder_fallback=int(s[31])))
 
     def perm(self):
         p = np.zeros(self.m, np.int32)

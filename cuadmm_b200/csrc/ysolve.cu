@@ -11,6 +11,7 @@
 #include <chrono>
 #include <thread>
 #include <atomic>
+#include <mutex>
 #include "dense.h"
 #include <algorithm>
 #include <numeric>
@@ -746,7 +747,8 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
     std::vector<Packed> packs, blobs;
     std::vector<int32_t> loc(H.n, -1), cidx(H.n, -1), height(H.n, 0), lvl_r(H.n, 0);
     int chain_max = kPkChainMax, chain_gain = 6;
-    if (const char* e = getenv("CUADMM_SWEEP_CHAIN_MAX")) chain_max = std::min(atoi(e), kPkMaxRowEntries);
+    // at most kPkChainMax: choose_subtrees reserves that many scratch slots in the packed kernel's shared memory
+    if (const char* e = getenv("CUADMM_SWEEP_CHAIN_MAX")) chain_max = std::min(atoi(e), kPkChainMax);
     const bool verbose = getenv("CUADMM_YSOLVE_VERBOSE") != nullptr;
     int64_t n_collapsed = 0, levels_before = 0, levels_after = 0, chain_entries = 0;
     kind.assign(H.n_sub, 0);
@@ -754,7 +756,7 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
     // one subtree at a time, on a pool of host threads: subtrees own disjoint rows of the scratch arrays (loc, cidx, height,
     // lvl_r), results land in per-subtree slots and are collected in subtree order afterwards (deterministic layout)
     std::vector<Packed> result(H.n_sub);
-    std::atomic<int64_t> a_collapsed{0}, a_before{0}, a_after{0}, a_entries{0};
+    std::atomic<int64_t> a_collapsed{0}, a_before{0}, a_after{0}, a_entries{0}, a_long{0};
     auto do_subtree = [&](int64_t t) {
         const std::vector<int32_t>& rows = members[t];       // in solve order
         const int32_t nr0 = (int32_t)rows.size();
@@ -937,6 +939,7 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
                 shorts.erase(shorts.begin(), shorts.begin() + promote);
             }
             std::stable_sort(longs.begin(), longs.end(), [](const PkRow* a, const PkRow* b) { return a->idx.size() > b->idx.size(); });
+            a_long += (int64_t)longs.size();
             bool first = true;
             for (const PkRow* r : longs) { add_record(make_record(&r, 1, true), first); first = false; }
             for (size_t q = 0; q < shorts.size(); q += 8) {
@@ -978,9 +981,11 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
     S.n_sub_pack = (int64_t)packs.size();
     S.n_sub_warp = (int64_t)blobs.size();
     S.pk_smem = 0; S.pk_rows = 0;
+    S.pk_collapsed = n_collapsed; S.pk_long_records = a_long; S.pk_max_chunks = 0;
     if (packs.empty() && blobs.empty()) return;
     // biggest first: CTAs are dispatched in index order
     std::stable_sort(packs.begin(), packs.end(), [](const Packed& a, const Packed& b) { return a.bytes.size() > b.bytes.size(); });
+    if (!packs.empty()) S.pk_max_chunks = (int64_t)((packs[0].bytes.size() + kPkChunk - 1) / kPkChunk);
     std::stable_sort(blobs.begin(), blobs.end(), [&](const Packed& a, const Packed& b) { return a.levels > b.levels; });
     std::vector<int64_t> chunk_off(1, 0), blob_off(1, 0), row_off(1, 0), ext_ptr(1, 0);
     std::vector<int32_t> prow_u, prow_src, prow_out, ext_dep;
@@ -1034,7 +1039,17 @@ static void pack_subtrees(const HostSweep& H, TriSweep& S, const std::vector<std
         S.pk_timeline_meta = meta;
     }
     S.pk_smem = (size_t)kPkRing * kPkChunk + 64 + sizeof(double) * (size_t)cta_slots;
-    CUADMM_CUDA(cudaFuncSetAttribute((const void*)tri_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S.pk_smem));
+    {
+        // the limit belongs to the kernel (per device), not to this y-solve: only ever raise it, or creating a y-solve with
+        // smaller subtrees would make every launch of one created before it fail
+        static std::mutex mu;
+        std::lock_guard<std::mutex> lock(mu);
+        cudaFuncAttributes fa;
+        CUADMM_CUDA(cudaFuncGetAttributes(&fa, (const void*)tri_packed_kernel));
+        if ((size_t)fa.maxDynamicSharedSizeBytes < S.pk_smem)
+            CUADMM_CUDA(cudaFuncSetAttribute((const void*)tri_packed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                             (int)S.pk_smem));
+    }
     if (verbose)
         fprintf(stderr, "[ysolve] %s packed: %zu CTA subtrees in %lld chunks (largest %zu), %zu warp subtrees in %zu bytes, "
                 "%lld slots, %lld external entries (%lld heavy rows), smem %zu; chains collapsed in %lld subtrees (%lld -> %lld levels, %lld inverse entries)\n",
@@ -1115,6 +1130,8 @@ static void upload_sweep(const HostSweep& H, TriSweep& S) {
         S.h_level_ptr[l + 1] = (int64_t)slot_info.size();
     }
     S.n_slots = (int64_t)slot_info.size();
+    S.top_long_slots = 0;
+    for (int64_t s = S.h_level_ptr[0]; s < S.n_slots; ++s) S.top_long_slots += slot_info[s] >> 30;
     int narrow_slots = kNarrowSlots;
     if (const char* e = getenv("CUADMM_SWEEP_NARROW_SLOTS")) narrow_slots = atoi(e);
     S.phases.clear();
@@ -1204,6 +1221,7 @@ static void pack_tail_matrix(int64_t r, const double* Linv, const int32_t* d_ipo
         }
         ptr.push_back((int32_t)(col.size() / 2));
     }
+    T.tiles = (int64_t)tiles.size() / 4;
     if (col.empty()) { col.assign(2, 0); off.push_back(0); }
     T.val.alloc(std::max<int64_t>(size, 1));
     pack_tiles(r, Linv, d_ipos, !lower, tiles, T.val.p);
@@ -1251,6 +1269,7 @@ static void build_tail(cuadmm_ysolve_s& Y, const SymCsc& C, const CholFactor& F,
         std::iota(pos.begin(), pos.end(), 0);
         scan();
     }
+    Y.tail_postorder_fallback = upper;
     if (verbose) {
         const int64_t lower = (int64_t)nt * (nt + 1) / 2, used = lower_used();
         fprintf(stderr, "[ysolve] dense tail %lld: non-zero lower 64x64 tiles of L22^-1: %lld of %lld (%.1f%%) in the tail order, "
@@ -1511,6 +1530,30 @@ int cuadmm_debug_ysolve_timeline(cuadmm_ysolve_t* ys, int which, long long* time
         CUADMM_CUDA(cudaDeviceSynchronize());
         CUADMM_CUDA(cudaMemcpy(timeline, S.pk_timeline.p, sizeof(long long) * 4 * (size_t)*n, cudaMemcpyDeviceToHost));
         if (meta) std::copy(S.pk_timeline_meta.begin(), S.pk_timeline_meta.end(), meta);
+    });
+}
+
+// debug: the kernel paths a solve takes, as chosen at create time.  out[14 * which + k] for the forward (which = 0)
+// and the backward sweep (1), k = 0 subtrees, 1 CTA-packed, 2 warp-packed, 3 generic (tri_subtree_kernel), 4 packed
+// rows, 5 heavy gather rows (a warp each), 6 any external entries, 7 collapsed chains, 8 chunks of the largest
+// CTA-packed subtree, 9 warp-wide records in packed subtrees, 10 top levels, 11 narrow phases, 12 wide phases,
+// 13 warp-wide slots in the top levels; out[28] dense tail rows, out[29] / out[30] stored tiles of L22^-1 / L22^-T,
+// out[31] 1 if the tail kept its own order because the postorder left a tile above the diagonal.
+int cuadmm_debug_ysolve_paths(const cuadmm_ysolve_t* ys, int64_t out[32]) {
+    return guarded([&] {
+        CUADMM_REQUIRE(ys && out, "null argument");
+        for (int w = 0; w < 2; ++w) {
+            const cuadmm::TriSweep& S = w ? ys->bwd : ys->fwd;
+            int64_t* o = out + 14 * w;
+            int64_t narrow = 0;
+            for (const cuadmm::TriSweep::Phase& ph : S.phases) narrow += ph.narrow ? 1 : 0;
+            o[0] = S.n_sub; o[1] = S.n_sub_pack; o[2] = S.n_sub_warp; o[3] = S.n_sub_cta;
+            o[4] = S.pk_rows; o[5] = S.pk_n_heavy; o[6] = S.pk_has_ext ? 1 : 0; o[7] = S.pk_collapsed;
+            o[8] = S.pk_max_chunks; o[9] = S.pk_long_records; o[10] = S.levels; o[11] = narrow;
+            o[12] = (int64_t)S.phases.size() - narrow; o[13] = S.top_long_slots;
+        }
+        out[28] = ys->n_tail; out[29] = ys->tail[0].tiles; out[30] = ys->tail[1].tiles;
+        out[31] = ys->tail_postorder_fallback ? 1 : 0;
     });
 }
 

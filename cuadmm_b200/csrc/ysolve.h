@@ -42,6 +42,11 @@ struct TriSweep {
     bool pk_has_ext = false;
     int sub_depth = 0;
     bool subtrees_first = true;
+    // path counters (cuadmm_debug_ysolve_paths): which kernel paths the packing and the level plan chose
+    int64_t pk_collapsed = 0;     // packed subtrees whose chain was collapsed into a dense inverse
+    int64_t pk_max_chunks = 0;    // chunks of the largest CTA-packed subtree
+    int64_t pk_long_records = 0;  // warp-wide records in packed subtrees (promoted short rows included)
+    int64_t top_long_slots = 0;   // warp-wide slots of the top levels
 };
 
 // side stream + events to run the two subtree kernels of a sweep concurrently
@@ -59,6 +64,7 @@ struct TailMatrix {
     DevBuf<int32_t> order;        // 8-row blocks, longest rows first (one-GPU kernel)
     DevBuf<int32_t> rank_order;   // sharded solver: this rank's 8-row blocks from tail_row0, longest rows first
     std::vector<double> cost;     // per tile row: columns read (work per row)
+    int64_t tiles = 0;            // stored 64 x 64 tiles
 };
 
 }  // namespace cuadmm
@@ -74,6 +80,7 @@ struct cuadmm_ysolve_s {
     cuadmm::DevBuf<double> x;          // backward result (permuted order)
     // dense tail: inverse of the trailing Cholesky block (lower) and its transpose (upper)
     cuadmm::TailMatrix tail[2];
+    bool tail_postorder_fallback = false;   // the postorder left a tile above the diagonal: tail order kept
     cuadmm::DevBuf<double> tail_tmp;
     cuadmm::DevBuf<double> d_rhs, d_y; // staging for the host entry
     std::vector<int32_t> h_perm;

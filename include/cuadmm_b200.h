@@ -165,7 +165,8 @@ void cuadmm_ysolve_destroy(cuadmm_ysolve_t* ys);
 int  cuadmm_ysolve(cuadmm_ysolve_t* ys, const double* d_rhs, double* d_y, void* stream);
 int  cuadmm_ysolve_host(cuadmm_ysolve_t* ys, const double* h_rhs, double* h_y);
 /* stats: out[0]=nnz(AAt lower) out[1]=nnz(L) out[2]=levels(sparse part) out[3]=dense tail size
- * out[4]=launches per solve out[5]=algorithmic bytes per solve */
+ * out[4]=launches per solve out[5]=algorithmic bytes per solve out[6]=pinned (deficient) pivots
+ * out[7]=subtrees * 100000 + deepest subtree (levels) */
 int  cuadmm_ysolve_stats(const cuadmm_ysolve_t* ys, int64_t out[8]);
 /* fill-reducing permutation used (length m), CHOLMOD's L->Perm analogue */
 int  cuadmm_ysolve_perm(const cuadmm_ysolve_t* ys, int32_t* perm);
