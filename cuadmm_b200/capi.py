@@ -364,6 +364,10 @@ _maybe("cuadmm_solver_set_XyS", C.c_int, vp, c_f64p, c_f64p, c_f64p, C.c_double)
 _maybe("cuadmm_solver_update_data", C.c_int, vp, c_i32p, c_f64p, C.c_int64, c_i32p, c_f64p, C.c_int64, C.c_int, C.c_double)
 _maybe("cuadmm_solver_iter_num", C.c_int64, vp)
 _maybe("cuadmm_solver_history", C.c_int, vp, C.c_int, c_f64p, C.c_int64)
+_maybe("cuadmm_solver_set_infeasibility_check", C.c_int, vp, C.c_int, C.c_double)
+_maybe("cuadmm_solver_stop_reason", C.c_int, vp)
+_maybe("cuadmm_solver_certificate", C.c_int, vp, C.c_int, c_f64p, c_f64p)
+_maybe("cuadmm_solver_infeasibility_stats", C.c_int, vp, c_f64p)
 _maybe("cuadmm_solver_times", C.c_int, vp, c_f64p)
 _maybe("cuadmm_solver_launches", C.c_int64, vp)
 _maybe("cuadmm_solver_run_iterations", C.c_int, vp, C.c_int, C.c_int, C.c_int, c_f64p)
@@ -575,6 +579,33 @@ class Solver:
         out = np.zeros(max(n, 1))
         _check(lib.cuadmm_solver_history(self.h, self.HIST[name], _p(out, c_f64p), n))
         return out[:n]
+
+    STOP_REASONS = {0: "not solved", 1: "converged", 2: "max_iter", 3: "primal_infeasible", 4: "dual_infeasible"}
+
+    def set_infeasibility_check(self, interval, eps=1e-7):
+        """check for primal / dual infeasibility every `interval` iterations (0: off) at tolerance eps; applies from the
+        next solve"""
+        _check(lib.cuadmm_solver_set_infeasibility_check(self.h, int(interval), float(eps)))
+
+    @property
+    def stop_reason(self):
+        """0 before the first solve, 1 converged, 2 max iterations, 3 primal infeasible, 4 dual infeasible"""
+        return lib.cuadmm_solver_stop_reason(self.h)
+
+    def certificate(self, which):
+        """(vector, ratio) of the last solve: which 0 the primal infeasibility certificate y-bar (b'y-bar = 1), which 1
+        the dual infeasibility certificate d (<C, d> = -1), in the caller's units"""
+        out = np.zeros(max(self.con_num if which == 0 else self.vec_len, 1))
+        ratio = np.zeros(1)
+        _check(lib.cuadmm_solver_certificate(self.h, int(which), _p(out, c_f64p), _p(ratio, c_f64p)))
+        return out[:self.con_num if which == 0 else self.vec_len], float(ratio[0])
+
+    def infeasibility_stats(self):
+        """what the checks of the last solve saw (cuadmm_solver_infeasibility_stats)"""
+        t = np.zeros(8)
+        _check(lib.cuadmm_solver_infeasibility_stats(self.h, _p(t, c_f64p)))
+        return dict(checks=int(t[0]), primal_projections=int(t[1]), dual_projections=int(t[2]), min_primal_ratio=t[3],
+                    min_dual_ratio=t[4], min_primal_guard=t[5], min_dual_guard=t[6], last_check_iter=int(t[7]))
 
     def times(self):
         t = np.zeros(8)

@@ -65,8 +65,9 @@ void PeerComm::init(int rank_, int world_, const char id[128], int device_, size
     d_epoch.alloc(1); d_count.alloc(2); d_err.alloc(1);
     d_epoch.zero(); d_count.zero(); d_err.zero();
     if (const char* e = getenv("CUADMM_PEER_TIMEOUT_S")) { const double s = atof(e); if (s > 0) timeout_ns = (unsigned long long)(s * 1e9); }
-    // control block: ready / fin flags (one 8-byte word per writer rank) and the two scalar boards (2 doubles per rank)
-    off_ready = 0; off_fin = 1024; off_scal_rd = 2048; off_scal_rp = 2048 + 512;
+    // control block: ready / fin flags (one 8-byte word per writer rank), the two scalar boards (2 doubles per rank) and
+    // the infeasibility check's board (two regions of 256 bytes: 3 and 2 doubles per rank)
+    off_ready = 0; off_fin = 1024; off_scal_rd = 2048; off_scal_rp = 2048 + 512; off_scal_chk = 3072;
     used = control_bytes();
     if (world > 1) {
         const std::string name = board_name(id);

@@ -45,7 +45,7 @@ struct PeerComm {
     DevBuf<unsigned long long> d_epoch;
     DevBuf<unsigned int> d_count;
     DevBuf<int> d_err;
-    size_t off_ready = 0, off_fin = 0, off_scal_rd = 0, off_scal_rp = 0;
+    size_t off_ready = 0, off_fin = 0, off_scal_rd = 0, off_scal_rp = 0, off_scal_chk = 0;
     unsigned long long timeout_ns = 120ull * 1000000000ull;   // ranks may reach their first handshake seconds apart (init skew)
 
     ~PeerComm();

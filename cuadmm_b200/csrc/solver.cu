@@ -218,6 +218,143 @@ __global__ void __launch_bounds__(256) data_residuals_kernel(DevState* st, const
     st->maxfeas = r.maxfeas; st->relgap = r.relgap;
 }
 
+// ---- infeasibility check (every chk_interval iterations, after the iteration; enqueued outside the iteration graphs).
+// Iterate differences over the window since the last check: dy = y_k - y_{k-p}, dX = X_k - X_{k-p} (scaled space).
+// A candidate counts only when b_s'dy (or -<C_s, dX>) exceeds kInfeasGamma times the product of the two norms: the
+// directions along which y drifts at rounding level (the null space of A_s', e.g. redundant constraints) never fire.
+static constexpr double kInfeasGamma = 1e-8;
+
+// store_cta_pair for N sums: this CTA's sums at partial[N * blockIdx.x + q]
+template <int N>
+__device__ __forceinline__ void store_cta_n(double (&a)[N], double* partial) {
+    __shared__ double red[N][kEwThreads / 32];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1)
+#pragma unroll
+        for (int q = 0; q < N; ++q) a[q] += __shfl_xor_sync(0xffffffffu, a[q], o);
+    if ((threadIdx.x & 31) == 0)
+        for (int q = 0; q < N; ++q) red[q][threadIdx.x >> 5] = a[q];
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int q = 0; q < N; ++q) {
+            double s = 0.0;
+            for (int k = 0; k < kEwThreads / 32; ++k) s += red[q][k];
+            partial[N * blockIdx.x + q] = s;
+        }
+    }
+}
+
+// one CTA of 256 threads: the sums of nb groups of N partials, in a fixed order (sum_pairs_256 for N sums)
+template <int N>
+__device__ __forceinline__ void sum_n_256(const double* __restrict__ p, int nb, double out[N]) {
+    __shared__ double sm[N][256];
+    double v[N] = {};
+    for (int i = threadIdx.x; i < nb; i += 256)
+        for (int q = 0; q < N; ++q) v[q] += p[N * i + q];
+    for (int q = 0; q < N; ++q) sm[q][threadIdx.x] = v[q];
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+        if (threadIdx.x < o) for (int q = 0; q < N; ++q) sm[q][threadIdx.x] += sm[q][threadIdx.x + o];
+        __syncthreads();
+    }
+    for (int q = 0; q < N; ++q) out[q] = sm[q][0];
+}
+
+// m side: dy and A_s dX = Rp_{k-p} - Rp_k, the snapshots move to this iteration; partials (b_s'dy, |dy|^2, |A_s dX|^2, |b_s|^2)
+__global__ void __launch_bounds__(kEwThreads) chk_m_kernel(int64_t m, const double* __restrict__ y, const double* __restrict__ Rp,
+        const double* __restrict__ bd, double* yprev, double* Rpprev, double* dy, const DevState* st, double* partial) {
+    if (st->done) return;
+    double a[4] = {};
+    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < m; i += (int64_t)gridDim.x * kEwThreads) {
+        const double yi = y[i], ri = Rp[i], bi = bd[i];
+        const double d = yi - yprev[i], r = Rpprev[i] - ri;
+        yprev[i] = yi; Rpprev[i] = ri; dy[i] = d;
+        a[0] = fma(bi, d, a[0]); a[1] = fma(d, d, a[1]); a[2] = fma(r, r, a[2]); a[3] = fma(bi, bi, a[3]);
+    }
+    store_cta_n<4>(a, partial);
+}
+
+// vec side: dX, the snapshot moves to this iteration; partials (<C_s, dX>, |dX|^2, |C_s|^2)
+__global__ void __launch_bounds__(kEwThreads) chk_x_kernel(int64_t n, const double* __restrict__ X, const double* __restrict__ Cd,
+        double* Xprev, double* dX, const DevState* st, double* partial) {
+    if (st->done) return;
+    double a[3] = {};
+    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
+        const double xi = X[i], ci = Cd[i];
+        const double d = xi - Xprev[i];
+        Xprev[i] = xi; dX[i] = d;
+        a[0] = fma(ci, d, a[0]); a[1] = fma(d, d, a[1]); a[2] = fma(ci, ci, a[2]);
+    }
+    store_cta_n<3>(a, partial);
+}
+
+// the guard of both tests; skip[0] / skip[1] are the done flags of the projections of A_s'dy / dX, so a candidate
+// that already fails its guard (or a check after the stop) costs no Jacobi sweep
+__global__ void __launch_bounds__(256) chk_pretest_kernel(DevState* st, const double* __restrict__ part_m, int nm,
+        const double* __restrict__ part_x, int nx, int* skip) {
+    if (st->done) { if (threadIdx.x == 0) { skip[0] = 1; skip[1] = 1; } return; }
+    double s[4], t[3];
+    sum_n_256<4>(part_m, nm, s);
+    sum_n_256<3>(part_x, nx, t);
+    if (threadIdx.x != 0) return;
+    const double beta = s[0], ndy = sqrt(s[1]), kappa = -t[0], ndx = sqrt(t[1]);
+    const double nby = sqrt(s[3]) * ndy, ncx = sqrt(t[2]) * ndx;
+    st->chk_beta = beta; st->chk_ndy = ndy; st->chk_nAdx = sqrt(s[2]); st->chk_kappa = kappa; st->chk_ndx = ndx;
+    const int s0 = !(beta > kInfeasGamma * nby);      // NaN fails too
+    const int s1 = !(kappa > kInfeasGamma * ncx);
+    skip[0] = s0; skip[1] = s1;
+    st->chk_count += 1;
+    if (!s0) { st->chk_nproj_p += 1; st->chk_min_cosp = fmin(st->chk_min_cosp, beta / nby); }
+    if (!s1) { st->chk_nproj_d += 1; st->chk_min_cosd = fmin(st->chk_min_cosd, kappa / ncx); }
+}
+
+// sharded solver: this rank's N sums (from nb groups of per-CTA partials, fixed order) into slot `rank` of every rank's
+// board, inside the enter / leave handshake; the one-CTA consumer then adds the world slots in a fixed order, so every
+// rank reaches the same decision bit for bit
+template <int N>
+__global__ void __launch_bounds__(256) chk_publish_kernel(PeerView pv, const double* __restrict__ part, int nb, PeerPtrs board,
+                                                          const int* __restrict__ done) {
+    if (*done) return;
+    const unsigned long long e = peer_epoch(pv);
+    peer_enter(pv, e);
+    double s[N];
+    sum_n_256<N>(part, nb, s);
+    if (threadIdx.x == 0)
+        for (int q = 0; q < pv.world; ++q)
+            for (int k = 0; k < N; ++k) board.p[q][N * pv.rank + k] = s[k];
+    peer_leave(pv, e);
+}
+
+// partials (|Pi_K(A_s'dy)|^2, |dX - Pi_K(dX)|^2); a skipped projection left its output unwritten and contributes 0
+__global__ void __launch_bounds__(kEwThreads) chk_norms_kernel(int64_t n, const double* __restrict__ pv, const double* __restrict__ dX,
+        const double* __restrict__ pdX, const int* __restrict__ skip, double* partial) {
+    const bool s0 = skip[0] != 0, s1 = skip[1] != 0;
+    if (s0 && s1) return;
+    double a0 = 0.0, a1 = 0.0;
+    for (int64_t i = (int64_t)blockIdx.x * kEwThreads + threadIdx.x; i < n; i += (int64_t)gridDim.x * kEwThreads) {
+        if (!s0) { const double p = pv[i]; a0 = fma(p, p, a0); }
+        if (!s1) { const double r = dX[i] - pdX[i]; a1 = fma(r, r, a1); }
+    }
+    store_cta_pair(a0, a1, partial);
+}
+
+// the decision: both ratios into the state, and the stop when one of them is <= eps (primal first)
+__global__ void __launch_bounds__(256) chk_decide_kernel(DevState* st, const double* __restrict__ part_n, int nn,
+        const int* __restrict__ skip, double eps) {
+    if (st->done) return;
+    const bool s0 = skip[0] != 0, s1 = skip[1] != 0;
+    double s[2] = {0.0, 0.0};
+    if (!(s0 && s1)) sum_n_256<2>(part_n, nn, s);
+    if (threadIdx.x != 0) return;
+    const double pr = s0 ? INFINITY : sqrt(s[0]) / st->chk_beta;
+    const double dr = s1 ? INFINITY : fmax(st->chk_nAdx, sqrt(s[1])) / st->chk_kappa;
+    const int fired = (pr <= eps ? 1 : 0) | (dr <= eps ? 2 : 0);
+    st->chk_iter = st->iter - 1;
+    st->chk_pratio = pr; st->chk_dratio = dr; st->chk_fired = fired;
+    st->chk_min_pratio = fmin(st->chk_min_pratio, pr); st->chk_min_dratio = fmin(st->chk_min_dratio, dr);
+    if (fired) { st->done = 1; st->stop_reason = (fired & 1) ? 3 : 4; }
+}
+
 static int ew_grid(int64_t n, int device) {
     int sms = 148;
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
@@ -491,6 +628,66 @@ void cuadmm_solver::launch_iteration(int iter, int switch_admm, bool prof) {
     asmc_valid = sgs;
 }
 
+// The infeasibility check after iteration st->iter - 1 (INTEGRATION.md §10): dy, A_s dX, dX and their sums, v = A_s' dy,
+// the guard, Pi_K(v) and Pi_K(dX) through chk_plan (cold Jacobi: the iteration plan's warm-start bases stay untouched),
+// the two distances, the decision.  Every kernel is a no-op once st->done, so a check after the stop changes nothing.
+void cuadmm_solver::enqueue_check() {
+    const int gm = ew_grid(con_num, device), gv = ew_grid(nloc, device);
+    double* part_m = chk_part.p;
+    double* part_x = part_m + 4 * (int64_t)gm;
+    double* part_n = part_x + 3 * (int64_t)gv;
+    chk_m_kernel<<<gm, kEwThreads, 0, stream>>>(con_num, y.p, Rp.p, bd.p, chk_yprev.p, chk_Rpprev.p, chk_dy.p, st.p, part_m);
+    chk_x_kernel<<<gv, kEwThreads, 0, stream>>>(nloc, X.p, Cd.p, chk_Xprev.p, chk_dX.p, st.p, part_x);
+    // the m-side sums come from replicated vectors and agree on every rank; the vec-side sums are this rank's share
+    const double* sum_x = part_x;
+    const double* sum_n = part_n;
+    int nsum_x = gv, nsum_n = gv;
+    if (world > 1) {
+        chk_publish_kernel<3><<<1, 256, 0, stream>>>(peer->view(), part_x, gv, peer->ptrs(peer->off_scal_chk), &st.p->done);
+        sum_x = peer->local<double>(peer->off_scal_chk); nsum_x = world;
+        sum_n = peer->local<double>(peer->off_scal_chk + 256); nsum_n = world;
+        ++launches;
+    }
+    SpmvEpilogue e;
+    spmv_launch(*At, 1.0, chk_dy.p, 0.0, chk_v.p, e, stream);
+    chk_pretest_kernel<<<1, 256, 0, stream>>>(st.p, part_m, gm, sum_x, nsum_x, chk_skip.p);
+    launches += 4;
+    chk_plan->done_flag = chk_skip.p;
+    launches += chk_plan->project(chk_v.p, chk_pv.p, stream, nullptr, false);
+    chk_plan->done_flag = chk_skip.p + 1;
+    launches += chk_plan->project(chk_dX.p, chk_pdX.p, stream, nullptr, false);
+    chk_norms_kernel<<<gv, kEwThreads, 0, stream>>>(nloc, chk_pv.p, chk_dX.p, chk_pdX.p, chk_skip.p, part_n);
+    if (world > 1) {
+        chk_publish_kernel<2><<<1, 256, 0, stream>>>(peer->view(), part_n, gv, peer->ptrs(peer->off_scal_chk + 256), &st.p->done);
+        ++launches;
+    }
+    chk_decide_kernel<<<1, 256, 0, stream>>>(st.p, sum_n, nsum_n, chk_skip.p, chk_eps);
+    launches += 2;
+    CUADMM_CUDA(cudaGetLastError());
+}
+
+// The certificate of the last solve in the caller's units: which 0: y-bar = dy ./ normA / (bscale beta), so b'y-bar = 1;
+// which 1: d = dX / (Cscale kappa), so <C, d> = -1 (full length: collective on a sharded solver)
+void cuadmm_solver::certificate(int which, double* h_out, double* h_ratio) {
+    CUADMM_REQUIRE(which == 0 || which == 1, "which must be 0 (primal infeasibility) or 1 (dual infeasibility)");
+    CUADMM_REQUIRE(cert_ok[which], which == 0 ? "the last solve produced no primal infeasibility certificate"
+                                              : "the last solve produced no dual infeasibility certificate");
+    CUADMM_REQUIRE(h_out, "null argument");
+    CUADMM_CUDA(cudaSetDevice(device));
+    if (which == 0) {
+        chk_dy.download(h_out, con_num, stream);
+        CUADMM_CUDA(cudaStreamSynchronize(stream));
+        const double s = bscale * cert_beta;
+        for (int64_t i = 0; i < con_num; ++i) h_out[i] = h_out[i] / h_normA[i] / s;
+    } else {
+        if (world > 1) gather_full(chk_dX, h_out);
+        else { chk_dX.download(h_out, vec_len, stream); CUADMM_CUDA(cudaStreamSynchronize(stream)); }
+        const double s = Cscale * cert_kappa;
+        for (int64_t i = 0; i < vec_len; ++i) h_out[i] /= s;
+    }
+    if (h_ratio) *h_ratio = cert_ratio[which];
+}
+
 // Sharded solver: sum over ranks of the partial products alpha * A[:, I_g] x_g.
 //   for_rp == false:  asmc = sum                                     (K1 / K5)
 //   for_rp == true :  Rp = b - sum, residual scalars for K9          (K8)
@@ -608,6 +805,23 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
         if (graph_sgs) { cudaGraphExecDestroy(graph_sgs); graph_sgs = nullptr; }
         if (graph_admm) { cudaGraphExecDestroy(graph_admm); graph_admm = nullptr; }
     }
+    const bool check = chk_interval > 0;
+    cert_ok[0] = cert_ok[1] = false;
+    if (check && !chk_plan) {
+        // a second plan over the same blocks without warm start: the projections of the check never see or move
+        // the iteration plan's Jacobi bases, so the iterates are the same with the check on or off
+        chk_plan.reset(new cuadmm_plan());
+        chk_plan->layout.init(shard.local_blk.data(), (int64_t)shard.local_blk.size(), shard.local_types.data());
+        chk_plan->device = device;
+        chk_plan->build_device();
+        chk_plan->warm_start = false;
+        chk_plan->d_Q.release();
+        const int64_t mm = std::max<int64_t>(m, 1), nn = std::max<int64_t>(n, 1);
+        chk_yprev.alloc(mm); chk_Rpprev.alloc(mm); chk_dy.alloc(mm);
+        chk_Xprev.alloc(nn); chk_dX.alloc(nn); chk_v.alloc(nn); chk_pv.alloc(nn); chk_pdX.alloc(nn);
+        chk_part.alloc(4 * (int64_t)ew_grid(m, device) + 5 * (int64_t)ew_grid(n, device));
+        chk_skip.alloc(2);
+    }
     info_iter_num = 0;
     for (auto& v : h_hist) v.clear();
     int64_t drained = 0;                 // iterations whose history entries are already on the host
@@ -662,7 +876,17 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     h_st->done = 0; h_st->stop_reason = 0;
     if (std::max(h_st->maxfeas, h_st->relgap) < stop_tol) { h_st->done = 1; h_st->stop_reason = 1; }
     if (1 > max_iter) { h_st->done = 1; h_st->stop_reason = 2; }
+    h_st->chk_iter = 0; h_st->chk_fired = 0;
+    h_st->chk_pratio = h_st->chk_dratio = INFINITY;
+    h_st->chk_count = h_st->chk_nproj_p = h_st->chk_nproj_d = 0;
+    h_st->chk_min_pratio = h_st->chk_min_dratio = h_st->chk_min_cosp = h_st->chk_min_cosd = INFINITY;
     CUADMM_CUDA(cudaMemcpyAsync(st.p, h_st, sizeof(DevState), cudaMemcpyHostToDevice, stream));
+    if (check) {
+        // the first window starts at the point this solve starts from
+        CUADMM_CUDA(cudaMemcpyAsync(chk_Xprev.p, X.p, sizeof(double) * n, cudaMemcpyDeviceToDevice, stream));
+        CUADMM_CUDA(cudaMemcpyAsync(chk_yprev.p, y.p, sizeof(double) * m, cudaMemcpyDeviceToDevice, stream));
+        CUADMM_CUDA(cudaMemcpyAsync(chk_Rpprev.p, Rp.p, sizeof(double) * m, cudaMemcpyDeviceToDevice, stream));
+    }
     CUADMM_CUDA(cudaStreamSynchronize(stream));
 
     if (rank != 0) verbose = false;   // one log per job
@@ -697,10 +921,25 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
         if (done) { stop_iter = cur; break; }
         int target = it + 1;
         while (!is_log_iter(target) && target <= max_iter) ++target;
-        for (int k = it; k < target; ++k) launch_iteration(k, switch_admm, false);
+        for (int k = it; k < target; ++k) {
+            launch_iteration(k, switch_admm, false);
+            if (check && k % chk_interval == 0) enqueue_check();
+        }
         it = target;
     }
     info_iter_num = stop_iter - 1;
+    last_stop_reason = h_st->stop_reason;
+    if (check && h_st->chk_fired && (last_stop_reason == 3 || last_stop_reason == 4)) {
+        cert_ok[0] = (h_st->chk_fired & 1) != 0; cert_ok[1] = (h_st->chk_fired & 2) != 0;
+        cert_ratio[0] = h_st->chk_pratio; cert_ratio[1] = h_st->chk_dratio;
+        cert_beta = h_st->chk_beta; cert_kappa = h_st->chk_kappa;
+    }
+    const double pratio = h_st->chk_pratio, dratio = h_st->chk_dratio;
+    {
+        const double v[8] = {(double)h_st->chk_count, (double)h_st->chk_nproj_p, (double)h_st->chk_nproj_d, h_st->chk_min_pratio,
+                             h_st->chk_min_dratio, h_st->chk_min_cosp, h_st->chk_min_cosd, (double)h_st->chk_iter};
+        for (int q = 0; q < 8; ++q) chk_stats[q] = v[q];
+    }
 
     // the partial iteration the reference runs before it breaks, then the best-iterate restore
     h_st->done = 0;
@@ -728,7 +967,12 @@ void cuadmm_solver::solve(int max_iter, double stop_tol, int sig_update_threshol
     if (peer) peer->check(stream);
     if (verbose) {
         printf("\n -------------------------------------------------------------------------------\n\n");
-        printf("%s\n", h_st->stop_reason == 2 ? "Solver ended: maximum iteration reached" : "Solver ended: converged.");
+        if (last_stop_reason == 3)
+            printf("Solver ended: primal infeasible (certificate ratio %2.1e at iteration %lld)\n", pratio, (long long)info_iter_num);
+        else if (last_stop_reason == 4)
+            printf("Solver ended: dual infeasible (certificate ratio %2.1e at iteration %lld)\n", dratio, (long long)info_iter_num);
+        else
+            printf("%s\n", h_st->stop_reason == 2 ? "Solver ended: maximum iteration reached" : "Solver ended: converged.");
         printf("\n primal infeasibility = %2.1e \n dual   infeasibility = %2.1e \n relative gap         = %2.1e",
                h_st->errRp, h_st->errRd, h_st->relgap);
         printf("\n primal objective = %- 9.8e \n dual   objective = %- 9.8e", h_st->pobj, h_st->dobj);
@@ -905,6 +1149,7 @@ void cuadmm_solver::load_data(const int32_t* b_idx, const double* b_val, int64_t
     iterate_scaled = true;
     info_iter_num = 0;
     for (auto& v : h_hist) v.clear();
+    cert_ok[0] = cert_ok[1] = false;     // they certified the old b and C
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1017,6 +1262,7 @@ int cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* h
         CUADMM_REQUIRE(s && s->initialised, "solver not initialised");
         CUADMM_CUDA(cudaSetDevice(s->device));
         s->set_iterate(h_X, h_y, h_S);
+        s->cert_ok[0] = s->cert_ok[1] = false;
         s->h_st->sig = sig;                 // pinned mirror: stays valid until the copy below has run
         CUADMM_CUDA(cudaMemcpyAsync(&s->st.p->sig, &s->h_st->sig, sizeof(double), cudaMemcpyHostToDevice, s->stream));
         CUADMM_CUDA(cudaStreamSynchronize(s->stream));
@@ -1024,6 +1270,32 @@ int cuadmm_solver_set_XyS(cuadmm_solver_t* s, const double* h_X, const double* h
 }
 
 int64_t cuadmm_solver_iter_num(const cuadmm_solver_t* s) { return s ? s->info_iter_num : -1; }
+
+int cuadmm_solver_set_infeasibility_check(cuadmm_solver_t* s, int interval, double eps) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s, "solver is null");
+        CUADMM_REQUIRE(interval >= 0, "interval < 0");
+        CUADMM_REQUIRE(interval == 0 || (eps > 0.0 && eps < 1.0), "eps must lie in (0, 1)");
+        s->chk_interval = interval;
+        if (interval > 0) s->chk_eps = eps;
+    });
+}
+
+int cuadmm_solver_infeasibility_stats(const cuadmm_solver_t* s, double out[8]) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s && out, "null argument");
+        for (int q = 0; q < 8; ++q) out[q] = s->chk_stats[q];
+    });
+}
+
+int cuadmm_solver_stop_reason(const cuadmm_solver_t* s) { return s ? s->last_stop_reason : CUADMM_EINVAL; }
+
+int cuadmm_solver_certificate(cuadmm_solver_t* s, int which, double* h_out, double* h_ratio) {
+    return guarded([&] {
+        CUADMM_REQUIRE(s, "solver is null");
+        s->certificate(which, h_out, h_ratio);
+    });
+}
 
 int cuadmm_solver_history(const cuadmm_solver_t* s, int which, double* out, int64_t cap) {
     return guarded([&] {

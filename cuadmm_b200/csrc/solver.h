@@ -25,8 +25,17 @@ struct DevState {
     int iter;            // index of the iteration about to run (1-based, as the reference's loop variable)
     int done;            // set by the scalar kernel when the stop test of the NEXT iteration fires
     int max_iter, sig_update_threshold, sig_update_stage_1, sig_update_stage_2, switch_admm;
-    int stop_reason;     // 1 converged, 2 max iterations
+    int stop_reason;     // 1 converged, 2 max iterations, 3 primal infeasible, 4 dual infeasible
     int pad_;
+    // infeasibility check (cuadmm_solver_set_infeasibility_check), written by its kernels only
+    int chk_iter;        // iteration of the last check that ran
+    int chk_fired;       // bit 0: primal infeasibility certificate at chk_iter, bit 1: dual
+    double chk_beta, chk_ndy, chk_nAdx, chk_kappa, chk_ndx;   // b_s'dy, |dy|, |A_s dX|, -<C_s, dX>, |dX|
+    double chk_pratio, chk_dratio;   // |Pi_K(A_s' dy)| / beta and max(|A_s dX|, |dX - Pi_K dX|) / kappa (inf: guard failed)
+    // over the checks of this solve: how many ran, how many ran each projection (candidate passed its guard), the
+    // smallest ratios, and the smallest guard values beta / (|b_s| |dy|) and kappa / (|C_s| |dX|) that passed
+    int chk_count, chk_nproj_p, chk_nproj_d, chk_pad_;
+    double chk_min_pratio, chk_min_dratio, chk_min_cosp, chk_min_cosd;
 };
 
 }  // namespace cuadmm
@@ -116,4 +125,20 @@ struct cuadmm_solver {
     cuadmm::DevBuf<double> asmc;             // -A (S-C) (summed over the ranks when sharded), reused by the next iteration's K1
     bool asmc_valid = false;
     void launch_iteration(int iter, int switch_admm, bool prof);
+    // infeasibility check every chk_interval iterations (0: off), enqueued by solve() between iteration graphs.
+    // Buffers and the second plan (cold Jacobi, its own scratch) exist only once the check has been enabled.
+    int chk_interval = 0;
+    double chk_eps = 1e-7;
+    std::unique_ptr<cuadmm_plan> chk_plan;
+    cuadmm::DevBuf<double> chk_yprev, chk_Rpprev, chk_dy;             // m: snapshots and dy of the last check
+    cuadmm::DevBuf<double> chk_Xprev, chk_dX, chk_v, chk_pv, chk_pdX;  // nloc: snapshot, dX, A_s' dy, the projections
+    cuadmm::DevBuf<double> chk_part;                                  // per-CTA partial sums
+    cuadmm::DevBuf<int> chk_skip;                                     // [2]: done flags of the two projections
+    int last_stop_reason = 0;                // of the last solve (0 before the first)
+    bool cert_ok[2] = {false, false};        // the last solve produced the primal / dual certificate
+    double cert_ratio[2] = {0, 0};
+    double cert_beta = 0, cert_kappa = 0;
+    double chk_stats[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // cuadmm_solver_infeasibility_stats of the last solve
+    void enqueue_check();
+    void certificate(int which, double* h_out, double* h_ratio);
 };

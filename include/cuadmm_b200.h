@@ -223,6 +223,33 @@ int  cuadmm_solver_update_data(cuadmm_solver_t* s,
  * which: 0 pobj 1 dobj 2 errRp 3 errRd 4 relgap 5 sig 6 bscale 7 Cscale */
 int64_t cuadmm_solver_iter_num(const cuadmm_solver_t* s);
 int  cuadmm_solver_history(const cuadmm_solver_t* s, int which, double* out, int64_t cap);
+/* Infeasibility detection (INTEGRATION.md §10).  Every `interval` iterations the solve compares the iterates with those
+ * `interval` iterations earlier (dy, dX, in the solver's scaled space) and stops with
+ *   reason 3 (primal infeasible) when b'dy > 0 and |Pi_K(A'dy)| <= eps b'dy, or
+ *   reason 4 (dual infeasible)   when <C, dX> < 0 and max(|A dX|, |dX - Pi_K(dX)|) <= eps |<C, dX>|,
+ * where a candidate whose b'dy (or -<C, dX>) is below 1e-8 times the product of the norms is ignored.  interval = 0
+ * (the default) turns the check off; it may be set before or after init and applies from the next solve.
+ * CUADMM_EINVAL for interval < 0 and for eps outside (0, 1) with interval > 0.  A sharded solver needs the same interval
+ * and eps on every rank; its ranks reach the same decision at the same check bit for bit.  The iteration
+ * itself is the same with the check on: X, y, S, the history and the stop of a solve the check does not stop are
+ * bit-identical to the solve without it.  A stop by the check returns X, y, S as the other stop reasons do, and
+ * info_iter_num is the iteration of the firing check. */
+int  cuadmm_solver_set_infeasibility_check(cuadmm_solver_t* s, int interval, double eps);
+/* why the last solve stopped: 0 before the first solve, 1 converged, 2 max iterations, 3 primal infeasible,
+ * 4 dual infeasible (CUADMM_EINVAL for a null solver) */
+int  cuadmm_solver_stop_reason(const cuadmm_solver_t* s);
+/* the certificate of the last solve, in the caller's units:
+ *   which 0: y-bar (con_num entries) with b'y-bar = 1 and A'y-bar in -K* up to the ratio (primal infeasibility);
+ *   which 1: d (vec_len entries) with <C, d> = -1, A d ~ 0 and d in K up to the ratio (dual infeasibility).
+ * h_ratio (may be NULL) receives the ratio of the stopping test.  CUADMM_EINVAL unless the last solve produced that
+ * certificate; when both tests fired at the same check the stop reason is 3 and both can be read.  update_data,
+ * set_XyS and the next solve discard them.  which = 1 is collective on a sharded solver (every rank receives all of d). */
+int  cuadmm_solver_certificate(cuadmm_solver_t* s, int which, double* h_out, double* h_ratio);
+/* what the checks of the last solve saw: out[0] checks run, out[1] / out[2] checks whose primal / dual candidate passed
+ * its guard (and so ran its projection), out[3] / out[4] the smallest primal / dual ratio, out[5] / out[6] the smallest
+ * guard value b'dy / (|b| |dy|) / -<C, dX> / (|C| |dX|) that passed (scaled space; inf when none), out[7] the
+ * iteration of the last check */
+int  cuadmm_solver_infeasibility_stats(const cuadmm_solver_t* s, double out[8]);
 /* timings in seconds: out[0]=total_time (since init or the last update_data, as the reference), out[1]=init,
  * out[2]=solve loop, out[3]=projection total, out[4]=y-solve total, out[5]=spmv total,
  * out[6]=last cuadmm_solver_update_data (0 before the first) */
